@@ -3,6 +3,14 @@
 
   python bench.py --gpus N --steps K --warmup W            # the CUDA path (libiris)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm
+  python bench.py ... --dump-outputs DIR                   # + the outputs of the last timed step
+
+--dump-outputs writes what the caller of the timed step holds after the last timed step as
+DIR/<name>.npy (float32 / float64, under 64 MB): `features` and `frame_labels` [n, ...] and
+`triples` [n, 3] of the clips listed in `clips` (all of them, or a fixed seeded sample when they do
+not fit), `counts` [6] (TP, FP, FN, sum n_true, sum n_pred, sum correct over warm-up + timed steps),
+and at N > 1 `counts_reduced` / `triples_global` of the all-reduce.  The banks, the uniforms of
+every step and the stand-in predictions are seeded, so the same arguments give the same inputs.
 
 Workload (`config.workload`).  N = 1: BASELINE.json configs[1] -- synthetic 2-ch 16 kHz 10 s
 clips, background + voices + noise mixed at sampled gains, 6 time + 1 frequency mask, batch 256,
@@ -44,6 +52,18 @@ CFG = dict(n_chan=2, batch=256, n_frame=626, max_voices=7, max_noises=2, snr=-20
            seed=20202, global_batch_cfg3=8192)
 METRIC = 'augmented spectrogram clips/sec'
 UNIT = 'clips/s'
+DUMP_BYTES = 64_000_000 - 4096     # --dump-outputs: array bytes of all files, .npy headers kept below 4 KB
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array (float32 / float64), so that two builds can be
+    compared output for output on the same seeded inputs."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(dirname, name + '.npy'), a)
+    sys.stderr.write('bench.py: %d arrays, %.1f MB written to %s\n'
+                     % (len(arrays), sum(a.nbytes for a in arrays.values()) / 1e6, dirname))
 
 
 def ncu_traffic():
@@ -353,8 +373,9 @@ def run_gpu_arm(args):
         st = dict(scfg=eng.step_config(cfg, L.FEAT_LOGMEL_MINMAX), n_u=uniforms_per_clip(cfg), b=b,
                   feat=[torch.empty((b, CFG['n_mels'], T, CFG['n_chan']), device=dev) for _ in range(2)],
                   frame=[torch.empty((b, T, K), device=dev) for _ in range(2)],
-                  # stand-in for the model output the metric kernels score (fixed, generated once)
-                  y_pred=torch.rand((b, T, K), device=dev),
+                  # stand-in for the model output the metric kernels score (fixed, seeded, generated once)
+                  y_pred=torch.rand((b, T, K), device=dev,
+                                    generator=torch.Generator(dev).manual_seed(CFG['seed'] + rank)),
                   counts=torch.zeros(6, dtype=torch.int64, device=dev),
                   reduced=torch.zeros(6, dtype=torch.int64, device=dev),
                   send=torch.zeros((b_global, 3), dtype=torch.int32, device=dev),
@@ -375,7 +396,27 @@ def run_gpu_arm(args):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     LAG = 2          # the reduced counts are a logged metric: consumed two steps late (N > 1)
 
-    def timed_loop(st, n_warm, n_steps, sampler=None):
+    def last_outputs(st, j):
+        """What the caller of the timed step holds after its last step: the features, frame labels and
+        per-sample triples of every clip (of a fixed, seeded sample of the clips when they exceed
+        DUMP_BYTES), the counts accumulated over all steps (+ the all-reduced ones at N > 1)."""
+        b, lo = st['b'], st['lo']
+        fixed = 6 * 8 + ((6 + st['b_global'] * 3) * 8 if comm is not None else 0)
+        per_clip = (st['feat'][j][0].numel() + st['frame'][j][0].numel()) * 4 + 3 * 8 + 8
+        n = min(b, (DUMP_BYTES - fixed) // per_clip)
+        clips = np.arange(b) if n == b else np.sort(np.random.default_rng(CFG['seed']).choice(b, n, replace=False))
+        idx = torch.from_numpy(clips).to(dev)
+        out = {'clips': clips.astype(np.float64),
+               'features': st['feat'][j].index_select(0, idx).cpu().numpy(),
+               'frame_labels': st['frame'][j].index_select(0, idx).cpu().numpy(),
+               'triples': st['send'][lo:lo + b].index_select(0, idx).cpu().numpy().astype(np.float64),
+               'counts': st['counts'].cpu().numpy().astype(np.float64)}
+        if comm is not None:
+            out['counts_reduced'] = st['reduced'].cpu().numpy().astype(np.float64)
+            out['triples_global'] = st['glob'].cpu().numpy().astype(np.float64)
+        return out
+
+    def timed_loop(st, n_warm, n_steps, sampler=None, keep_last=False):
         us = [rng.random((st['b'], st['n_u'])) for _ in range(n_warm + n_steps)]
         eng.profile(False)
         for s in range(n_warm):
@@ -403,6 +444,7 @@ def run_gpu_arm(args):
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
+        last = last_outputs(st, (n_steps - 1) & 1) if keep_last else None   # before the replay below overwrites them
         total_ms = float(np.sum([a.elapsed_time(b) for a, b in ev]))
         fused_ms, n_fused = eng.profile_read()
         eng.profile(False)
@@ -424,12 +466,12 @@ def run_gpu_arm(args):
             alg += bi + bo
             ker += ki + ko
         return dict(total_ms=total_ms, total_ms_max=float(t.item()), fused_ms=fused_ms, n_fused=n_fused,
-                    alg_bytes=alg / n_steps, kernel_bytes=ker / n_steps, kernel_clips=k_clips)
+                    alg_bytes=alg / n_steps, kernel_bytes=ker / n_steps, kernel_clips=k_clips, last=last)
 
     # ---- device-timed: inputs (banks) resident, the uniforms of every step drawn beforehand ----
     st = step_setup(B, Bg, lo)
     sampler = ClockSampler(local)
-    r = timed_loop(st, args.warmup, args.steps, sampler)
+    r = timed_loop(st, args.warmup, args.steps, sampler, keep_last=args.dump_outputs is not None and rank == 0)
     value = Bg * args.steps / (r['total_ms_max'] / 1e3)
 
     # ---- end to end through the public drop-in call chain: host uniforms in (numpy) -> one iris_step
@@ -601,6 +643,8 @@ def run_gpu_arm(args):
     if rank == 0:
         if not args.no_cpu_baseline:      # the CPU leg, on rank 0's host cores, at every N
             out['cpu_baseline'] = cpu_baseline()
+        if args.dump_outputs is not None:
+            dump_outputs(args.dump_outputs, r['last'])
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()
@@ -698,7 +742,13 @@ def main():
     ap.add_argument('--batch', type=int, default=0, help='N = 1 only: another batch size (experiments)')
     ap.add_argument('--no-cfg3', action='store_true', help='skip the 8192-clip single-GPU leg (profiling runs)')
     ap.add_argument('--no-consumer-check', action='store_true', help='skip the configs[4] substitute-consumer leg')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step (rank 0) to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs is not None and args.impl != 'b200':
+        ap.error('--dump-outputs needs --impl b200 (the reference arm keeps no outputs)')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':
         run_reference_arm(args)
