@@ -31,8 +31,8 @@ def _stale(target, deps):
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force=False, verbose=False, extra_flags=(), lib=None, obj_dir=None):
-    """``extra_flags`` / ``lib`` / ``obj_dir`` build experiment variants (scripts/ only)."""
+def build(force=False, verbose=False, lib=None, obj_dir=None):
+    """``lib`` / ``obj_dir``: build elsewhere than in-tree (e.g. another revision, loaded with IRIS_LIB)."""
     nvcc = _nvcc()
     global OBJ, LIB
     if lib:
@@ -50,7 +50,7 @@ def build(force=False, verbose=False, extra_flags=(), lib=None, obj_dir=None):
         o = os.path.join(OBJ, src.replace('.cu', '.o'))
         objs.append(o)
         if force or _stale(o, [s] + headers):
-            cmd = [nvcc] + NVCC_FLAGS + list(extra_flags) + (['-Xptxas', '-v'] if verbose else []) + ['-c', s, '-o', o]
+            cmd = [nvcc] + NVCC_FLAGS + (['-Xptxas', '-v'] if verbose else []) + ['-c', s, '-o', o]
             r = subprocess.run(cmd, capture_output=True, text=True)
             if verbose or r.returncode:
                 sys.stderr.write(r.stdout + r.stderr)

@@ -35,18 +35,9 @@ IRIS_HD int xw_read_off(int k1, int m) { return k1 * kXwRowBytes + m * 16; }    
 // same address are served by one broadcast, so a 128-bit read of the warp touches 16 distinct
 // 16-byte pieces (2 wavefronts) instead of 32 (4 wavefronts).  Row stride 272 B puts rows
 // k1 = 0..7 into distinct 16-byte bank groups, so those two wavefronts are conflict-free.
-#ifndef IRIS_LANE_MAP
-#define IRIS_LANE_MAP 1
-#endif
-#if IRIS_LANE_MAP == 1
 IRIS_HD int warp_k1(int lane) { return lane >> 1; }
 IRIS_HD int warp_par(int lane) { return lane & 1; }
 IRIS_HD int warp_lane_of(int k1, int par) { return 2 * k1 + par; }
-#else
-IRIS_HD int warp_k1(int lane) { return lane & 15; }
-IRIS_HD int warp_par(int lane) { return lane >> 4; }
-IRIS_HD int warp_lane_of(int k1, int par) { return k1 + 16 * par; }
-#endif
 // bin held by register j of a lane after pass 2
 IRIS_HD int warp_bin(int lane, int j) { return warp_k1(lane) + 16 * (2 * j + warp_par(lane)); }
 // lane holding the mirror bins of this lane (k1 = 0: the lane itself)

@@ -48,8 +48,8 @@ int build_tables(iris_ctx* c) {
     CU(cudaMemcpy(c->tw.p, tw.data(), tw.size() * 4, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(c->ts.p, ts.data(), ts.size() * 4, cudaMemcpyHostToDevice));
     CU(cudaMemcpy(c->whalf.p, hann.data(), hann.size() * 4, cudaMemcpyHostToDevice));
-    CU(c->sched.reserve(8 * 64));     // (next chunk, CTAs finished) per launch of a split batch; [2], [3]: post tickets of an unsplit launch
-    CU(cudaMemset(c->sched.p, 0, 8 * 64));
+    CU(c->sched.reserve(8));   // k_fused work counters: next chunk, CTAs finished
+    CU(cudaMemset(c->sched.p, 0, 8));
     return IRIS_OK;
 }
 
@@ -73,7 +73,7 @@ void set_geometry(iris_ctx* c, FusedParams& p, int n_chan, bool mel) {
     p.n_pairs = (n_chan + 1) / 2;
     p.c_out = n_chan;
     if (!mel) p.mel_taps = 0;   // no mel tables in shared memory
-    p.fr = fused_pick_fr(p.T, p.mel_taps);
+    p.fr = fused_pick_fr(p.mel_taps);
     (void)c;
 }
 
@@ -141,10 +141,9 @@ int run_labels(iris_ctx* c, float* d_vtk, float* d_frame, uint8_t* d_keep_out, c
 // tile-block scratch + launch parameters of a launch
 int prepare_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs) {
     p.max_segs = max_segs < 1 ? 1 : max_segs;
-    p.stage_out = fused_stages_output(mode, p.remap, p.fr) && !getenv("IRIS_NO_STAGE") ? 1 : 0;
+    p.stage_out = fused_stages_output(mode, p.remap, p.fr) ? 1 : 0;
     p.fm_bits = (mode == FM_MEL && p.mel_f_lo + p.mel_f_n <= 128) ? 1 : 0;   // = the NJ == 4 kernels
-    p.pair_merge = p.stage_out && p.C == 4 && !getenv("IRIS_NO_PAIR_MERGE") ? 1 : 0;
-    p.l2_hints = getenv("IRIS_NO_L2_HINTS") ? 0 : 1;   // measured: min-max log-mel 255 -> 250 us
+    p.pair_merge = p.stage_out && p.C == 4 ? 1 : 0;
     int stride = 0;
     const size_t bytes = fused_tile_bytes(p, &stride);
     const void* before = c->tiles.p;
@@ -156,13 +155,7 @@ int prepare_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs) {
     // tiles per work claim.  With the claims shrinking towards the end of a launch (fused_schedule) larger
     // chunks no longer cost a longer tail: 4 / 6 / 8 / 16 tiles -> k_fused 173.6 / 172.4 / 172.6 / 177.6 us
     p.chunk = 6;
-    if (const char* e = getenv("IRIS_CHUNK")) {
-        const int v = atoi(e);
-        if (v >= 1 && v <= 4096) p.chunk = v;
-    }
     if (p.pair_merge && (p.chunk & 1)) ++p.chunk;   // both pairs of a (clip, time) range in one work claim
-    p.tile_first = 0;
-    p.tile_count = 0;
     return IRIS_OK;
 }
 
@@ -188,9 +181,7 @@ void tile_sig_set(iris_ctx* c, const FusedParams& p) {
 int run_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs, cudaStream_t st) {
     int rc = prepare_fused(c, p, mode, max_segs);
     if (rc) return rc;
-    const bool have = tile_sig_matches(c, p);
-    CU(launch_fused(p, mode, c->num_sms, st,
-                    have ? (FUSED_LAUNCH_KERNEL | FUSED_LAUNCH_PDL) : (FUSED_LAUNCH_TILES | FUSED_LAUNCH_KERNEL)));
+    CU(launch_fused(p, mode, c->num_sms, st, !tile_sig_matches(c, p)));
     tile_sig_set(c, p);
     if (c->ev_after_fused) {   // iris_step: the metric leg starts behind the feature kernel
         CU(cudaEventRecord(c->ev_after_fused, st));
@@ -223,79 +214,14 @@ int timed_fused(iris_ctx* c, FusedParams& p, int mode, cudaStream_t st) {
     return IRIS_OK;
 }
 
-// Clips per part of a split min-max log-mel launch (0: one launch).  k_logmel_post needs every
-// mel value of a clip, i.e. it can only follow k_fused; with the batch cut into parts that
-// alternate between two streams the second pass of part i runs beside k_fused of part i + 1
-// (one small CTA fits next to the two resident k_fused CTAs of an SM) and reads its rows out of
-// L2 even when the whole batch is far larger than L2.
-int split_part_clips(int B) {
-    // Experiment switch, off by default.  Measured on B200 (profiles/r02_split_ab.txt): every k_fused
-    // launch pays ~30 us of ramp-up and tail (t = 30 us + 0.62 us per clip), which is more than the
-    // overlap returns: batch 256 in two parts 239 -> 258 us, batch 1024 in four 855 -> 875 us,
-    // batch 8192 in 32 parts 6.68 -> 7.04 ms.
-    int part = 0;
-    if (const char* e = getenv("IRIS_SPLIT")) part = atoi(e);
-    if (part <= 0 || B < 2 * part) return 0;
-    const int max_parts = 64;   // work counters of c->sched
-    if ((B + part - 1) / part > max_parts) part = (B + max_parts - 1) / max_parts;
-    return part;
-}
-
-// min-max log-mel: k_tiles (whole batch) -> per part {k_fused -> k_logmel_post}
+// min-max log-mel: k_fused (features + per-clip extrema) -> k_logmel_post (normalise + log in place)
 int run_logmel_minmax(iris_ctx* c, FusedParams& p, float* d_out, cudaStream_t st) {
     const size_t per_clip = size_t(c->n_mel) * c->T * c->C;
     uint32_t* mm = c->minmax.as<uint32_t>();
     unsigned* done = reinterpret_cast<unsigned*>(mm + 2 * size_t(c->B));
-    const int part = split_part_clips(c->B);
-    if (part == 0) {
-        // fixed 2-channel instance: a post warp per CTA runs the second pass inside k_fused
-        int rc = prepare_fused(c, p, FM_MEL, c->max_segs);
-        if (rc) return rc;
-        p.clip_done = reinterpret_cast<uint32_t*>(done + c->B);
-        p.post_parts = p.clip_done + c->B;
-        p.post_in_kernel = fused_can_post_in_kernel(p) ? 1 : 0;
-        rc = timed_fused(c, p, FM_MEL, st);
-        if (rc) return rc;
-        if (!p.post_in_kernel) CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
-        return IRIS_OK;
-    }
-    if (!c->aux) {
-        CU(cudaStreamCreateWithFlags(&c->aux, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&c->ev_tiles, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
-    }
-    int rc = prepare_fused(c, p, FM_MEL, c->max_segs);
+    int rc = timed_fused(c, p, FM_MEL, st);
     if (rc) return rc;
-    tile_sig_set(c, p);   // (this path always runs k_tiles)
-    const int per_clip_tiles = ((c->T + p.fr - 1) / p.fr) * p.n_pairs;
-    std::pair<cudaEvent_t, cudaEvent_t>* ev = nullptr;
-    if (c->profile) {   // the roofline hook times k_tiles + k_fused of the first part
-        rc = prof_events(c, &ev);
-        if (rc) return rc;
-        CU(cudaEventRecord(ev->first, st));
-    }
-    int n_parts = 0;
-    for (int b0 = 0; b0 < c->B; b0 += part, ++n_parts) {
-        const int nb = std::min(part, c->B - b0);
-        cudaStream_t s = (n_parts & 1) ? c->aux : st;
-        FusedParams q = p;
-        q.tile_first = b0 * per_clip_tiles;
-        q.tile_count = nb * per_clip_tiles;
-        q.sched = c->sched.as<uint32_t>() + 2 * n_parts;
-        CU(launch_fused(q, FM_MEL, c->num_sms, s, n_parts == 0 ? (FUSED_LAUNCH_TILES | FUSED_LAUNCH_KERNEL) : FUSED_LAUNCH_KERNEL));
-        if (n_parts == 0) {
-            if (ev) {
-                CU(cudaEventRecord(ev->second, st));
-                c->prof_clips = nb;
-            }
-            // the other stream starts behind k_tiles (and behind whatever the caller queued before)
-            CU(cudaEventRecord(c->ev_tiles, st));
-            CU(cudaStreamWaitEvent(c->aux, c->ev_tiles, 0));
-        }
-        CU(launch_logmel_post(d_out + size_t(b0) * per_clip, mm + 2 * size_t(b0), done + b0, nb, per_clip, 1, 1, s));
-    }
-    CU(cudaEventRecord(c->ev_join, c->aux));
-    CU(cudaStreamWaitEvent(st, c->ev_join, 0));
+    CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
     return IRIS_OK;
 }
 
@@ -461,9 +387,6 @@ int iris_ctx_destroy(iris_ctx* c) {
         if (c->stage_free[i]) cudaEventDestroy(c->stage_free[i]);
     }
     iris_step_release(c);
-    if (c->aux) cudaStreamDestroy(c->aux);
-    if (c->ev_tiles) cudaEventDestroy(c->ev_tiles);
-    if (c->ev_join) cudaEventDestroy(c->ev_join);
     for (auto& ev : c->prof_events) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
     delete c;
     return IRIS_OK;
@@ -577,8 +500,7 @@ int iris_set_mel(iris_ctx* c, int n_mel, int n_bins, const float* w) {
         auto next = [&]() { rng = rng * 1664525u + 1013904223u; return rng >> 8; };
         double temp = 2.0;
         const int used_rounds = (n_mel + 31) / 32;
-        const int iters = getenv("IRIS_MEL_NATURAL") ? 0 : 60000;   // A/B switch: filter m on lane m % 32 of round m / 32
-        for (int it = 0; it < iters && best_cost > 2 * taps; ++it) {
+        for (int it = 0; it < 60000 && best_cost > 2 * taps; ++it) {
             const int a = int(next() % uint32_t(32 * used_rounds)), b = int(next() % uint32_t(32 * used_rounds));
             if (a == b || slot[a] == slot[b]) continue;
             std::swap(slot[a], slot[b]);
@@ -1117,7 +1039,7 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
         if (p.do_minmax) {   // per-clip (~min, max) bit patterns; k_logmel_post leaves them
                              // zeroed, so only a fresh allocation is cleared
             const void* before = c->minmax.p;
-            CU(c->minmax.reserve(size_t(c->B) * 20));   // [B,2] min/max words + [B] k_logmel_post counters + [B] tiles done + [B] parts posted
+            CU(c->minmax.reserve(size_t(c->B) * 12));   // [B,2] min/max words + [B] k_logmel_post counters
             if (c->minmax.p != before) CU(cudaMemsetAsync(c->minmax.p, 0, c->minmax.cap, st));
             p.minmax = c->minmax.as<uint32_t>();
         }

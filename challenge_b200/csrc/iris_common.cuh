@@ -60,24 +60,17 @@ struct FusedParams {
     int32_t chunk;               // consecutive tiles per work claim
     int32_t n_big, n_mid;        // claim schedule (launch_fused): n_big claims of `chunk` tiles, n_mid of
     int32_t chunk_mid, chunk_tail;   // `chunk_mid`, the rest `chunk_tail`
-    int32_t tile_first, tile_count;   // tiles [tile_first, tile_first + tile_count) of the batch belong to this launch
     int32_t seg_select;          // 0: every segment; 1: voices only; 2: background + noises only
                                  // (only_voice / only_noise of pipeline.py:37-38, 82-83, 104-108)
-    uint32_t* sched;             // [4] next chunk, CTAs finished, next post item, post warps finished; zero between launches
+    uint32_t* sched;             // [2] next chunk, CTAs finished; zero between launches
     // outputs
     float* out;             // layout depends on mode
     int32_t stage_out;      // spectrogram modes: store through the shared-memory staging area
     int32_t pair_merge;     // stage_out with C == 4: the two channel pairs of a tile are stored together
-    int32_t l2_hints;       // L2 eviction hints on the bank stream / the mel rows
     uint8_t* activity;      // FM_ACTIVITY: [B, T]
     // FM_MEL epilogue variants: log(x + 1e-8) and per-clip min-max before the log
     int32_t do_log, do_minmax;
     uint32_t* minmax;       // [B,2] atomicMax of (~bits(min), bits(max)); zeroed by k_tiles
-    // second pass inside k_fused (min-max log-mel, fixed 2-channel instance): consumer warps count the
-    // finished tiles of every clip, a post warp per CTA normalises + logs a clip as soon as it is whole
-    int32_t post_in_kernel;
-    uint32_t* clip_done;    // [B] tiles of the clip whose features are written (zero between launches)
-    uint32_t* post_parts;   // [B] parts of the clip the post warps have finished (zero between launches)
     // mel projection: filters are handled in rounds of 32 (m = lane + 32 r); every filter of
     // round r reads mel_L[r] consecutive magnitudes starting at bin mel_f_lo + mel_info[m]
     // (shorter filters are zero-padded), weights at mel_w[(row0(r) + i) * 32 + lane]
@@ -92,10 +85,6 @@ struct FusedParams {
     const float4* tw1;      // [8][32] {W512^(n2*2q), W512^(n2*(2q+1))}
     const float4* ts;       // [8][2]  {t(2m), t(2m+1)}, t(i) = par ? W32^i : 1
     const float* hann;      // [512] periodic Hann
-#ifdef IRIS_TRACE
-    unsigned long long* trace;   // experiment builds (scripts/trace_fused.py): [grid + 1][64] time stamps
-    int32_t trace_grid;
-#endif
 };
 
 // ---- PTX helpers: mbarrier + bulk async copy (TMA 1-D) ----
@@ -165,15 +154,6 @@ __device__ __forceinline__ void red_max_u32_if(uint32_t* addr, uint32_t v, bool 
         "r"(v), "r"(uint32_t(pred))
         : "memory");
 }
-// global -> shared bulk copy, completion signalled on an mbarrier (SASS: UBLKCP)
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes,
-                                         uint64_t* bar) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::
-            "r"(smem_u32(dst_smem)),
-        "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
 // L2 cache policies: the streamed bank rows are marked evict-first, the mel rows that the
 // second pass (k_logmel_post) re-reads right after the kernel evict-last, so the 102 MB of
 // features survive in the 126 MB L2 next to the input stream
@@ -187,6 +167,7 @@ __device__ __forceinline__ uint64_t l2_policy_evict_last() {
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
     return pol;
 }
+// global -> shared bulk copy under an L2 cache policy, completion signalled on an mbarrier (SASS: UBLKCP)
 __device__ __forceinline__ void bulk_g2s_hint(void* dst_smem, const void* src_gmem, uint32_t bytes,
                                               uint64_t* bar, uint64_t policy) {
     asm volatile(
@@ -194,20 +175,6 @@ __device__ __forceinline__ void bulk_g2s_hint(void* dst_smem, const void* src_gm
             "r"(smem_u32(dst_smem)),
         "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
         : "memory");
-}
-// L2 prefetch of a span that a bulk copy will fetch shortly (no shared memory involved)
-__device__ __forceinline__ void bulk_prefetch_l2_if(const void* src_gmem, uint32_t bytes, bool pred) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.u32 p, %2, 0;\n\t"
-        "@p cp.async.bulk.prefetch.L2.global [%0], %1;\n\t}" ::"l"(src_gmem),
-        "r"(bytes), "r"(uint32_t(pred))
-        : "memory");
-}
-__device__ __forceinline__ uint32_t ld_acquire_gpu_u32(const uint32_t* p) {
-    uint32_t v;
-    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
 }
 __device__ __forceinline__ void st_f2_hint(float* addr, float a, float b, uint64_t policy) {
     asm volatile("st.global.L2::cache_hint.v2.f32 [%0], {%1, %2}, %3;" ::"l"(addr), "f"(a), "f"(b), "l"(policy)
@@ -243,33 +210,6 @@ __device__ __forceinline__ float fast_atan2f(float y, float x) {
     if (ay > ax) r = 1.57079632679489662f - r;
     if (__float_as_uint(x) >> 31) r = 3.14159265358979324f - r;
     return copysignf(r, y);
-}
-// two atan2 at once: the octant reduction and the sign fix-ups stay scalar, the degree-17 polynomial
-// runs on packed pairs (FMUL2 / FFMA2: 10 instructions for both instead of 20).  Same operations in
-// the same order as fast_atan2f, so the results are bit-identical to two scalar calls.
-__device__ __forceinline__ void fast_atan2f_x2(float y0, float x0, float y1, float x1, float& r0, float& r1) {
-    const float ax0 = fabsf(x0), ay0 = fabsf(y0), ax1 = fabsf(x1), ay1 = fabsf(y1);
-    const float hi0 = fmaxf(ax0, ay0), lo0 = fminf(ax0, ay0);
-    const float hi1 = fmaxf(ax1, ay1), lo1 = fminf(ax1, ay1);
-    const cpx a{hi0 > 0.f ? __fdividef(lo0, hi0) : 0.f, hi1 > 0.f ? __fdividef(lo1, hi1) : 0.f};
-    const cpx s = cmul2(a, a);
-    cpx r{0.0028662257f, 0.0028662257f};
-    r = cfma2(r, s, cpx{-0.0161657367f, -0.0161657367f});
-    r = cfma2(r, s, cpx{0.0429096138f, 0.0429096138f});
-    r = cfma2(r, s, cpx{-0.0752896400f, -0.0752896400f});
-    r = cfma2(r, s, cpx{0.1065626393f, 0.1065626393f});
-    r = cfma2(r, s, cpx{-0.1420889944f, -0.1420889944f});
-    r = cfma2(r, s, cpx{0.1999355085f, 0.1999355085f});
-    r = cfma2(r, s, cpx{-0.3333314528f, -0.3333314528f});
-    r = cfma2(r, s, cpx{1.0f, 1.0f});
-    r = cmul2(r, a);
-    float q0 = r.x, q1 = r.y;
-    if (ay0 > ax0) q0 = 1.57079632679489662f - q0;
-    if (ay1 > ax1) q1 = 1.57079632679489662f - q1;
-    if (__float_as_uint(x0) >> 31) q0 = 3.14159265358979324f - q0;
-    if (__float_as_uint(x1) >> 31) q1 = 3.14159265358979324f - q1;
-    r0 = copysignf(q0, y0);
-    r1 = copysignf(q1, y1);
 }
 // Two atan2 for cells whose magnitude m = sqrt(x^2 + y^2) is already there (the mag/phase epilogue of
 // k_fused): half-angle form.  With d = m + |x|, t = y / d lies in [-1, 1] for every (x, y), so the

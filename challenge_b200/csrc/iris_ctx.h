@@ -121,16 +121,12 @@ struct iris_ctx {
     bool profile = false;
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
     size_t prof_used = 0;
-    int prof_clips = 0;               // clips of the launch the hook timed last (a split batch: its first part)
+    int prof_clips = 0;               // clips of the launch the hook timed last
     // stand-alone ops (iris_ops_abi.cu): dense mel matrix + column supports, small scratch
     DevBuf mel_dense, mel_lo, mel_len, op_small, minmax_ops, eval_scratch, spec_scratch;
     bool spec_mode = false;            // the uploaded plan mixes spectrogram banks
     int mel_bins = 0;
     bool mel_fusable = false;
-    // split feature launches (iris_abi.cu): parts of a large batch alternate between the caller's
-    // stream and `aux`, so that k_logmel_post of one part runs beside k_fused of the next
-    cudaStream_t aux = nullptr;
-    cudaEvent_t ev_tiles = nullptr, ev_join = nullptr;
     // ---- one-call step (iris_step.cu) ----
     cudaStream_t side = nullptr;       // metric leg: counting + count all-reduce beside the feature kernel
     cudaEvent_t ev_labels = nullptr;   // labels of the current step are written

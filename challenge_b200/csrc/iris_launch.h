@@ -7,20 +7,16 @@ namespace iris {
 
 struct FusedParams;
 
-// FUSED_LAUNCH_PDL: launch k_fused with programmatic stream serialization although k_tiles is not
-// launched in front of it (the kernel in front -- k_labels -- triggers early and wrote the tile blocks)
-enum { FUSED_LAUNCH_TILES = 1, FUSED_LAUNCH_KERNEL = 2, FUSED_LAUNCH_PDL = 4 };
-cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream,
-                         int what = FUSED_LAUNCH_TILES | FUSED_LAUNCH_KERNEL);
+// build_tiles: k_tiles builds the tile blocks first; false: the kernel in front (k_labels) wrote them
+cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream, bool build_tiles);
 size_t fused_smem_bytes(const FusedParams& p, int mode);
 void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge, int32_t out[5]);
-bool fused_can_post_in_kernel(const FusedParams& p);   // min-max log-mel: second pass inside k_fused (no k_logmel_post)
 int fused_max_segments();      // mixing segments one clip may have
 bool fused_stages_output(int mode, int remap, int fr);   // FusedParams::stage_out for a launch
 int fused_max_mel_taps();      // sum over the 32-filter rounds of the longest filter
 int fused_max_mel_filter();    // taps of the longest filter
 int fused_max_frames_per_tile();
-int fused_pick_fr(int T, int mel_taps);   // frames per tile (consumer warps per CTA)
+int fused_pick_fr(int mel_taps);   // frames per tile (consumer warps per CTA)
 size_t fused_tile_bytes(const FusedParams& p, int* stride_out);   // size of p.tile_blocks
 
 // k_post.cu

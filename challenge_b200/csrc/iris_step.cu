@@ -389,9 +389,7 @@ int iris_step(iris_ctx* c, const iris_step_config* cfg, const iris_step_io* io, 
     // k_fused and runs beside k_logmel_post (31 us, the leg takes ~10): k_labels -> k_fused stay
     // adjacent in the stream, so k_fused's programmatic launch overlaps its prologue with k_labels.
     // Other modes have no second pass to hide the leg behind: it forks right behind k_labels.
-    static const bool late_env = getenv("IRIS_METRIC_LATE") ? atoi(getenv("IRIS_METRIC_LATE")) != 0 : true;
-    bool late = metric && late_env && cfg->feature_mode == IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode;
-    if (getenv("IRIS_METRIC_EARLY")) late = false;
+    const bool late = metric && cfg->feature_mode == IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode;
     if (late) {
         c->ev_after_fused = c->ev_labels;
         rc = iris_features(c, cfg->feature_mode, io->d_features, stream);

@@ -32,9 +32,7 @@
 //    source row enters the SM once per tile.
 //  * LOGMEL_MINMAX: the warps of a CTA combine the extrema of a run of tiles of one clip in shared
 //    memory and the last one sends them to global atomics; k_logmel_post (k_post.cu) normalises and
-//    logs the batch in place right after (EPI_POST: a post warp per CTA
-//    does that inside this kernel instead -- opt-in, measured equal at the step level).
-#include <cstdio>
+//    logs the batch in place right after.
 #include <cstdlib>
 #include <cstring>
 
@@ -46,33 +44,9 @@
 
 namespace iris {
 
-// Experiment builds (-DIRIS_TRACE, scripts/trace_fused.py): per-CTA time stamps of the ramp-up, the
-// steady state and the tail of the persistent kernel.  Slot 0 / 10 are %globaltimer (aligns the
-// CTAs), the others clock64 of the SM.  Compiled out of the product build.
-#ifdef IRIS_TRACE
-__device__ __forceinline__ unsigned long long tr_gtimer() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-#define IRIS_TR(slot, val)                                                                   \
-    do {                                                                                     \
-        if (p.trace) p.trace[size_t(blockIdx.x) * 64 + (slot)] = (unsigned long long)(val);  \
-    } while (0)
-#define IRIS_TRC(slot) IRIS_TR(slot, clock64())
-#else
-#define IRIS_TR(slot, val) do { } while (0)
-#define IRIS_TRC(slot) do { } while (0)
-#endif
-
 constexpr int kRing = 8;         // TileBlock ring entries (> stage buffers + 1, see the producer)
-#ifndef IRIS_MAX_FR
-#define IRIS_MAX_FR 16
-#endif
-#ifndef IRIS_MAX_REGS
-#define IRIS_MAX_REGS 96   // no spills; 2 CTAs x 9 warps (FR = 8) or 17 warps (FR = 16) per SM fit the register file
-#endif
-constexpr int kMaxFR = IRIS_MAX_FR;   // consumer warps per CTA (sets the register budget)
+constexpr int kMaxFR = 16;       // consumer warps per CTA (sets the register budget)
+constexpr int kMaxRegs = 96;     // no spills; 2 CTAs x 9 warps (FR = 8) or 17 warps (FR = 16) per SM fit the register file
 constexpr int kMaxMel = 128;
 constexpr int kMaxTaps = 64;     // sum over the 32-filter rounds of the longest filter
 constexpr int kMaxFilter = 16;   // taps of the longest mel filter the fused epilogue takes
@@ -97,10 +71,8 @@ __host__ __device__ inline uint32_t off_slots(int mel_taps, int fr) {
 __host__ __device__ inline uint32_t slot_bytes(int fr) { return uint32_t(fr + 1) * 2048u; }
 // stage buffers per CTA: the modes that write whole spectrograms trade one stage buffer for
 // the store staging area below
-#ifndef IRIS_MEL_SLOTS
-#define IRIS_MEL_SLOTS 3
-#endif
-__host__ __device__ constexpr int slots_of(int mode) { return (mode == FM_MEL || mode == FM_ACTIVITY) ? IRIS_MEL_SLOTS : 2; }
+constexpr int kMelSlots = 3;
+__host__ __device__ constexpr int slots_of(int mode) { return (mode == FM_MEL || mode == FM_ACTIVITY) ? kMelSlots : 2; }
 // staging of a tile's [257 bins][FR frames] x 16 B output pieces (16-byte columns XOR-swizzled
 // by the bin so that both the per-frame writes and the per-bin reads are conflict-free)
 __host__ __device__ inline uint32_t stage_bytes(int fr) { return uint32_t(kBins) * uint32_t(fr) * 16u; }
@@ -120,9 +92,6 @@ __global__ void __launch_bounds__(128) k_tiles(const FusedParams p) {
     // programmatic dependent launch: k_fused may start its prologue (barriers, zero fill of the stage
     // buffers) now; it waits for this grid before it touches a tile block
     cudaTriggerProgrammaticLaunchCompletion();
-#ifdef IRIS_TRACE
-    if (p.trace && tile == 0) p.trace[size_t(p.trace_grid) * 64] = tr_gtimer();
-#endif
     const int per_clip = ((p.T + p.fr - 1) / p.fr) * p.n_pairs;
     if (tile >= p.B * per_clip) return;
     if (tile < p.B && p.minmax != nullptr) {   // per-clip extrema scratch of the launch that follows
@@ -164,11 +133,7 @@ __device__ __forceinline__ float4 make_piece(const FusedParams& p, int f, float 
     if (MODE != FM_COMPLEX) {
         a0 = sqrt_approx(fmaf(r0, r0, i0 * i0));   // transforms.py:116
         a1 = sqrt_approx(fmaf(r1, r1, i1 * i1));
-#ifdef IRIS_ATAN2_OCTANT
-        fast_atan2f_x2(i0, r0, i1, r1, b0, b1);    // transforms.py:117
-#else
         fast_atan2f_mag_x2(i0, r0, a0, i1, r1, a1, b0, b1);    // transforms.py:117, from the magnitudes above
-#endif
         if (MODE == FM_LOGMAGPHASE) {            // transforms.py:80-86
             a0 = __logf(a0 + 1e-8f);   // MUFU.LG2 * ln 2, as in the log-mel epilogue (|error| ~1e-6)
             a1 = __logf(a1 + 1e-8f);
@@ -204,44 +169,18 @@ __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, 
 // per-round flag branches, no odd-channel selects, C folded into the address arithmetic, the
 // projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.
 constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4;
-// EPI_POST (with EPI_MINMAX): the CTA carries one more warp that runs the second pass of the min-max
-// log-mel features -- (x - min) / max(max - min, 1e-8), log(. + 1e-8), data_utils.py:37-55 -- on every
-// clip as soon as its last tile is written, in kPostParts pieces handed out by a global ticket.  The
-// separate k_logmel_post launch (31 us behind a 173 us k_fused at 256 clips) disappears: the post
-// warps run in issue slots and L2 bandwidth the feature warps leave idle.
-constexpr int EPI_POST = 8;
-#ifndef IRIS_POST_PARTS
-#define IRIS_POST_PARTS 64   // 6.3 KB of a 400 KB clip per item: one round of 13 loads per lane (16 parts: 8-12 us per item in the tail)
-#endif
-#ifndef IRIS_POST_UNROLL
-#define IRIS_POST_UNROLL 13
-#endif
-#ifndef IRIS_POST_SLEEP
-#define IRIS_POST_SLEEP 1000
-#endif
-constexpr int kPostParts = IRIS_POST_PARTS;
-constexpr int kPostUnroll = IRIS_POST_UNROLL;
-#ifndef IRIS_FIX_FR
-#define IRIS_FIX_FR 8   // frames per tile of the fixed mel variants (experiment builds: 9 = 10 warps per CTA)
-#endif
+constexpr int kFixFR = 8;   // frames per tile of the fixed mel variants
 __host__ __device__ constexpr int fixed_mel_L(int r) { return r == 0 ? 2 : (r == 1 ? 4 : (r == 2 ? 6 : 0)); }
 template <int MODE, int NJ, int EPI>
-__global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ FusedParams p) {
+__global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParams p) {
     extern __shared__ __align__(128) unsigned char sm[];
     // per-clip extrema of the CTA: {~bits(min), bits(max), warps arrived, -} per run of tiles of one
     // clip; the consumer warps are never more than S <= 3 tiles apart, 8 entries never collide
     __shared__ uint32_t s_mm[8][4];
-    // kPost: {clip, tiles} of the run in entry r & 7, the generation of every entry (bumped by the post
-    // warp when it has published the run and the entry may be reused) and the consumer warps that have
-    // left the tile loop
-    __shared__ uint32_t s_run[8][2];
-    __shared__ uint32_t s_gen[8];
-    __shared__ uint32_t s_exit;
     constexpr bool kMel = (MODE == FM_MEL);
     constexpr bool kFix = (EPI != 0);      // switches below are compile-time constants
     static_assert(!kFix || kMel, "fixed epilogues exist for the mel modes only");
     constexpr int S = slots_of(MODE);      // stage buffers
-    constexpr bool kPost = kFix && (EPI & EPI_POST) && (EPI & EPI_MINMAX);
     const bool do_minmax = kFix ? bool(EPI & EPI_MINMAX) : (p.do_minmax != 0);
     const bool do_lg = kFix ? bool(EPI & EPI_LOG) : (p.do_log && !p.do_minmax);
     const int C = kFix ? 2 : p.C;
@@ -249,12 +188,11 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
     const int warp = tid >> 5, lane = tid & 31;
     // fixed variants: 8 frames per tile and the 12 taps of the default mel shape, so that the
     // shared-memory map folds into immediates
-    if (tid == 0) { IRIS_TR(0, tr_gtimer()); IRIS_TRC(1); }
-    const int FR = kFix ? IRIS_FIX_FR : p.fr;
+    const int FR = kFix ? kFixFR : p.fr;
     const int mel_taps = kFix ? (fixed_mel_L(0) + fixed_mel_L(1) + fixed_mel_L(2)) : p.mel_taps;
     uint64_t* full = reinterpret_cast<uint64_t*>(sm + OFF_FULL);
     uint64_t* empty = reinterpret_cast<uint64_t*>(sm + OFF_EMPTY);
-    const int n_tiles = p.tile_count;   // of this launch (a batch may be split over several launches)
+    const int n_tiles = p.B * ((p.T + FR - 1) / FR) * p.n_pairs;   // of the whole batch
     const uint32_t slotB = slot_bytes(FR);
     unsigned char* slots = sm + off_slots(mel_taps, FR);
 
@@ -266,7 +204,7 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         return iris::claim_range(CH, CM, CT, n_big, n_mid, q, len);
     };
     auto load_block = [&](int tile) -> int4 {
-        const unsigned char* blk = p.tile_blocks + size_t(tile + p.tile_first) * p.tile_stride;
+        const unsigned char* blk = p.tile_blocks + size_t(tile) * p.tile_stride;
         return lane < chunks16 ? __ldg(reinterpret_cast<const int4*>(blk) + lane) : make_int4(0, 0, 0, 0);
     };
     // the block of the CTA's first tile is requested before the setup below, not after it
@@ -287,8 +225,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         float4* z = reinterpret_cast<float4*>(slots);
         for (uint32_t i = tid; i < S * slotB / 16; i += blockDim.x) z[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         if (tid < 32) s_mm[tid >> 2][tid & 3] = 0u;
-        if (tid < 8) s_gen[tid] = 0u;
-        if (tid == 0) s_exit = 0u;
         if (tid == 0) {
             for (int s = 0; s < S; ++s) {
                 mbar_init(&full[s], 1);
@@ -299,129 +235,9 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         fence_proxy_async();   // the zero fill (generic proxy) precedes the bulk copies (async proxy)
         __syncthreads();
     }
-    if (tid == 0) IRIS_TRC(2);
     // everything above overlapped k_tiles (programmatic dependent launch); its tile blocks and the
     // zeroed extrema scratch are visible from here on
     cudaGridDependencySynchronize();
-    if (tid == 0) IRIS_TRC(3);
-
-    // ---- second pass (kPost): the post warp of the CTA from the start, the consumer warps once they
-    // have run out of tiles ----
-    // Runs of tiles of one clip that the FR consumer warps of this CTA have all finished are published
-    // by the POST warp: it sends the run's extrema to the global scratch and, behind ONE device-scope
-    // fence, adds its tiles to the clip's count.  (With the fence in the consumer warp that arrived last
-    // the kernel took 204 us instead of 173: the warp stalls on the fence and the stage ring stalls
-    // with it.)  Only lane 0 of the post warp calls this.
-    uint32_t run_tail = 0;
-    auto service_runs = [&]() {
-        while (true) {
-            uint32_t* sl = s_mm[run_tail & 7];
-            if (*reinterpret_cast<volatile uint32_t*>(&sl[2]) != uint32_t(FR)) break;
-            __threadfence_block();
-            const uint32_t a = *reinterpret_cast<volatile uint32_t*>(&sl[0]);
-            const uint32_t c = *reinterpret_cast<volatile uint32_t*>(&sl[1]);
-            const uint32_t clip = *reinterpret_cast<volatile uint32_t*>(&s_run[run_tail & 7][0]);
-            const uint32_t tiles = *reinterpret_cast<volatile uint32_t*>(&s_run[run_tail & 7][1]);
-            *reinterpret_cast<volatile uint32_t*>(&sl[0]) = 0u;
-            *reinterpret_cast<volatile uint32_t*>(&sl[1]) = 0u;
-            *reinterpret_cast<volatile uint32_t*>(&sl[2]) = 0u;
-            __threadfence_block();
-            *reinterpret_cast<volatile uint32_t*>(&s_gen[run_tail & 7]) = (run_tail >> 3) + 1u;   // entry free for run + 8
-            red_max_u32_if(&p.minmax[2 * clip], a, (a | c) != 0u);
-            red_max_u32_if(&p.minmax[2 * clip + 1], c, (a | c) != 0u);
-            __threadfence();
-            atomicAdd(&p.clip_done[clip], tiles);
-            ++run_tail;
-        }
-    };
-    // own_runs: the caller is the post warp (it also publishes the runs of its CTA while it waits and works)
-    auto post_loop = [&](const bool own_runs) {
-        // items = (clip, part) in clip order; a clip is whole when clip_done reaches its tile count
-        const uint32_t tpc = uint32_t((p.T + FR - 1) / FR) * uint32_t(p.n_pairs);
-        const size_t clip_elems = size_t(p.n_mel) * p.T * C;
-        const uint32_t n4 = uint32_t(clip_elems >> 2);   // float4 per clip (the launcher checks clip_elems % 4 == 0)
-        const uint32_t n_items = uint32_t(p.B) * kPostParts;
-#ifdef IRIS_TRACE
-        long long pw = 0, pp = 0, pn = 0, pt0 = clock64();
-#endif
-        while (true) {
-            uint32_t t = 0;
-            if (lane == 0) {
-                if (own_runs) service_runs();
-                t = atomicAdd(&p.sched[2], 1u);
-            }
-            t = __shfl_sync(0xffffffffu, t, 0);
-            if (t >= n_items) break;
-            const uint32_t b = t / kPostParts, part = t - b * kPostParts;
-#ifdef IRIS_TRACE
-            const long long q0 = clock64();
-#endif
-            if (lane == 0)
-                while (ld_acquire_gpu_u32(&p.clip_done[b]) < tpc) {
-                    if (own_runs) service_runs();   // (the clip may be waiting for a run of this very CTA)
-                    __nanosleep(IRIS_POST_SLEEP);
-                }
-            __syncwarp();
-#ifdef IRIS_TRACE
-            const long long q1 = clock64();
-            pw += q1 - q0;
-#endif
-            const float mn = __uint_as_float(~__ldcg(&p.minmax[2 * b]));
-            const float mx = __uint_as_float(__ldcg(&p.minmax[2 * b + 1]));
-            const float inv = 1.f / fmaxf(mx - mn, 1e-8f);
-            float4* v = reinterpret_cast<float4*>(p.out + size_t(b) * clip_elems);
-            const uint32_t lo = uint32_t((uint64_t(n4) * part) / kPostParts);
-            const uint32_t hi = uint32_t((uint64_t(n4) * (part + 1)) / kPostParts);
-            for (uint32_t i0 = lo + lane; i0 < hi; i0 += 32 * kPostUnroll) {
-                float4 a[kPostUnroll];
-#pragma unroll
-                for (int u = 0; u < kPostUnroll; ++u)
-                    if (i0 + 32 * u < hi) a[u] = __ldcg(v + i0 + 32 * u);
-#pragma unroll
-                for (int u = 0; u < kPostUnroll; ++u)
-                    if (i0 + 32 * u < hi) {
-                        // same arithmetic as k_logmel_post (k_post.cu): x - min first
-                        a[u].x = __logf(fmaf(a[u].x - mn, inv, 1e-8f));
-                        a[u].y = __logf(fmaf(a[u].y - mn, inv, 1e-8f));
-                        a[u].z = __logf(fmaf(a[u].z - mn, inv, 1e-8f));
-                        a[u].w = __logf(fmaf(a[u].w - mn, inv, 1e-8f));
-                        v[i0 + 32 * u] = a[u];
-                    }
-                if (own_runs && lane == 0) service_runs();
-            }
-            __syncwarp();
-#ifdef IRIS_TRACE
-            pp += clock64() - q1;
-            ++pn;
-#endif
-            // the last part of a clip leaves its scratch zeroed for the next launch
-            if (lane == 0 && atomicAdd(&p.post_parts[b], 1u) == kPostParts - 1) {
-                p.minmax[2 * b] = 0u;
-                p.minmax[2 * b + 1] = 0u;
-                p.clip_done[b] = 0u;
-                p.post_parts[b] = 0u;
-            }
-        }
-#ifdef IRIS_TRACE
-        if (lane == 0 && warp == FR + 1) { IRIS_TR(60, pw); IRIS_TR(61, pp); IRIS_TR(62, pn); IRIS_TR(63, clock64() - pt0); }
-        if (lane == 0 && warp == 0) { IRIS_TR(15, pn); IRIS_TR(12, pp); IRIS_TR(13, pw); }
-#endif
-        if (own_runs) {   // the consumer warps may still be at their last tiles: publish until all have left
-            if (lane == 0) {
-                while (*reinterpret_cast<volatile uint32_t*>(&s_exit) != uint32_t(FR)) {
-                    service_runs();
-                    __nanosleep(64);
-                }
-                __threadfence_block();
-                service_runs();
-            }
-            __syncwarp();
-        }
-        if (lane == 0 && atomicAdd(&p.sched[3], 1u) == gridDim.x * uint32_t(FR + 1) - 1u) {   // last warp of the grid
-            p.sched[2] = 0u;
-            p.sched[3] = 0u;
-        }
-    };
 
     if (warp == FR) {
         // =========================== producer warp ===========================
@@ -439,7 +255,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         // chunk.  Consecutive tiles of a clip mostly stay on one SM (per-clip state changes rarely,
         // the row shared by two tiles is re-read one tile later).
         int i = 0;
-        if (lane == 0) IRIS_TRC(4);
         if (first < n_tiles) {
             int tile = int(first);
             int last = int(min((long long)n_tiles, first + len));
@@ -450,16 +265,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 __syncwarp();
                 const int n = __shfl_sync(0xffffffffu, c.x, 0);
                 const TileBlock* tb = reinterpret_cast<const TileBlock*>(ent);
-#ifdef IRIS_L2_PREFETCH   // measured on B200: cfg2 mel -1 us, cfg1 +2 us, min-max log-mel step +1.6 us (the prefetched lines compete with the mel rows kept for k_logmel_post): off
-                // The stages of this tile go out as stage buffers fall free, the later ones of a
-                // tile with more than S stages only one release + one DRAM round trip at a time:
-                // lane 2 + s holds StageDesc s of the block and asks L2 for its span right away.
-                {
-                    const uint32_t cnt = uint32_t(c.z) >> 16;   // StageDesc: {src.lo, src.hi, j_lo | j_cnt << 16, gain}
-                    const void* src = reinterpret_cast<const void*>((uint64_t(uint32_t(c.y)) << 32) | uint32_t(c.x));
-                    bulk_prefetch_l2_if(src, (cnt + 1u) * 2048u, lane >= 2 && lane < 2 + n && cnt != 0u);
-                }
-#endif
                 // look ahead: the block of the next tile of this claim is fetched while the stages of
                 // this one are issued; at the last tile of a claim the next claim goes out instead
                 const bool more = tile + 1 < last;
@@ -478,11 +283,7 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                         } else {
                             const uint32_t bytes = (uint32_t(d.j_cnt) + 1u) * 2048u;
                             mbar_arrive_expect_tx(&full[slot], bytes);
-                            if (p.l2_hints)
-                                bulk_g2s_hint(slots + slot * slotB + uint32_t(d.j_lo) * 2048u, d.src, bytes, &full[slot], pol_stream);
-                            else
-                                bulk_g2s(slots + slot * slotB + uint32_t(d.j_lo) * 2048u, d.src, bytes, &full[slot]);
-                            if (i == 0 && s == 0) IRIS_TRC(5);
+                            bulk_g2s_hint(slots + slot * slotB + uint32_t(d.j_lo) * 2048u, d.src, bytes, &full[slot], pol_stream);
                         }
                     }
                     if (++slot == S) { slot = 0; phase ^= 1u; }
@@ -504,7 +305,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         // no work left to claim: a kernel launched behind this one with programmatic stream
         // serialization (k_logmel_post) may be scheduled; it still waits for the whole grid
         cudaTriggerProgrammaticLaunchCompletion();
-        if (lane == 0) { IRIS_TRC(11); IRIS_TR(9, i); }
         // end marker: a TileBlock with n == 0 behind one more (empty) stage
         {
             unsigned char* ent = sm + OFF_RING + (i & (kRing - 1)) * kTileBlockBytes;
@@ -520,8 +320,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 }
             }
         }
-    } else if (kPost && warp == FR + 1) {
-        post_loop(true);
     } else {
         // =========================== consumer warps ===========================
         {
@@ -558,7 +356,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
         float mn = __int_as_float(0x7f800000), mx = 0.f;
         int mm_clip = -1;
         uint32_t mm_run = 0;   // runs of tiles of one clip this warp has flushed (the same sequence in every warp)
-        uint32_t mm_tiles = 0; // tiles of the current run (kPost)
         // The extrema of a run are combined in shared memory; the last of the FR warps to arrive sends
         // the CTA's pair to the global scratch.  (One red.global pair per WARP and clip change --
         // 81 k per 256-clip launch on 512 addresses -- measured 4 us of the kernel.)
@@ -568,23 +365,14 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
                 mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
             }
-            __syncwarp();   // (kPost: the feature stores of all lanes are ordered before lane 0's fences)
             if (lane == 0) {
                 uint32_t* sl = s_mm[mm_run & 7];
-                if (kPost) {
-                    // the entry is free once the post warp has published the run that used it 8 runs ago
-                    // (it always has, unless the post warp fell far behind)
-                    while (*reinterpret_cast<volatile uint32_t*>(&s_gen[mm_run & 7]) != (mm_run >> 3)) __nanosleep(32);
-                    __threadfence_block();
-                    *reinterpret_cast<volatile uint32_t*>(&s_run[mm_run & 7][0]) = uint32_t(mm_clip);   // (the same
-                    *reinterpret_cast<volatile uint32_t*>(&s_run[mm_run & 7][1]) = mm_tiles;            // in every warp)
-                }
                 if (mn <= mx) {
                     atomicMax(&sl[0], ~__float_as_uint(mn));
                     atomicMax(&sl[1], __float_as_uint(mx));
                 }
                 __threadfence_block();
-                if (atomicAdd(&sl[2], 1u) == uint32_t(FR) - 1u && !kPost) {
+                if (atomicAdd(&sl[2], 1u) == uint32_t(FR) - 1u) {
                     __threadfence_block();
                     const uint32_t a = *reinterpret_cast<volatile uint32_t*>(&sl[0]);
                     const uint32_t c = *reinterpret_cast<volatile uint32_t*>(&sl[1]);
@@ -597,41 +385,24 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
             }
             __syncwarp();
             ++mm_run;
-            mm_tiles = 0;
             mn = __int_as_float(0x7f800000);
             mx = 0.f;
         };
 
         uint32_t slot = 0, phase = 0;
         const uint64_t pol_keep = l2_policy_evict_last();
-        // mel rows are re-read by k_logmel_post: ask L2 to keep them (fixed variants: hints are on; a
-        // 256-clip batch does not fit anyway, but the hint measures 4-8 us better than plain stores)
-        const bool keep_l2 = kFix ? bool(EPI & EPI_MINMAX) : (kMel && p.l2_hints && do_minmax);
+        // mel rows are re-read by k_logmel_post: ask L2 to keep them (a 256-clip batch does not fit
+        // anyway, but the hint measures 4-8 us better than plain stores)
+        const bool keep_l2 = kMel && do_minmax;
         float* clip_out = p.out;      // out[b, 0, 0, 0] of the current clip (mel modes)
         uint32_t zbits = 0;
         int zb_clip = -1;
         const size_t clip_elems = size_t(p.n_mel) * p.T * C;
-#ifdef IRIS_TRACE
-        // where the time of a consumer warp goes (clock64 sums over its tiles): wait for the first
-        // stage of a tile, waits for the later stages, mix, FFT, epilogue
-        long long a_w0 = 0, a_w1 = 0, a_mix = 0, a_fft = 0, a_epi = 0, a_st = 0, c0, c1, c2, c3, c4 = 0;
-#define IRIS_ACC(dst, from, to) dst += (to) - (from)
-#else
-#define IRIS_ACC(dst, from, to) do { } while (0)
-#endif
         for (int i = 0;; ++i) {
             const TileBlock* tb = reinterpret_cast<const TileBlock*>(sm + OFF_RING + (i & (kRing - 1)) * kTileBlockBytes);
             // ---- gather + mix: v = sum over the stages of this tile of gain * frame ----
             cpx v[16];
-#ifdef IRIS_TRACE
-            c0 = clock64();
-            if (i > 0) IRIS_ACC(a_epi, c4, c0);
-#endif
             mbar_wait_parked(&full[slot], phase);           // also publishes the TileBlock of this tile
-#ifdef IRIS_TRACE
-            c1 = clock64();
-            IRIS_ACC(a_w0, c0, c1);
-#endif
             // the rows of the first stage are requested before the tile header is looked at (the end
             // marker's rows are stale but finite): the header's load-to-use latency hides behind them
             {
@@ -644,12 +415,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
             }
             const int4 hdr = *reinterpret_cast<const int4*>(tb);
             const int n_st = hdr.x;
-            if (i == 0 && tid == 0) IRIS_TRC(6);
-#ifdef IRIS_TRACE
-            if (tid == 0 && i > 0 && (i & 1) == 0 && (i >> 1) < 32) IRIS_TRC(16 + (i >> 1));   // tiles 0 .. i-1 done
-            if (tid == 0 && i == 1) IRIS_TRC(7);
-            if (tid == 0 && i == 21) IRIS_TRC(12);
-#endif
             if (n_st == 0) break;                    // end marker
             // (skipping the row reads of time-masked frames -- ~11 % of the frames -- was measured on
             // B200: +2..5 % kernel time; the extra branch costs registers (93 -> 96 + a spill) and the
@@ -665,14 +430,7 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 if (++slot == S) { slot = 0; phase ^= 1u; }
             }
             for (int e = 1; e < n_st; ++e) {
-#ifdef IRIS_TRACE
-                c2 = clock64();
-#endif
                 mbar_wait_parked(&full[slot], phase);
-#ifdef IRIS_TRACE
-                c3 = clock64();
-                IRIS_ACC(a_w1, c2, c3);
-#endif
                 const uint2 dd = *reinterpret_cast<const uint2*>(&tb->d[e].j_lo);
                 const bool active = unsigned(j - int(dd.x & 0xffffu)) < (dd.x >> 16);
                 if (active) {
@@ -689,12 +447,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 if (++slot == S) { slot = 0; phase ^= 1u; }
             }
 
-            if (tid == 0 && i == 21) IRIS_TRC(13);   // mix of tile 21 done
-#ifdef IRIS_TRACE
-            c2 = clock64();
-            IRIS_ACC(a_mix, c1, c2);
-            a_st += n_st;
-#endif
             const int b = hdr.y;
             const int pair = kFix ? 0 : (hdr.z >> 24);
             const int t = (hdr.z & 0xffffff) + j;
@@ -767,11 +519,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                 __syncwarp();   // every lane is done with the exchange rows (reused for |X| below)
             }
 
-            if (tid == 0 && i == 21) IRIS_TRC(14);   // FFT of tile 21 done
-#ifdef IRIS_TRACE
-            c4 = clock64();
-            IRIS_ACC(a_fft, c2, c4);
-#endif
             // ---- epilogue ----
             // register jj holds bin f = k1 + 16 (2 jj + par); its mirror 512 - f is register
             // 15 - jj of the partner lane (lane 0: its own register (16 - jj) & 15)
@@ -784,7 +531,6 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
                     if (mm_clip >= 0) flush_minmax();
                     mm_clip = b;
                 }
-                if (kPost) ++mm_tiles;
                 // (|ch0|, |ch1|) of every bin the lane holds, indexed by the bin itself (at most 257 x 8 B
                 // of the warp's 4352-byte exchange rows): no range checks on the way in
                 float2* mg = reinterpret_cast<float2*>(xch);
@@ -958,38 +704,7 @@ __global__ void __maxnreg__(IRIS_MAX_REGS) k_fused(const __grid_constant__ Fused
             }
         }
         if (kMel && do_minmax && mm_clip >= 0) flush_minmax();
-        if (tid == 0) { IRIS_TRC(8); IRIS_TR(10, tr_gtimer()); }
-        if (kPost) {   // out of tiles: help with the clips that are still to be normalised
-            __syncwarp();
-            if (lane == 0) {
-                __threadfence_block();
-                atomicAdd(&s_exit, 1u);
-            }
-            post_loop(false);
-        }
-#ifdef IRIS_TRACE
-        if (lane == 0 && (warp == 0 || warp == 5)) {
-            const int o = warp == 0 ? 48 : 54;
-            IRIS_TR(o, a_w0); IRIS_TR(o + 1, a_w1); IRIS_TR(o + 2, a_mix); IRIS_TR(o + 3, a_fft);
-            IRIS_TR(o + 4, a_epi); IRIS_TR(o + 5, a_st);
-        }
-#endif
     }
-}
-
-// the second pass runs inside k_fused for the fixed 2-channel min-max instance (launch_fused picks it
-// under the same conditions) when a clip is a whole number of float4
-bool fused_can_post_in_kernel(const FusedParams& p) {
-    // Opt-in (IRIS_POST_IN_KERNEL=1).  Measured on B200, cfg2, 256 clips (profiles/r02_post_in_kernel.txt):
-    // the kernel grows from 173 to 196 us (run publishing +7, tickets and waits +5, the loads +5,
-    // arithmetic and stores +5 us) while k_logmel_post alone takes 29 us and hides the metric leg
-    // (10 us) behind it: the step is 231 us either way, so the separate pass stays the default.
-    static const bool on = getenv("IRIS_POST_IN_KERNEL") && atoi(getenv("IRIS_POST_IN_KERNEL")) != 0;
-    if (!on || getenv("IRIS_NO_FIXED_EPI")) return false;
-    return p.do_minmax && p.C == 2 && p.mel_f_lo + p.mel_f_n <= 128 && p.mel_L[0] == fixed_mel_L(0) &&
-           p.mel_L[1] == fixed_mel_L(1) && p.mel_L[2] == fixed_mel_L(2) && p.mel_L[3] == fixed_mel_L(3) &&
-           p.l2_hints && p.fr == IRIS_FIX_FR && p.mel_taps == 12 && ((size_t(p.n_mel) * p.T * p.C) & 3) == 0 &&
-           p.tile_first == 0 && p.tile_count == 0;
 }
 
 size_t fused_smem_bytes(const FusedParams& p, int mode) { return smem_total(p.mel_taps, p.fr, mode, p.stage_out != 0); }
@@ -1002,15 +717,10 @@ int fused_max_frames_per_tile() { return kMaxFR; }
 // Frames per tile = consumer warps per CTA.  FR = 8 (two CTAs of 8 + 1 warps per SM: the
 // consumer warps spread evenly over the 4 schedulers and two independent CTAs hide each
 // other's load waits) measured fastest on B200: cfg2 mel 216 us vs 228 us for FR = 16 x 1 CTA
-// and 271 us for FR = 20 at 80 registers (spills).  IRIS_FR overrides it for experiments.
-int fused_pick_fr(int T, int mel_taps) {
-    int want = mel_taps > 0 ? IRIS_FIX_FR : 8;
-    if (const char* e = getenv("IRIS_FR")) {
-        const int v = atoi(e);
-        if (v >= 1 && v <= kMaxFR) want = v;
-    }
+// and 271 us for FR = 20 at 80 registers (spills).
+int fused_pick_fr(int mel_taps) {
+    int want = kFixFR;
     while (want > 1 && smem_total(mel_taps, want, FM_MEL, false) > 227u * 1024u - 256u) --want;
-    (void)T;
     return want;
 }
 
@@ -1023,22 +733,13 @@ size_t fused_tile_bytes(const FusedParams& p, int* stride_out) {
     return size_t(n_tiles) * size_t(stride);
 }
 
-// p.tile_blocks (fused_tile_bytes) is provided by the caller.  what: FUSED_LAUNCH_TILES builds the tile
-// blocks of the whole batch (k_tiles), FUSED_LAUNCH_KERNEL runs k_fused on the tiles
-// [p.tile_first, p.tile_first + p.tile_count) (tile_count 0: all of them).
 // Claim schedule of a launch (see the producer warp): whole chunks first, then half chunks for the
 // last kTailMid tiles per CTA, single tiles (tile pairs of a 4-channel clip) for the last kTailOne.
 // Measured on B200 (profiles/r02_trace_*.txt): with whole chunks to the end the CTAs of a 256-clip
 // launch finish 22 us apart (the slower of the two CTAs of an SM needs ~13 us for a chunk of 4 and
 // used to own a second one).
+constexpr int kTailOne = 2, kTailMid = 6;
 static void fused_schedule(FusedParams& p, long long n_tiles, int grid) {
-    static int t_one = -1, t_mid = -1;
-    if (t_one < 0) {
-        const char* e1 = getenv("IRIS_TAIL1");
-        const char* e2 = getenv("IRIS_TAIL2");
-        t_one = e1 ? atoi(e1) : 2;
-        t_mid = e2 ? atoi(e2) : 6;
-    }
     const int unit = p.pair_merge ? 2 : 1;   // both channel pairs of a (clip, time) range in one claim
     p.chunk_tail = unit;
     p.chunk_mid = (p.chunk / 2) / unit * unit;
@@ -1049,7 +750,7 @@ static void fused_schedule(FusedParams& p, long long n_tiles, int grid) {
         p.n_mid = 0;
         return;
     }
-    const long long tail_one = (long long)grid * t_one, tail_mid = (long long)grid * t_mid;
+    const long long tail_one = (long long)grid * kTailOne, tail_mid = (long long)grid * kTailMid;
     const long long rem = n_tiles > tail_one ? n_tiles - tail_one : 0;
     const long long mid = rem < tail_mid ? rem : tail_mid;
     p.n_big = int32_t((rem - mid) / p.chunk);
@@ -1067,69 +768,22 @@ void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge
     out[0] = p.chunk; out[1] = p.chunk_mid; out[2] = p.chunk_tail; out[3] = p.n_big; out[4] = p.n_mid;
 }
 
-#ifdef IRIS_TRACE
-// the stamps of the last launch go to $IRIS_TRACE_FILE as raw uint64 [grid + 1][64]
-static unsigned long long* g_trace_buf = nullptr;
-static size_t g_trace_cap = 0;
-static int g_trace_grid = 0;
-static void trace_begin(FusedParams& p, int num_sms, cudaStream_t stream) {
-    p.trace = nullptr;
-    p.trace_grid = 0;
-    if (!getenv("IRIS_TRACE_FILE")) return;
-    const size_t need = size_t(num_sms * 4 + 1) * 64 * 8;
-    if (g_trace_cap < need) {
-        cudaFree(g_trace_buf);
-        cudaMalloc(&g_trace_buf, need);
-        g_trace_cap = need;
-    }
-    cudaMemsetAsync(g_trace_buf, 0, need, stream);
-    p.trace = g_trace_buf;
-    p.trace_grid = num_sms * 4;   // row of the k_tiles stamp
-    g_trace_grid = num_sms * 4;
-}
-static void trace_end(int grid, cudaStream_t stream) {
-    const char* f = getenv("IRIS_TRACE_FILE");
-    if (!f || !g_trace_buf) return;
-    cudaStreamSynchronize(stream);
-    (void)grid;
-    const size_t n = size_t(g_trace_grid + 1) * 64;
-    unsigned long long* h = static_cast<unsigned long long*>(malloc(n * 8));
-    cudaMemcpy(h, g_trace_buf, n * 8, cudaMemcpyDeviceToHost);
-    if (FILE* fp = fopen(f, "wb")) {
-        fwrite(h, 8, n, fp);
-        fclose(fp);
-    }
-    free(h);
-}
-#define IRIS_TRACE_BEGIN(grid)
-#define IRIS_TRACE_END(grid) trace_end(grid, stream);
-#else
-#define IRIS_TRACE_BEGIN(grid)
-#define IRIS_TRACE_END(grid)
-#endif
-
-cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStream_t stream, int what) {
+// p.tile_blocks (fused_tile_bytes) is provided by the caller; build_tiles: k_tiles builds them first
+// (otherwise the kernel in front -- k_labels -- has built them and triggers early)
+cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStream_t stream, bool build_tiles) {
     FusedParams p = p_in;
     const int FR = p.fr;
     if (FR < 1 || FR > kMaxFR) return cudaErrorInvalidValue;
     const int tpc = (p.T + FR - 1) / FR;
-    const long long all_tiles = (long long)p.B * p.n_pairs * tpc;
-    if (all_tiles <= 0) return cudaSuccess;
-    if (p.tile_count == 0) { p.tile_first = 0; p.tile_count = int32_t(all_tiles); }
-    const long long n_tiles = p.tile_count;
-    if (p.tile_first < 0 || p.tile_first + n_tiles > all_tiles) return cudaErrorInvalidValue;
-    if (all_tiles > 0x7fffffffLL || p.max_segs > kMaxStages || p.n_pairs > 127) return cudaErrorInvalidValue;
+    const long long n_tiles = (long long)p.B * p.n_pairs * tpc;
+    if (n_tiles <= 0) return cudaSuccess;
+    if (n_tiles > 0x7fffffffLL || p.max_segs > kMaxStages || p.n_pairs > 127) return cudaErrorInvalidValue;
     if (mode == FM_MEL && (long long)p.n_mel * p.T * p.C > 0x7fffffffLL) return cudaErrorInvalidValue;   // 32-bit row offsets inside a clip
     const size_t smem = fused_smem_bytes(p, mode);
     if (smem > 227 * 1024 - 256) return cudaErrorInvalidValue;   // (128 B of static shared memory: s_mm)
-#ifdef IRIS_TRACE
-    trace_begin(p, num_sms, stream);
-#endif
-    if (what & FUSED_LAUNCH_TILES) k_tiles<<<unsigned((all_tiles + 127) / 128), 128, 0, stream>>>(p);
-    if (!(what & FUSED_LAUNCH_KERNEL)) return cudaGetLastError();
-    // programmatic dependent launch behind k_tiles of the same call (prologue overlap); a launch on
-    // its own (later part of a split batch) is an ordinary one
-    const int pdl = (what & (FUSED_LAUNCH_TILES | FUSED_LAUNCH_PDL)) && !getenv("IRIS_NO_PDL") ? 1 : 0;
+    if (build_tiles) k_tiles<<<unsigned((n_tiles + 127) / 128), 128, 0, stream>>>(p);
+    // k_fused is a programmatic dependent launch behind k_tiles / k_labels: its prologue overlaps
+    // their tail
     int dev = 0;
     cudaGetDevice(&dev);
     // persistent grid: as many CTAs as are resident at once, asked of the occupancy calculator once
@@ -1138,7 +792,7 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     // registers are granted per warp in larger units) -- 4-ch COMPLEX 570 -> 730 us, mel 200 -> 265 us.
 #define IRIS_LAUNCH(M, NJV, EPIV)                                                                     \
     {                                                                                           \
-        const int threads = (FR + 1 + (((EPIV) & EPI_POST) ? 1 : 0)) * 32;                      \
+        const int threads = (FR + 1) * 32;                                                      \
         static int attr_dev = -1;   /* function attributes are per device */                    \
         static int per_sm = 1;                                                                  \
         static size_t per_sm_smem = 0;                                                          \
@@ -1162,9 +816,6 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
             if (e != cudaSuccess) return e;                                                     \
             per_sm = nb < 1 ? 1 : nb;                                                           \
             per_sm_smem = smem;                                                                 \
-            if (getenv("IRIS_VERBOSE"))                                                         \
-                fprintf(stderr, "k_fused<%d,%d,%d>: %d CTAs/SM (%zu B smem, %d threads)\n",     \
-                        int(M), NJV, EPIV, per_sm, smem, threads);                              \
         }                                                                                       \
         const long long max_ctas = (long long)num_sms * per_sm;                                 \
         const int grid = int(n_tiles < max_ctas ? n_tiles : max_ctas);                          \
@@ -1176,13 +827,11 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         cfg.stream = stream;                                                                    \
         cudaLaunchAttribute attr[1];                                                            \
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                        \
-        attr[0].val.programmaticStreamSerializationAllowed = pdl;                               \
+        attr[0].val.programmaticStreamSerializationAllowed = 1;                                 \
         cfg.attrs = attr;                                                                       \
         cfg.numAttrs = 1;                                                                       \
-        IRIS_TRACE_BEGIN(grid)                                                                  \
         cudaError_t le = cudaLaunchKernelEx(&cfg, k_fused<M, NJV, EPIV>, p);                    \
         if (le != cudaSuccess) return le;                                                       \
-        IRIS_TRACE_END(grid)                                                                    \
     }
     switch (mode) {
         case FM_COMPLEX: IRIS_LAUNCH(FM_COMPLEX, 8, 0) break;
@@ -1192,9 +841,8 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
             if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH(FM_MEL, 8, 0)
             else if (p.C != 2 || p.mel_L[0] != fixed_mel_L(0) || p.mel_L[1] != fixed_mel_L(1) ||
                      p.mel_L[2] != fixed_mel_L(2) || p.mel_L[3] != fixed_mel_L(3) ||
-                     !p.l2_hints || FR != IRIS_FIX_FR || p.mel_taps != 12 || getenv("IRIS_NO_FIXED_EPI"))
+                     FR != kFixFR || p.mel_taps != 12 || getenv("IRIS_NO_FIXED_EPI"))
                 IRIS_LAUNCH(FM_MEL, 4, 0)
-            else if (p.do_minmax && p.post_in_kernel) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX | EPI_POST)
             else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX)
             else if (p.do_log) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_LOG)
             else IRIS_LAUNCH(FM_MEL, 4, EPI_C2)

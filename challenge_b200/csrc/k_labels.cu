@@ -4,7 +4,6 @@
 // activity flags (activity = reduce_max(voice, (f, 2C)) > 0, pipeline.py:55).
 // One CTA per clip; voices are visited in order because acceptance of voice v depends
 // on the labels of the voices accepted before it (pipeline.py:78-84).
-#include <cstdlib>
 #include <cstring>
 
 #include "iris_common.cuh"
@@ -143,11 +142,7 @@ cudaError_t launch_labels(const LabelParams& p, cudaStream_t stream, const Fused
     // one wave of clips (two 1024-thread CTAs per SM): one frame per thread is fastest; larger batches run in
     // several waves and the kernel is latency-bound per CTA, so half-size CTAs (four per SM) finish sooner
     // (1024 clips: step 0.82 -> 0.81 ms; 256 clips: 226.3 vs 226.7 us)
-    int threads = p.B > 296 ? 512 : 1024;
-    if (const char* e = getenv("IRIS_LABEL_THREADS")) {
-        const int v = atoi(e);
-        if (v >= 64 && v <= 1024 && v % 32 == 0) threads = v;
-    }
+    const int threads = p.B > 296 ? 512 : 1024;
     k_labels<<<p.B, threads, smem, stream>>>(p, tiles ? 1 : 0, tiles ? *tiles : none);
     return cudaGetLastError();
 }

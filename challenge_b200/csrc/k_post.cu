@@ -8,7 +8,6 @@
 //   y = log((x - min) / max(max - min, 1e-8) + 1e-8)
 // is evaluated as log2((x - min) * inv + 1e-8) * ln2 with inv = 1 / max(max - min, 1e-8):
 // FADD, FFMA, MUFU.LG2, FMUL per element.
-#include <cstdlib>
 
 #include "iris_common.cuh"
 #include "iris_launch.h"
@@ -86,7 +85,7 @@ cudaError_t launch_logmel_post(float* x, uint32_t* minmax, unsigned* done, int B
         cfg.stream = stream;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = getenv("IRIS_NO_PDL") ? 0 : 1;
+        attr[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = attr;
         cfg.numAttrs = 1;
         cudaError_t e = cudaLaunchKernelEx(&cfg, k_logmel_post, x + size_t(b0) * per_clip,

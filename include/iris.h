@@ -186,9 +186,7 @@ int iris_debug_claims(int64_t n_tiles, int grid, int chunk, int pair_merge, int6
  * iris_profile_read() synchronises them and returns the summed device time. */
 int iris_profile_enable(iris_ctx* ctx, int enable);
 int iris_profile_read(iris_ctx* ctx, double* total_ms, int32_t* n_launches, int reset);
-/* Clips of the launch the hook timed last: the whole batch, or -- when a large min-max log-mel
- * batch is split into parts whose second pass overlaps the next part's feature kernel -- the
- * first part (the one launch whose start and end are not entangled with another kernel). */
+/* Clips of the launch the hook timed last (the whole batch of that feature launch). */
 int iris_profile_clips(iris_ctx* ctx);
 
 /* ---------------------------------------------------------------------------------------

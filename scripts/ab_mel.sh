@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B of k_fused builds on one box: scripts/kb_mel.py for every variant given as
 # name=path[,ENV=VALUE...] (default build when path is empty), interleaved three times.
-# usage: scripts/ab_mel.sh nok1=gpurun_scratch/nok1/libiris.so natural=,IRIS_MEL_NATURAL=1 new=
+# usage: scripts/ab_mel.sh old=challenge_b200/build_old/libiris.so generic=,IRIS_NO_FIXED_EPI=1 new=
 mkdir -p gpurun_out
 : > gpurun_out/ab_mel.log
 for rep in 1 2 3; do

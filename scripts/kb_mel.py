@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Times iris_features(MEL / LOGMEL_MINMAX) for cfg1 / cfg2 at C=2, B=256 (experiment variants via IRIS_LIB / IRIS_FR)."""
+"""Times iris_features(MEL / LOGMEL_MINMAX) for cfg1 / cfg2 at C=2, B=256 (other builds via IRIS_LIB)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -33,4 +33,4 @@ for name, d in plans.items():
         o = torch.empty(eng.feature_shape(mode), device='cuda')
         med, mn = timeit(lambda: eng.features(mode, out=o))
         out.append('%s %s %.1f/%.1f' % (name, mname, med, mn))
-print('%-28s FR=%-3s %s' % (os.path.basename(os.path.dirname(os.environ.get('IRIS_LIB') or 'x/default/l')), os.environ.get('IRIS_FR', '-'), ' | '.join(out)))
+print('%-28s %s' % (os.path.basename(os.path.dirname(os.environ.get('IRIS_LIB') or 'x/default/l')), ' | '.join(out)))

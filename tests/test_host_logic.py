@@ -200,6 +200,20 @@ def test_product_never_imports_oracle():
                 assert not re.search(r'^\s*(from|import)\s+oracle\b', src, flags=re.M), f
 
 
+def test_native_environment_switches_are_the_documented_ones():
+    """Every getenv of the native library is a switch INTEGRATION.md section 6 documents; the
+    product path takes no other run-time option."""
+    csrc = os.path.join(ROOT, 'challenge_b200', 'csrc')
+    names = set()
+    for f in os.listdir(csrc):
+        names |= set(re.findall(r'getenv\(\s*"([^"]+)"\s*\)', open(os.path.join(csrc, f)).read()))
+    assert names == {'IRIS_NCCL_LIB', 'IRIS_NO_FIXED_EPI', 'IRIS_NO_LABEL_TILES'}
+    doc = open(os.path.join(ROOT, 'INTEGRATION.md')).read()
+    section = re.search(r'^## 6\..*?(?=^## |\Z)', doc, flags=re.M | re.S).group(0)
+    for n in names:
+        assert '`%s' % n in section, n
+
+
 def test_fftcore_math_on_host(tmp_path):
     """fftcore.cuh compiled with g++: the 16-lane x 32-point decomposition, the 4-round
     exchange geometry and the lane-local two-channel split reproduce a float64 DFT."""
