@@ -15,6 +15,9 @@ BANK_BG, BANK_VOICE, BANK_NOISE = 0, 1, 2
 FEAT_COMPLEX, FEAT_MAGPHASE, FEAT_LOG_MAGPHASE, FEAT_MEL, FEAT_LOGMEL, FEAT_LOGMEL_MINMAX = range(6)
 REMAP_NONE, REMAP_STEREO_MONO, REMAP_MERGE_AUG = 0, 1, 2
 SELECT_ALL, SELECT_VOICES, SELECT_BG_NOISE = 0, 1, 2
+# output element type, OR-ed into a feature mode (none: float32)
+OUT_BF16, OUT_F16 = 0x100, 0x200
+MODE_MASK = 0xff
 
 _i32p = C.POINTER(C.c_int32)
 _f32p = C.POINTER(C.c_float)
@@ -197,6 +200,22 @@ def dlpack_pointer(capsule):
     C.pythonapi.PyCapsule_GetPointer.restype = C.c_void_p
     C.pythonapi.PyCapsule_GetPointer.argtypes = [C.py_object, C.c_char_p]
     return C.c_void_p(C.pythonapi.PyCapsule_GetPointer(capsule, b'dltensor'))
+
+
+class _DLDataType(C.Structure):
+    _fields_ = [('code', C.c_uint8), ('bits', C.c_uint8), ('lanes', C.c_uint16)]
+
+
+class _DLTensorHead(C.Structure):   # the leading fields of DLTensor (include/iris_dlpack.h)
+    _fields_ = [('data', C.c_void_p), ('device_type', C.c_int32), ('device_id', C.c_int32),
+                ('ndim', C.c_int32), ('dtype', _DLDataType)]
+
+
+def dlpack_out_flag(managed):
+    """OUT_BF16 / OUT_F16 for a bfloat16 / float16 ``DLManagedTensor*``, else 0 (the library checks
+    the dtype against the flag)."""
+    dt = _DLTensorHead.from_address(managed.value).dtype
+    return {(4, 16): OUT_BF16, (2, 16): OUT_F16}.get((dt.code, dt.bits), 0)
 
 
 def check(rc):

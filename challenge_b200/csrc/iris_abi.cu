@@ -178,10 +178,10 @@ void tile_sig_set(iris_ctx* c, const FusedParams& p) {
 
 // k_tiles + k_fused over the whole batch; k_tiles is skipped when the tile blocks of this plan
 // already exist in this layout (built by k_labels or by an earlier feature launch)
-int run_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs, cudaStream_t st) {
+int run_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs, cudaStream_t st, int out_type = OUT_F32) {
     int rc = prepare_fused(c, p, mode, max_segs);
     if (rc) return rc;
-    CU(launch_fused(p, mode, c->num_sms, st, !tile_sig_matches(c, p)));
+    CU(launch_fused(p, mode, c->num_sms, st, !tile_sig_matches(c, p), out_type));
     tile_sig_set(c, p);
     if (c->ev_after_fused) {   // iris_step: the metric leg starts behind the feature kernel
         CU(cudaEventRecord(c->ev_after_fused, st));
@@ -201,27 +201,37 @@ int prof_events(iris_ctx* c, std::pair<cudaEvent_t, cudaEvent_t>** out) {
     return IRIS_OK;
 }
 
-int timed_fused(iris_ctx* c, FusedParams& p, int mode, cudaStream_t st) {
-    if (!c->profile) return run_fused(c, p, mode, c->max_segs, st);
+int timed_fused(iris_ctx* c, FusedParams& p, int mode, cudaStream_t st, int out_type) {
+    if (!c->profile) return run_fused(c, p, mode, c->max_segs, st, out_type);
     std::pair<cudaEvent_t, cudaEvent_t>* ev = nullptr;
     int rc = prof_events(c, &ev);
     if (rc) return rc;
     CU(cudaEventRecord(ev->first, st));
-    rc = run_fused(c, p, mode, c->max_segs, st);
+    rc = run_fused(c, p, mode, c->max_segs, st, out_type);
     if (rc) return rc;
     CU(cudaEventRecord(ev->second, st));
     c->prof_clips = c->B;
     return IRIS_OK;
 }
 
-// min-max log-mel: k_fused (features + per-clip extrema) -> k_logmel_post (normalise + log in place)
-int run_logmel_minmax(iris_ctx* c, FusedParams& p, float* d_out, cudaStream_t st) {
+// min-max log-mel: k_fused (fp32 features + per-clip extrema at p.out) -> k_logmel_post (normalise + log
+// in place at d_out == p.out), or for bfloat16 / float16 features k_logmel_post_to from the fp32
+// scratch at p.out into d_out
+int run_logmel_minmax(iris_ctx* c, FusedParams& p, void* d_out, cudaStream_t st, int out_type) {
     const size_t per_clip = size_t(c->n_mel) * c->T * c->C;
     uint32_t* mm = c->minmax.as<uint32_t>();
     unsigned* done = reinterpret_cast<unsigned*>(mm + 2 * size_t(c->B));
-    int rc = timed_fused(c, p, FM_MEL, st);
+    int rc = timed_fused(c, p, FM_MEL, st, OUT_F32);
     if (rc) return rc;
-    CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
+    if (out_type == OUT_F32) CU(launch_logmel_post(p.out, mm, done, c->B, per_clip, 1, 1, st));
+    else CU(launch_logmel_post_to(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
+    return IRIS_OK;
+}
+
+// fp32 mel scratch [B, n_mel, T, C] of a half-width launch whose last pass converts
+int mel_scratch(iris_ctx* c, float** out) {
+    CU(c->mel_scratch.reserve(size_t(c->B) * c->n_mel * c->T * c->C * 4));
+    *out = c->mel_scratch.as<float>();
     return IRIS_OK;
 }
 
@@ -256,7 +266,7 @@ int feature_params(iris_ctx* c, int mode, int select, FusedParams& p) {
 
 // Features from spectrogram banks: the mix + per-cell epilogue is one streaming kernel
 // (k_spec.cu), for the mel modes with the projection and the per-clip extrema fused in.
-int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t st) {
+int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t st, int out_type) {
     const bool mel = mode >= IRIS_FEAT_MEL;
     if (mel && c->remap != IRIS_REMAP_NONE)
         return fail(IRIS_ERR_UNSUPPORTED, "mel features with a channel remap run unfused");
@@ -281,7 +291,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
     }
     if (!mel) {
         p.out = d_out;
-        CU(launch_specmix(p, mode, nullptr, nullptr, nullptr, st));
+        CU(launch_specmix(p, mode, nullptr, nullptr, nullptr, st, out_type));
         return IRIS_OK;
     }
     const size_t per_clip = size_t(c->n_mel) * c->T * c->C;
@@ -290,29 +300,44 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         p.out = d_out;
         p.do_log = mode != IRIS_FEAT_MEL;
         p.do_minmax = mode == IRIS_FEAT_LOGMEL_MINMAX;
+        const bool convert = p.do_minmax && out_type != OUT_F32;   // fp32 mel in scratch, k_logmel_post_to converts
         if (p.do_minmax) {
             CU(c->minmax.reserve(size_t(c->B) * 12));
             CU(cudaMemsetAsync(c->minmax.p, 0, size_t(c->B) * 12, st));
             p.minmax = c->minmax.as<uint32_t>();
+            if (convert) {
+                int rc = mel_scratch(c, &p.out);
+                if (rc) return rc;
+            }
         }
         CU(launch_specmix(p, FM_MEL, c->mel_dense.as<float>(), c->mel_lo.as<int32_t>(),
-                          c->mel_len.as<int32_t>(), st));
-        if (p.do_minmax)
-            CU(launch_logmel_post(d_out, c->minmax.as<uint32_t>(), c->minmax.as<unsigned>() + 2 * size_t(c->B), c->B,
-                                  per_clip, 1, 1, st));
+                          c->mel_len.as<int32_t>(), st, convert ? OUT_F32 : out_type));
+        uint32_t* mm = c->minmax.as<uint32_t>();
+        unsigned* done = c->minmax.as<unsigned>() + 2 * size_t(c->B);
+        if (convert) CU(launch_logmel_post_to(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
+        else if (p.do_minmax) CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
         return IRIS_OK;
     }
-    // many channels: magnitudes through a scratch spectrogram, then the stand-alone kernels
+    // many channels: magnitudes through a scratch spectrogram, then the stand-alone kernels (fp32; for
+    // bfloat16 / float16 features the mel goes to a scratch and the last pass converts)
     CU(c->spec_scratch.reserve(size_t(c->B) * kBins * c->T * 2 * c->C * 4));
     p.out = c->spec_scratch.as<float>();
-    CU(launch_specmix(p, FM_MAGPHASE, nullptr, nullptr, nullptr, st));
-    CU(launch_mel_project(p.out, c->mel_dense.as<float>(), c->mel_lo.as<int32_t>(), c->mel_len.as<int32_t>(),
-                          d_out, c->B, kBins, c->T, c->C, c->n_mel, st));
-    if (mode == IRIS_FEAT_LOGMEL_MINMAX) {
-        int rc = iris_op_minmax(c, 0, d_out, d_out, c->B, int64_t(per_clip), 1, st);
+    CU(launch_specmix(p, FM_MAGPHASE, nullptr, nullptr, nullptr, st, OUT_F32));
+    float* mel_out = d_out;
+    if (out_type != OUT_F32) {
+        int rc = mel_scratch(c, &mel_out);
         if (rc) return rc;
     }
-    if (mode != IRIS_FEAT_MEL) CU(launch_logmel_post(d_out, nullptr, nullptr, c->B, per_clip, 0, 1, st));
+    CU(launch_mel_project(p.out, c->mel_dense.as<float>(), c->mel_lo.as<int32_t>(), c->mel_len.as<int32_t>(),
+                          mel_out, c->B, kBins, c->T, c->C, c->n_mel, st));
+    if (mode == IRIS_FEAT_LOGMEL_MINMAX) {
+        int rc = iris_op_minmax(c, 0, mel_out, mel_out, c->B, int64_t(per_clip), 1, st);
+        if (rc) return rc;
+    }
+    if (out_type != OUT_F32)
+        CU(launch_logmel_post_to(mel_out, d_out, out_type, nullptr, nullptr, c->B, per_clip, 0, mode != IRIS_FEAT_MEL, st));
+    else if (mode != IRIS_FEAT_MEL)
+        CU(launch_logmel_post(d_out, nullptr, nullptr, c->B, per_clip, 0, 1, st));
     return IRIS_OK;
 }
 
@@ -380,7 +405,8 @@ int iris_ctx_destroy(iris_ctx* c) {
     }
     for (DevBuf* d : {&c->tw, &c->whalf, &c->mel_info, &c->mel_w, &c->keep,
                       &c->minmax, &c->scratch_labels, &c->stft_pad, &c->stft_small, &c->tiles, &c->ts, &c->sched,
-                      &c->mel_dense, &c->mel_lo, &c->mel_len, &c->op_small, &c->minmax_ops, &c->eval_scratch, &c->spec_scratch})
+                      &c->mel_dense, &c->mel_lo, &c->mel_len, &c->op_small, &c->minmax_ops, &c->eval_scratch, &c->spec_scratch,
+                      &c->mel_scratch})
         d->release();
     for (int i = 0; i < iris_ctx::kStageRing; ++i) {
         if (c->h_stage[i]) cudaFreeHost(c->h_stage[i]);
@@ -1006,6 +1032,9 @@ int iris_features(iris_ctx* c, int mode, float* d_out, iris_stream stream) {
 
 int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_stream stream) {
     if (!c || !d_out) return fail(IRIS_ERR_INVALID, "NULL argument");
+    int out_type = OUT_F32;
+    if (!split_feature_mode(mode, &mode, &out_type))
+        return fail(IRIS_ERR_INVALID, "bad feature mode: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the mode");
     if (reinterpret_cast<uintptr_t>(d_out) & 15)
         return fail(IRIS_ERR_INVALID, "the feature buffer must be 16-byte aligned (vector stores)");
     if (select < IRIS_SELECT_ALL || select > IRIS_SELECT_BG_NOISE) return fail(IRIS_ERR_INVALID, "bad segment selection");
@@ -1023,7 +1052,7 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
     }
     const bool mel = mode >= IRIS_FEAT_MEL;
     if (mel && c->n_mel == 0) return fail(IRIS_ERR_STATE, "iris_set_mel not called");
-    if (c->spec_mode) return spec_features(c, mode, select, d_out, st);
+    if (c->spec_mode) return spec_features(c, mode, select, d_out, st, out_type);
     if (mel && !c->mel_fusable)
         return fail(IRIS_ERR_UNSUPPORTED,
                     "a mel filter wider than 16 bins (or more than 64 taps over the 32-filter rounds): run "
@@ -1042,11 +1071,15 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
             CU(c->minmax.reserve(size_t(c->B) * 12));   // [B,2] min/max words + [B] k_logmel_post counters
             if (c->minmax.p != before) CU(cudaMemsetAsync(c->minmax.p, 0, c->minmax.cap, st));
             p.minmax = c->minmax.as<uint32_t>();
+            if (out_type != OUT_F32) {   // k_fused writes fp32 mel + extrema to scratch, k_logmel_post_to converts
+                rc = mel_scratch(c, &p.out);
+                if (rc) return rc;
+            }
         }
-        rc = p.do_minmax ? run_logmel_minmax(c, p, d_out, st) : timed_fused(c, p, FM_MEL, st);
+        rc = p.do_minmax ? run_logmel_minmax(c, p, d_out, st, out_type) : timed_fused(c, p, FM_MEL, st, out_type);
         if (rc) return rc;
     } else {
-        rc = timed_fused(c, p, mode, st);
+        rc = timed_fused(c, p, mode, st, out_type);
     }
     if (rc) return rc;
     return IRIS_OK;
@@ -1159,6 +1192,10 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
                           int64_t* bytes_in, int64_t* bytes_out) {
     if (!c || !c->has_plan) return fail(IRIS_ERR_STATE, "no plan uploaded");
     if (clip_lo < 0 || clip_hi > c->B || clip_lo > clip_hi) return fail(IRIS_ERR_INVALID, "bad clip range");
+    int out_type = OUT_F32;
+    if (!split_feature_mode(mode, &mode, &out_type))
+        return fail(IRIS_ERR_INVALID, "bad feature mode: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the mode");
+    const int64_t out_elem = out_type == OUT_F32 ? 4 : 2;
     int64_t in = 0;
     for (size_t i = size_t(c->h_seg_ptr[clip_lo]); i < size_t(c->h_seg_ptr[clip_hi]); ++i) {
         const Seg& s = c->h_segs[i];
@@ -1175,8 +1212,8 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
         in += samples * 4 * c->C;
     }
     int64_t out;
-    if (mode >= IRIS_FEAT_MEL) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->C * 4;
-    else out = int64_t(clip_hi - clip_lo) * kBins * c->T * 2 * c->c_out * 4;
+    if (mode >= IRIS_FEAT_MEL) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->C * out_elem;
+    else out = int64_t(clip_hi - clip_lo) * kBins * c->T * 2 * c->c_out * out_elem;
     if (bytes_in) *bytes_in = in;
     if (bytes_out) *bytes_out = out;
     return IRIS_OK;

@@ -1,5 +1,7 @@
 // Shared device-side definitions for libiris (sm_100a only).
 #pragma once
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -33,6 +35,40 @@ enum FusedMode : int {
 };
 
 enum ChanRemap : int { REMAP_NONE = 0, REMAP_STEREO_MONO = 1, REMAP_MERGE_AUG = 2 };
+
+// element type of the feature output (IRIS_OUT_BF16 / IRIS_OUT_F16 of include/iris.h)
+enum OutType : int { OUT_F32 = 0, OUT_BF16 = 1, OUT_F16 = 2 };
+
+// ---- feature stores: the one place that knows the output format ----
+// All arithmetic is fp32; a half-width output converts at the store with round-to-nearest-even
+// (bit for bit what torch's .to(bfloat16 / float16) does to the fp32 result, fp16 overflow -> +-inf).
+// 1, 2 or 4 consecutive elements; 2 and 4 need 2- / 4-element alignment (8 / 16 bytes for float).
+template <class T> __device__ __forceinline__ T out_cvt(float a);
+template <> __device__ __forceinline__ float out_cvt<float>(float a) { return a; }
+template <> __device__ __forceinline__ __nv_bfloat16 out_cvt<__nv_bfloat16>(float a) { return __float2bfloat16_rn(a); }
+template <> __device__ __forceinline__ __half out_cvt<__half>(float a) { return __float2half_rn(a); }
+// two values as one 32-bit word, a in the low half (the lower address)
+template <class T> __device__ __forceinline__ uint32_t out_pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t out_pack2<__nv_bfloat16>(float a, float b) {
+    const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+template <> __device__ __forceinline__ uint32_t out_pack2<__half>(float a, float b) {
+    const __half2 h = __floats2half2_rn(a, b);
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+template <class T>
+__device__ __forceinline__ void store_out1(T* o, float a) { *o = out_cvt<T>(a); }
+template <class T>
+__device__ __forceinline__ void store_out2(T* o, float a, float b) {
+    if constexpr (sizeof(T) == 4) *reinterpret_cast<float2*>(o) = make_float2(a, b);
+    else *reinterpret_cast<uint32_t*>(o) = out_pack2<T>(a, b);
+}
+template <class T>
+__device__ __forceinline__ void store_out4(T* o, float4 v) {
+    if constexpr (sizeof(T) == 4) *reinterpret_cast<float4*>(o) = v;
+    else *reinterpret_cast<uint2*>(o) = make_uint2(out_pack2<T>(v.x, v.y), out_pack2<T>(v.z, v.w));
+}
 
 struct FusedParams {
     const Seg* segs;

@@ -65,6 +65,18 @@ struct Bank {
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// mode argument of the feature entry points: IRIS_FEAT_* in the low 8 bits, at most one IRIS_OUT_*
+// flag above them.  false: any other high bit (the base mode is range-checked by the caller).
+inline bool split_feature_mode(int mode, int* base, int* out_type) {
+    *base = mode & 0xff;
+    switch (mode & ~0xff) {
+        case 0: *out_type = OUT_F32; return true;
+        case IRIS_OUT_BF16: *out_type = OUT_BF16; return true;
+        case IRIS_OUT_F16: *out_type = OUT_F16; return true;
+        default: return false;
+    }
+}
+
 }  // namespace iris
 
 struct iris_ctx {
@@ -124,6 +136,9 @@ struct iris_ctx {
     int prof_clips = 0;               // clips of the launch the hook timed last
     // stand-alone ops (iris_ops_abi.cu): dense mel matrix + column supports, small scratch
     DevBuf mel_dense, mel_lo, mel_len, op_small, minmax_ops, eval_scratch, spec_scratch;
+    // fp32 mel features [B, n_mel, T, C] of a bfloat16 / float16 launch whose last pass (k_logmel_post_to)
+    // converts: the min-max log-mel modes and the many-channel spectrogram-bank fallback
+    DevBuf mel_scratch;
     bool spec_mode = false;            // the uploaded plan mixes spectrogram banks
     int mel_bins = 0;
     bool mel_fusable = false;

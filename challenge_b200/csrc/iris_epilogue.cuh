@@ -6,8 +6,9 @@
 namespace iris {
 
 // One (bin f, frame t, channel pair) of the output: (r0, i0) / (r1, i1) are the complex values of
-// channels 2*pair and 2*pair + 1, m the product of the SpecAugment masks of this cell.
-template <int MODE>
+// channels 2*pair and 2*pair + 1, m the product of the SpecAugment masks of this cell.  OutT: the
+// element type of p.out (iris_common.cuh, store_out*).
+template <int MODE, class OutT>
 __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, int t, int pair,
                                           bool has1, float r0, float i0, float r1, float i1,
                                           float m) {
@@ -16,7 +17,7 @@ __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, in
     const float filt = (f >= 1 && f <= p.filter_k) ? 0.f : 1.f;   // data_utils.py:126-136
     if (p.remap == REMAP_NONE) {
         const int C = p.C;
-        float* o = p.out + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * C);
+        OutT* o = reinterpret_cast<OutT*>(p.out) + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * C);
         if (p.filter_k > 0) { r0 *= filt; i0 *= filt; r1 *= filt; i1 *= filt; }
         float a0 = r0, a1 = r1, b0 = i0, b1 = i1;   // first half / second half of the last dim
         if (MODE != FM_COMPLEX) {
@@ -30,22 +31,22 @@ __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, in
             }
         }
         if (C == 2) {
-            *reinterpret_cast<float4*>(o) = make_float4(a0, a1, b0, b1);
+            store_out4(o, make_float4(a0, a1, b0, b1));
         } else if (has1 && (C & 1) == 0) {
-            *reinterpret_cast<float2*>(o + 2 * pair) = make_float2(a0, a1);
-            *reinterpret_cast<float2*>(o + C + 2 * pair) = make_float2(b0, b1);
+            store_out2(o + 2 * pair, a0, a1);
+            store_out2(o + C + 2 * pair, b0, b1);
         } else {
-            o[2 * pair] = a0;
-            o[C + 2 * pair] = b0;
+            store_out1(o + 2 * pair, a0);
+            store_out1(o + (C + 2 * pair), b0);
             if (has1) {
-                o[2 * pair + 1] = a1;
-                o[C + 2 * pair + 1] = b1;
+                store_out1(o + (2 * pair + 1), a1);
+                store_out1(o + (C + 2 * pair + 1), b1);
             }
         }
     } else {
         // C == 2 input; c_out output channels (data_utils.py:79-82, 100-117)
         const int Co = p.c_out;
-        float* o = p.out + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * Co);
+        OutT* o = reinterpret_cast<OutT*>(p.out) + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * Co);
         for (int c = 0; c < Co; ++c) {
             float re, im;
             if (c == 0) { re = r0; im = i0; }
@@ -64,8 +65,8 @@ __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, in
                 ph = fast_atan2f(im, re);
                 if (MODE == FM_LOGMAGPHASE) a = __logf(a + 1e-8f);
             }
-            o[c] = a;
-            o[Co + c] = ph;
+            store_out1(o + c, a);
+            store_out1(o + (Co + c), ph);
         }
     }
 }

@@ -7,8 +7,10 @@ namespace iris {
 
 struct FusedParams;
 
-// build_tiles: k_tiles builds the tile blocks first; false: the kernel in front (k_labels) wrote them
-cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream, bool build_tiles);
+// build_tiles: k_tiles builds the tile blocks first; false: the kernel in front (k_labels) wrote them.
+// out_type: OutType (iris_common.cuh) of p.out
+cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream, bool build_tiles,
+                         int out_type);
 size_t fused_smem_bytes(const FusedParams& p, int mode);
 void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge, int32_t out[5]);
 int fused_max_segments();      // mixing segments one clip may have
@@ -23,6 +25,10 @@ size_t fused_tile_bytes(const FusedParams& p, int* stride_out);   // size of p.t
 // minmax: [B,2] extrema words of the clips at x; done: [B] zeroed counters (both may be null without do_minmax)
 cudaError_t launch_logmel_post(float* x, uint32_t* minmax, unsigned* done, int B, size_t per_clip, int do_minmax,
                                int do_log, cudaStream_t stream);
+// the same from the fp32 features at src into dst of OutType out_type (OUT_BF16 / OUT_F16); with neither
+// do_minmax nor do_log it only converts
+cudaError_t launch_logmel_post_to(const float* src, void* dst, int out_type, uint32_t* minmax, unsigned* done,
+                                  int B, size_t per_clip, int do_minmax, int do_log, cudaStream_t stream);
 
 // k_bank.cu
 cudaError_t launch_bank_prepare(const float* wav, const int64_t* d_offsets, const int64_t* d_pad_offsets,
@@ -92,7 +98,7 @@ cudaError_t launch_resample(const float* wav, float* out, int n_chan, long long 
 cudaError_t launch_spec_activity(const float* specs, const int64_t* frame_off, int n_items, int F, int W,
                                  int max_frames, uint8_t* activity, cudaStream_t st);
 cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,
-                           const int32_t* mel_len, cudaStream_t st);
+                           const int32_t* mel_len, cudaStream_t st, int out_type);   // out_type: OutType of p.out
 size_t specmix_mel_smem(int C, int f_n);
 
 // k_eval.cu -- evaluation-side chain of metrics.evaluate (metrics.py:59-87, 109-133, 176-214)

@@ -135,17 +135,20 @@ int ensure_step_state(iris_ctx* c) {
     return IRIS_OK;
 }
 
-// DLManagedTensor -> device pointer after checking device / dtype / layout / shape
+// DLManagedTensor -> device pointer after checking device / dtype / layout / shape; dtype: float32, or
+// for features the OutType of the mode's IRIS_OUT_* flag
 int dl_device_ptr(iris_ctx* c, void* managed, const int64_t* want_shape, int want_ndim, const char* what,
-                  float** out) {
+                  float** out, int out_type = OUT_F32) {
     if (!managed) return fail(IRIS_ERR_INVALID, std::string(what) + ": NULL DLManagedTensor");
     const DLTensor& t = static_cast<DLManagedTensor*>(managed)->dl_tensor;
     if (t.device.device_type != kDLCUDA)
         return fail(IRIS_ERR_INVALID, std::string(what) + ": DLPack tensor is not in CUDA device memory");
     if (t.device.device_id != c->device)
         return fail(IRIS_ERR_INVALID, std::string(what) + ": DLPack tensor lives on another device than the context");
-    if (t.dtype.code != kDLFloat || t.dtype.bits != 32 || t.dtype.lanes != 1)
-        return fail(IRIS_ERR_INVALID, std::string(what) + ": DLPack tensor must be float32");
+    static const struct { int code, bits; const char* name; } kWant[3] = {
+        {kDLFloat, 32, "float32"}, {kDLBfloat, 16, "bfloat16 (IRIS_OUT_BF16)"}, {kDLFloat, 16, "float16 (IRIS_OUT_F16)"}};
+    if (t.dtype.code != kWant[out_type].code || t.dtype.bits != kWant[out_type].bits || t.dtype.lanes != 1)
+        return fail(IRIS_ERR_INVALID, std::string(what) + ": DLPack tensor must be " + kWant[out_type].name);
     if (t.ndim != want_ndim) return fail(IRIS_ERR_INVALID, std::string(what) + ": wrong rank");
     int64_t stride = 1;
     for (int i = t.ndim - 1; i >= 0; --i) {
@@ -164,6 +167,7 @@ int dl_device_ptr(iris_ctx* c, void* managed, const int64_t* want_shape, int wan
     return IRIS_OK;
 }
 
+// mode: the base mode (IRIS_FEAT_*)
 void feature_shape(const iris_ctx* c, int mode, int64_t (&shape)[4]) {
     shape[0] = c->B;
     if (mode >= IRIS_FEAT_MEL) { shape[1] = c->n_mel; shape[2] = c->T; shape[3] = c->C; }
@@ -310,6 +314,9 @@ int iris_draw_batch(const iris_draw_config* cfg, const int32_t* bg_frames, int n
 
 int iris_step(iris_ctx* c, const iris_step_config* cfg, const iris_step_io* io, iris_stream stream) {
     if (!c || !cfg || !io || !io->uniforms || !io->d_features) return fail(IRIS_ERR_INVALID, "iris_step: NULL argument");
+    int base_mode = 0, out_type = OUT_F32;   // the output flag is iris_features' business; the rest needs the mode
+    if (!split_feature_mode(cfg->feature_mode, &base_mode, &out_type))
+        return fail(IRIS_ERR_INVALID, "iris_step: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the feature mode");
     int rc = iris_set_device(c);
     if (rc) return rc;
     rc = ensure_step_state(c);
@@ -381,7 +388,7 @@ int iris_step(iris_ctx* c, const iris_step_config* cfg, const iris_step_io* io, 
         for (auto& l : c->legs)
             if (l.seq && l.labels == io->d_frame_labels) CU(cudaStreamWaitEvent(st, l.done, 0));
     if (V > 0) {
-        c->feat_hint = cfg->feature_mode;   // k_labels also builds the tile blocks of the feature launch
+        c->feat_hint = base_mode;   // k_labels also builds the tile blocks of the feature launch
         rc = iris_labels(c, io->d_labels_vtk, io->d_frame_labels, io->d_keep, stream);
         if (rc) return rc;
     }
@@ -389,7 +396,7 @@ int iris_step(iris_ctx* c, const iris_step_config* cfg, const iris_step_io* io, 
     // k_fused and runs beside k_logmel_post (31 us, the leg takes ~10): k_labels -> k_fused stay
     // adjacent in the stream, so k_fused's programmatic launch overlaps its prologue with k_labels.
     // Other modes have no second pass to hide the leg behind: it forks right behind k_labels.
-    const bool late = metric && cfg->feature_mode == IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode;
+    const bool late = metric && base_mode == IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode;
     if (late) {
         c->ev_after_fused = c->ev_labels;
         rc = iris_features(c, cfg->feature_mode, io->d_features, stream);
@@ -557,11 +564,13 @@ int iris_host_free(iris_ctx* c, void* p, size_t bytes) {
 int iris_features_dlpack(iris_ctx* c, int mode, void* managed, iris_stream stream) {
     if (!c) return fail(IRIS_ERR_INVALID, "NULL ctx");
     if (!c->has_plan) return fail(IRIS_ERR_STATE, "no plan uploaded");
-    if (mode < IRIS_FEAT_COMPLEX || mode > IRIS_FEAT_LOGMEL_MINMAX) return fail(IRIS_ERR_INVALID, "bad feature mode");
+    int base = 0, out_type = OUT_F32;
+    if (!split_feature_mode(mode, &base, &out_type) || base < IRIS_FEAT_COMPLEX || base > IRIS_FEAT_LOGMEL_MINMAX)
+        return fail(IRIS_ERR_INVALID, "bad feature mode");
     int64_t shape[4];
-    feature_shape(c, mode, shape);
+    feature_shape(c, base, shape);
     float* out = nullptr;
-    int rc = dl_device_ptr(c, managed, shape, 4, "features", &out);
+    int rc = dl_device_ptr(c, managed, shape, 4, "features", &out, out_type);
     if (rc) return rc;
     return iris_features(c, mode, out, stream);
 }
@@ -589,16 +598,19 @@ int iris_step_dlpack(iris_ctx* c, const iris_step_config* cfg, const double* uni
     const iris_draw_config& g = cfg->draw;
     const Bank& bg = c->banks[IRIS_BANK_BG];
     if (!bg.ready) return fail(IRIS_ERR_STATE, "background bank not registered");
+    int base_mode = 0, out_type = OUT_F32;
+    if (!split_feature_mode(cfg->feature_mode, &base_mode, &out_type))
+        return fail(IRIS_ERR_INVALID, "iris_step_dlpack: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the feature mode");
     int c_out = bg.n_chan;
     if (cfg->chan_remap == IRIS_REMAP_STEREO_MONO) c_out = 3;
     else if (cfg->chan_remap == IRIS_REMAP_MERGE_AUG) c_out = cfg->n_out_chan;
     int64_t fs[4] = {g.batch, kBins, g.n_frame, 2 * c_out};
-    if (cfg->feature_mode >= IRIS_FEAT_MEL) { fs[1] = c->n_mel; fs[3] = bg.n_chan; }
+    if (base_mode >= IRIS_FEAT_MEL) { fs[1] = c->n_mel; fs[3] = bg.n_chan; }
     iris_step_io io;
     memset(&io, 0, sizeof io);
     io.uniforms = uniforms;
     io.streams = streams;
-    int rc = dl_device_ptr(c, managed_features, fs, 4, "features", &io.d_features);
+    int rc = dl_device_ptr(c, managed_features, fs, 4, "features", &io.d_features, out_type);
     if (rc) return rc;
     if (managed_frame_labels) {
         const int64_t s3[3] = {g.batch, g.n_frame, c->banks[IRIS_BANK_VOICE].n_classes};

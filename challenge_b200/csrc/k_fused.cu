@@ -141,21 +141,22 @@ __device__ __forceinline__ float4 make_piece(const FusedParams& p, int f, float 
     }
     return make_float4(a0, a1, b0, b1);
 }
+template <class OutT>
 __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, int t, int pair, bool has1,
                                             float4 v) {
     const int C = p.C;
-    float* o = p.out + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * C);
+    OutT* o = reinterpret_cast<OutT*>(p.out) + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * C);
     if (C == 2) {
-        *reinterpret_cast<float4*>(o) = v;
+        store_out4(o, v);
     } else if (has1 && (C & 1) == 0) {
-        *reinterpret_cast<float2*>(o + 2 * pair) = make_float2(v.x, v.y);
-        *reinterpret_cast<float2*>(o + C + 2 * pair) = make_float2(v.z, v.w);
+        store_out2(o + 2 * pair, v.x, v.y);
+        store_out2(o + C + 2 * pair, v.z, v.w);
     } else {
-        o[2 * pair] = v.x;
-        o[C + 2 * pair] = v.z;
+        store_out1(o + 2 * pair, v.x);
+        store_out1(o + (C + 2 * pair), v.z);
         if (has1) {
-            o[2 * pair + 1] = v.y;
-            o[C + 2 * pair + 1] = v.w;
+            store_out1(o + (2 * pair + 1), v.y);
+            store_out1(o + (C + 2 * pair + 1), v.w);
         }
     }
 }
@@ -168,10 +169,12 @@ __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, 
 // with their switches fixed at compile time (EPI_C2 | EPI_MINMAX or EPI_LOG or neither): no
 // per-round flag branches, no odd-channel selects, C folded into the address arithmetic, the
 // projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.
+// OutT: element type of p.out (float, __nv_bfloat16, __half).  The half instances have no min-max
+// epilogue: the min-max log-mel features are normalised by k_logmel_post, which converts.
 constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4;
 constexpr int kFixFR = 8;   // frames per tile of the fixed mel variants
 __host__ __device__ constexpr int fixed_mel_L(int r) { return r == 0 ? 2 : (r == 1 ? 4 : (r == 2 ? 6 : 0)); }
-template <int MODE, int NJ, int EPI>
+template <int MODE, int NJ, int EPI, class OutT>
 __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParams p) {
     extern __shared__ __align__(128) unsigned char sm[];
     // per-clip extrema of the CTA: {~bits(min), bits(max), warps arrived, -} per run of tiles of one
@@ -180,8 +183,10 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
     constexpr bool kMel = (MODE == FM_MEL);
     constexpr bool kFix = (EPI != 0);      // switches below are compile-time constants
     static_assert(!kFix || kMel, "fixed epilogues exist for the mel modes only");
+    constexpr bool kF32 = sizeof(OutT) == 4;
+    static_assert(kF32 || (MODE != FM_ACTIVITY && !(EPI & EPI_MINMAX)), "activity flags and the min-max epilogue are fp32 only");
     constexpr int S = slots_of(MODE);      // stage buffers
-    const bool do_minmax = kFix ? bool(EPI & EPI_MINMAX) : (p.do_minmax != 0);
+    const bool do_minmax = !kF32 ? false : kFix ? bool(EPI & EPI_MINMAX) : (p.do_minmax != 0);
     const bool do_lg = kFix ? bool(EPI & EPI_LOG) : (p.do_log && !p.do_minmax);
     const int C = kFix ? 2 : p.C;
     const int tid = threadIdx.x;
@@ -394,7 +399,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
         // mel rows are re-read by k_logmel_post: ask L2 to keep them (a 256-clip batch does not fit
         // anyway, but the hint measures 4-8 us better than plain stores)
         const bool keep_l2 = kMel && do_minmax;
-        float* clip_out = p.out;      // out[b, 0, 0, 0] of the current clip (mel modes)
+        OutT* clip_out = reinterpret_cast<OutT*>(p.out);   // out[b, 0, 0, 0] of the current clip (mel modes)
         uint32_t zbits = 0;
         int zb_clip = -1;
         const size_t clip_elems = size_t(p.n_mel) * p.T * C;
@@ -462,7 +467,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
             // bit 8 -> bin 256.  Recomputed when the clip changes.
             if (b != zb_clip) {
                 zb_clip = b;
-                if (kMel) clip_out = p.out + size_t(b) * clip_elems;
+                if (kMel) clip_out = reinterpret_cast<OutT*>(p.out) + size_t(b) * clip_elems;
                 zbits = 0;
                 const int4 fmv = *reinterpret_cast<const int4*>(tb->fm);
                 if (kMel && NJ == 4) {
@@ -584,7 +589,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 }
                 // ---- every lane stores its own mel values: out[b, m, t, 2*pair .. +1] ----
                 if (in_range) {
-                    float* o_t = clip_out + t * C + 2 * pair;
+                    OutT* o_t = clip_out + t * C + 2 * pair;
                     const uint32_t row_elems = uint32_t(p.T) * uint32_t(C);
                     const bool lg = do_lg;
 #pragma unroll
@@ -592,7 +597,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                         if (kFix ? (fixed_mel_L(r) == 0) : (p.mel_L[r] == 0)) break;   // uniform: no work behind the last round
                         const uint32_t mrow = ms[32 * r] >> 16;   // mel row of this slot; 0xffff: idle lane
                         if (mrow != 0xffffu) {
-                            float* o = o_t + mrow * row_elems;
+                            OutT* o = o_t + mrow * row_elems;
                             float a0 = acc0[r], a1 = acc1[r];
                             if (do_minmax) {
                                 mn = fminf(mn, has1 ? fminf(a0, a1) : a0);
@@ -603,11 +608,15 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                                 a1 = __logf(a1 + 1e-8f);
                             }
                             if ((C & 1) == 0) {
-                                if (keep_l2) st_f2_hint(o, a0, a1, pol_keep);
-                                else *reinterpret_cast<float2*>(o) = make_float2(a0, a1);
+                                if constexpr (kF32) {
+                                    if (keep_l2) st_f2_hint(o, a0, a1, pol_keep);
+                                    else store_out2(o, a0, a1);
+                                } else {
+                                    store_out2(o, a0, a1);
+                                }
                             } else {
-                                o[0] = a0;
-                                if (has1) o[1] = a1;
+                                store_out1(o, a0);
+                                if (has1) store_out1(o + 1, a1);
                             }
                         }
                     }
@@ -666,11 +675,11 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                         if (tt < p.T) {
                             const unsigned char* x1 = sm + off_xch(mel_taps) + jt * kXwBytes + half * 8;
                             const unsigned char* x0 = reinterpret_cast<const unsigned char*>(stg) + half * 8;
-                            float* o = p.out + (size_t(b) * kBins * p.T + tt) * 8 + half * 4;
+                            OutT* o = reinterpret_cast<OutT*>(p.out) + (size_t(b) * kBins * p.T + tt) * 8 + half * 4;
                             for (int f = warp * 2 + (lane >> 4); f < kBins; f += FR * 2) {
                                 const float2 a = *reinterpret_cast<const float2*>(x0 + (f * FR + (jt ^ (f & 7))) * 16);
                                 const float2 c = *reinterpret_cast<const float2*>(x1 + ((f ^ jt) << 4));
-                                *reinterpret_cast<float4*>(o + size_t(f) * p.T * 8) = make_float4(a.x, a.y, c.x, c.y);
+                                store_out4(o + size_t(f) * p.T * 8, make_float4(a.x, a.y, c.x, c.y));
                             }
                         }
                         named_bar_sync(1, FR * 32);   // staging + exchange rows are read before they are reused
@@ -683,7 +692,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                     const int tt = (hdr.z & 0xffffff) + jt;
                     if (tt < p.T) {
                         for (int f = warp * 4 + (lane >> 3); f < kBins; f += FR * 4)
-                            store_piece(p, b, f, tt, pair, has1, stg[f * FR + (jt ^ (f & 7))]);
+                            store_piece<OutT>(p, b, f, tt, pair, has1, stg[f * FR + (jt ^ (f & 7))]);
                     }
                 }
                 named_bar_sync(1, FR * 32);   // the pieces are read before the next tile overwrites them
@@ -693,12 +702,12 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 for (int jj = 0; jj < 8; ++jj) {
                     const int f = k1 + 16 * (2 * jj + par);
                     const cpx zf = u[jj], zm = mirror(jj);
-                    store_bin<MODE>(p, b, f, t, pair, has1, zf.x + zm.x, zf.y - zm.y, zf.y + zm.y,
+                    store_bin<MODE, OutT>(p, b, f, t, pair, has1, zf.x + zm.x, zf.y - zm.y, zf.y + zm.y,
                                     zm.x - zf.x, ((zbits >> jj) & 1u) ? 0.f : mt);
                 }
                 if (l0) {
                     const cpx zf = u[8];
-                    store_bin<MODE>(p, b, 256, t, pair, has1, zf.x + zf.x, zf.y - zf.y, zf.y + zf.y,
+                    store_bin<MODE, OutT>(p, b, 256, t, pair, has1, zf.x + zf.x, zf.y - zf.y, zf.y + zf.y,
                                     zf.x - zf.x, ((zbits >> 8) & 1u) ? 0.f : mt);
                 }
             }
@@ -769,8 +778,10 @@ void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge
 }
 
 // p.tile_blocks (fused_tile_bytes) is provided by the caller; build_tiles: k_tiles builds them first
-// (otherwise the kernel in front -- k_labels -- has built them and triggers early)
-cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStream_t stream, bool build_tiles) {
+// (otherwise the kernel in front -- k_labels -- has built them and triggers early).  out_type: OutType
+// of p.out; FM_ACTIVITY and the min-max epilogue write fp32 only.
+cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStream_t stream, bool build_tiles,
+                         int out_type) {
     FusedParams p = p_in;
     const int FR = p.fr;
     if (FR < 1 || FR > kMaxFR) return cudaErrorInvalidValue;
@@ -781,6 +792,8 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     if (mode == FM_MEL && (long long)p.n_mel * p.T * p.C > 0x7fffffffLL) return cudaErrorInvalidValue;   // 32-bit row offsets inside a clip
     const size_t smem = fused_smem_bytes(p, mode);
     if (smem > 227 * 1024 - 256) return cudaErrorInvalidValue;   // (128 B of static shared memory: s_mm)
+    if (out_type != OUT_F32 && ((out_type != OUT_BF16 && out_type != OUT_F16) || mode == FM_ACTIVITY || p.do_minmax))
+        return cudaErrorInvalidValue;
     if (build_tiles) k_tiles<<<unsigned((n_tiles + 127) / 128), 128, 0, stream>>>(p);
     // k_fused is a programmatic dependent launch behind k_tiles / k_labels: its prologue overlaps
     // their tail
@@ -790,7 +803,7 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     // per kernel variant.  The register cap decides between 1 and 2 CTAs per SM: measured on B200,
     // 96 registers give 2 x 9 warps, 104 and 112 only one CTA (576 x 112 = 64512 < 65536, but
     // registers are granted per warp in larger units) -- 4-ch COMPLEX 570 -> 730 us, mel 200 -> 265 us.
-#define IRIS_LAUNCH(M, NJV, EPIV)                                                                     \
+#define IRIS_LAUNCH(M, NJV, EPIV, T)                                                                   \
     {                                                                                           \
         const int threads = (FR + 1) * 32;                                                      \
         static int attr_dev = -1;   /* function attributes are per device */                    \
@@ -798,20 +811,20 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         static size_t per_sm_smem = 0;                                                          \
         if (attr_dev != dev) {                                                                  \
             cudaFuncAttributes fa;                                                              \
-            cudaError_t e = cudaFuncGetAttributes(&fa, k_fused<M, NJV, EPIV>);                  \
+            cudaError_t e = cudaFuncGetAttributes(&fa, k_fused<M, NJV, EPIV, T>);                  \
             if (e != cudaSuccess) return e;                                                     \
-            e = cudaFuncSetAttribute(k_fused<M, NJV, EPIV>,                                     \
+            e = cudaFuncSetAttribute(k_fused<M, NJV, EPIV, T>,                                     \
                                      cudaFuncAttributeMaxDynamicSharedMemorySize,               \
                                      227 * 1024 - int(fa.sharedSizeBytes));                     \
             if (e != cudaSuccess) return e;                                                     \
-            cudaFuncSetAttribute(k_fused<M, NJV, EPIV>, cudaFuncAttributePreferredSharedMemoryCarveout, \
+            cudaFuncSetAttribute(k_fused<M, NJV, EPIV, T>, cudaFuncAttributePreferredSharedMemoryCarveout, \
                                  cudaSharedmemCarveoutMaxShared);                               \
             attr_dev = dev;                                                                     \
             per_sm_smem = 0;                                                                    \
         }                                                                                       \
         if (per_sm_smem != smem) {                                                              \
             int nb = 0;                                                                         \
-            cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_fused<M, NJV, EPIV>, \
+            cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_fused<M, NJV, EPIV, T>, \
                                                                           threads, smem);       \
             if (e != cudaSuccess) return e;                                                     \
             per_sm = nb < 1 ? 1 : nb;                                                           \
@@ -830,26 +843,33 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         attr[0].val.programmaticStreamSerializationAllowed = 1;                                 \
         cfg.attrs = attr;                                                                       \
         cfg.numAttrs = 1;                                                                       \
-        cudaError_t le = cudaLaunchKernelEx(&cfg, k_fused<M, NJV, EPIV>, p);                    \
+        cudaError_t le = cudaLaunchKernelEx(&cfg, k_fused<M, NJV, EPIV, T>, p);                    \
         if (le != cudaSuccess) return le;                                                       \
     }
+#define IRIS_LAUNCH_OUT(M, NJV, EPIV)                                                         \
+    {                                                                                           \
+        if (out_type == OUT_BF16) IRIS_LAUNCH(M, NJV, EPIV, __nv_bfloat16)                      \
+        else if (out_type == OUT_F16) IRIS_LAUNCH(M, NJV, EPIV, __half)                         \
+        else IRIS_LAUNCH(M, NJV, EPIV, float)                                                   \
+    }
     switch (mode) {
-        case FM_COMPLEX: IRIS_LAUNCH(FM_COMPLEX, 8, 0) break;
-        case FM_MAGPHASE: IRIS_LAUNCH(FM_MAGPHASE, 8, 0) break;
-        case FM_LOGMAGPHASE: IRIS_LAUNCH(FM_LOGMAGPHASE, 8, 0) break;
+        case FM_COMPLEX: IRIS_LAUNCH_OUT(FM_COMPLEX, 8, 0) break;
+        case FM_MAGPHASE: IRIS_LAUNCH_OUT(FM_MAGPHASE, 8, 0) break;
+        case FM_LOGMAGPHASE: IRIS_LAUNCH_OUT(FM_LOGMAGPHASE, 8, 0) break;
         case FM_MEL:
-            if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH(FM_MEL, 8, 0)
+            if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
             else if (p.C != 2 || p.mel_L[0] != fixed_mel_L(0) || p.mel_L[1] != fixed_mel_L(1) ||
                      p.mel_L[2] != fixed_mel_L(2) || p.mel_L[3] != fixed_mel_L(3) ||
                      FR != kFixFR || p.mel_taps != 12 || getenv("IRIS_NO_FIXED_EPI"))
-                IRIS_LAUNCH(FM_MEL, 4, 0)
-            else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX)
-            else if (p.do_log) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_LOG)
-            else IRIS_LAUNCH(FM_MEL, 4, EPI_C2)
+                IRIS_LAUNCH_OUT(FM_MEL, 4, 0)
+            else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX, float)
+            else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | EPI_LOG)
+            else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2)
             break;
-        case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0) break;
+        case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0, float) break;
         default: return cudaErrorInvalidValue;
     }
+#undef IRIS_LAUNCH_OUT
 #undef IRIS_LAUNCH
     return cudaGetLastError();
 }

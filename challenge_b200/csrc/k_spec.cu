@@ -50,7 +50,7 @@ constexpr int kSpecTile = 32;      // frames per CTA
 constexpr int kSpecWarps = 8;
 constexpr int kSpecMaxSegs = 48;   // staged segments per tile; more fall back to the global list
 
-template <int MODE>
+template <int MODE, class OutT>
 __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_constant__ FusedParams p,
                                                             const float* __restrict__ melW,
                                                             const int32_t* __restrict__ mel_lo,
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                     o[0] = sqrt_approx(fmaf(a0, a0, b0 * b0));   // transforms.py:116
                     if (has1) o[1] = sqrt_approx(fmaf(a1, a1, b1 * b1));
                 } else if (live) {
-                    store_bin<MODE>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
+                    store_bin<MODE, OutT>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
                 }
             }
         }
@@ -205,7 +205,8 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
             if (live) {
                 mn = fminf(mn, acc);
                 mx = fmaxf(mx, acc);
-                p.out[((size_t(b) * p.n_mel + mi) * p.T + t) * C + c] = lg ? __logf(acc + 1e-8f) : acc;
+                store_out1(reinterpret_cast<OutT*>(p.out) + ((size_t(b) * p.n_mel + mi) * p.T + t) * C + c,
+                           lg ? __logf(acc + 1e-8f) : acc);
             }
         }
     }
@@ -231,34 +232,47 @@ cudaError_t launch_spec_activity(const float* specs, const int64_t* frame_off, i
 
 size_t specmix_mel_smem(int C, int f_n) { return size_t(f_n) * kSpecTile * C * 4; }
 
-// mode FM_MEL: p.out [B, n_mel, T, C], p.do_log / p.do_minmax / p.minmax as in the fused kernel;
-// melW dense [257, n_mel] with the non-zero rows [lo, lo + len) of every filter.
-cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,
-                           const int32_t* mel_len, cudaStream_t st) {
-    if (p.B <= 0 || p.T <= 0) return cudaSuccess;
-    if (p.B > 65535) return cudaErrorInvalidValue;
+template <class OutT>
+static cudaError_t launch_specmix_t(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,
+                                    const int32_t* mel_len, cudaStream_t st) {
     dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
     const int threads = kSpecWarps * 32;
     switch (mode) {
-        case FM_COMPLEX: k_specmix<FM_COMPLEX><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
-        case FM_MAGPHASE: k_specmix<FM_MAGPHASE><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
-        case FM_LOGMAGPHASE: k_specmix<FM_LOGMAGPHASE><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
+        case FM_COMPLEX: k_specmix<FM_COMPLEX, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
+        case FM_MAGPHASE: k_specmix<FM_MAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
+        case FM_LOGMAGPHASE: k_specmix<FM_LOGMAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
         case FM_MEL: {
             const size_t smem = specmix_mel_smem(p.C, p.mel_f_n);
             if (smem > 200 * 1024) return cudaErrorInvalidValue;
-            static bool attr_set = false;
+            static bool attr_set = false;   // per instance
             if (!attr_set) {
-                cudaError_t e = cudaFuncSetAttribute(k_specmix<FM_MEL>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                cudaError_t e = cudaFuncSetAttribute(k_specmix<FM_MEL, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                                      200 * 1024);
                 if (e != cudaSuccess) return e;
                 attr_set = true;
             }
-            k_specmix<FM_MEL><<<grid, threads, smem, st>>>(p, melW, mel_lo, mel_len);
+            k_specmix<FM_MEL, OutT><<<grid, threads, smem, st>>>(p, melW, mel_lo, mel_len);
             break;
         }
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
+}
+
+// mode FM_MEL: p.out [B, n_mel, T, C], p.do_log / p.do_minmax / p.minmax as in the fused kernel;
+// melW dense [257, n_mel] with the non-zero rows [lo, lo + len) of every filter.  out_type: OutType
+// of p.out (the min-max mel features are fp32: k_logmel_post normalises them).
+cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,
+                           const int32_t* mel_len, cudaStream_t st, int out_type) {
+    if (p.B <= 0 || p.T <= 0) return cudaSuccess;
+    if (p.B > 65535) return cudaErrorInvalidValue;
+    if (out_type != OUT_F32 && p.do_minmax) return cudaErrorInvalidValue;
+    switch (out_type) {
+        case OUT_F32: return launch_specmix_t<float>(p, mode, melW, mel_lo, mel_len, st);
+        case OUT_BF16: return launch_specmix_t<__nv_bfloat16>(p, mode, melW, mel_lo, mel_len, st);
+        case OUT_F16: return launch_specmix_t<__half>(p, mode, melW, mel_lo, mel_len, st);
+        default: return cudaErrorInvalidValue;
+    }
 }
 
 }  // namespace iris

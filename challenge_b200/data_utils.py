@@ -181,6 +181,27 @@ def stft_filter(filter_num):
     return _stft_filter
 
 
+def cast_features(dtype):
+    """Not a reference function: the drop-in form of ``.map(lambda x, y: (tf.cast(x, dtype), y))``,
+    e.g. for a trainer that runs in bfloat16 / float16.  ``dtype``: torch.bfloat16, torch.float16,
+    torch.float32 or their names; anything else raises ValueError here.  Mapped after ``.batch()``
+    behind stages the fused launch absorbs, it is absorbed too: the feature kernels store that dtype
+    (the float32 features rounded to nearest even, bit for bit ``x.to(dtype)``).  Anywhere else it
+    runs ``x.to(dtype)``.  Labels are not touched."""
+    from .engine import out_flag
+    import torch
+    flag = out_flag(dtype)
+    dt = {0: torch.float32, L.OUT_BF16: torch.bfloat16, L.OUT_F16: torch.float16}[flag]
+
+    def _cast_features(x, y=None):
+        x = x.to(dt) if isinstance(x, torch.Tensor) else O.dev(x).to(dt)
+        if y is None:
+            return x
+        return x, y
+    _cast_features._iris_stage = ('cast', flag)
+    return _cast_features
+
+
 def speech_enhancement_preprocess(x, y=None):
     """
     :param y: ([..., n_voices, n_frames, n_classes], ..., ...)

@@ -13,6 +13,28 @@ def _torch():
     return torch
 
 
+def out_flag(dtype):
+    """IRIS_OUT_* flag of a feature dtype: 0 for torch.float32, OUT_BF16 / OUT_F16 for torch.bfloat16 /
+    torch.float16 (or their names).  Any other dtype raises ValueError."""
+    torch = _torch()
+    if isinstance(dtype, str):
+        dtype = getattr(torch, dtype, None) if dtype in ('float32', 'bfloat16', 'float16') else None
+    flags = {torch.float32: 0, torch.bfloat16: L.OUT_BF16, torch.float16: L.OUT_F16}
+    if dtype not in flags:
+        raise ValueError('features are float32, bfloat16 or float16, not %r' % (dtype,))
+    return flags[dtype]
+
+
+def out_dtype(mode):
+    """torch dtype of the features of a mode with or without an IRIS_OUT_* flag."""
+    torch = _torch()
+    dtypes = {0: torch.float32, L.OUT_BF16: torch.bfloat16, L.OUT_F16: torch.float16}
+    flag = int(mode) & ~L.MODE_MASK
+    if flag not in dtypes:
+        raise ValueError('feature mode 0x%x: at most one of OUT_BF16 / OUT_F16 above the mode' % int(mode))
+    return dtypes[flag]
+
+
 def default_mel_matrix(num_mel_bins=80, num_spectrogram_bins=257, sample_rate=16000,
                        lower_edge_hertz=125.0, upper_edge_hertz=3800.0):
     """``tf.signal.linear_to_mel_weight_matrix`` (called at transforms.py:55-56), rebuilt
@@ -210,25 +232,33 @@ class Engine:
 
     def feature_shape(self, mode):
         pl = self._plan
-        if mode >= L.FEAT_MEL:
+        if int(mode) & L.MODE_MASK >= L.FEAT_MEL:
             return (pl['B'], self.n_mel, pl['T'], self.bank_chan)
         return (pl['B'], 257, pl['T'], 2 * pl['c_out'])
 
-    def features(self, mode, out=None, select=L.SELECT_ALL):
+    def features(self, mode, out=None, select=L.SELECT_ALL, dtype=None):
         """``select``: SELECT_VOICES / SELECT_BG_NOISE give ``only_voice`` / ``only_noise`` of
-        ``merge_complex_specs(seperate_noise_voice=True)`` (plain complex spectrograms)."""
+        ``merge_complex_specs(seperate_noise_voice=True)`` (plain complex spectrograms).  ``dtype``:
+        torch.float32 (default), torch.bfloat16 or torch.float16 -- the float32 features rounded to
+        nearest even by the kernel's store; default: the dtype of ``out``, else float32."""
+        torch = _torch()
         pl = self._plan
+        if dtype is None:
+            dtype = out.dtype if out is not None else torch.float32
+        mode = int(mode) | out_flag(dtype)
         shape = self.feature_shape(mode) if select == L.SELECT_ALL else (pl['B'], 257, pl['T'], 2 * self.bank_chan)
         if out is None:
-            out = self._empty(shape)
+            out = self._empty(shape, dtype)
         else:
-            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda
-        L.check(self.lib.iris_features_select(self._ctx, int(mode), int(select), self._ptr(out), self._stream()))
+            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == dtype
+        L.check(self.lib.iris_features_select(self._ctx, mode, int(select), self._ptr(out), self._stream()))
         return out
 
     # ---- one call per batch (iris_step) ----
-    def step_config(self, draw_cfg, mode, stft_filter=0, chan_remap=L.REMAP_NONE, n_out_chan=0):
-        return L.IrisStepConfig(draw_cfg, int(stft_filter), int(chan_remap), int(n_out_chan), int(mode))
+    def step_config(self, draw_cfg, mode, stft_filter=0, chan_remap=L.REMAP_NONE, n_out_chan=0, out_dtype=None):
+        """``out_dtype``: torch.float32 (default), torch.bfloat16 or torch.float16 features."""
+        flag = 0 if out_dtype is None else out_flag(out_dtype)
+        return L.IrisStepConfig(draw_cfg, int(stft_filter), int(chan_remap), int(n_out_chan), int(mode) | flag)
 
     def step(self, scfg, uniforms, streams=None, out=None, frame=None, want_frame=True, vtk=None,
              keep=None, y_pred=None, triples=None, counts=None, comm=None, counts_reduced=None,
@@ -248,9 +278,9 @@ class Engine:
         mode = scfg.feature_mode
         shape = self.feature_shape(mode)
         if out is None:
-            out = self._empty(shape)
+            out = self._empty(shape, out_dtype(mode))
         else:
-            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda
+            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == out_dtype(mode)
         if frame is None and want_frame and V > 0:
             frame = self._empty((B, T, self.n_classes))
         u = uniforms if uniforms.flags['C_CONTIGUOUS'] and uniforms.dtype == np.float64 \
@@ -320,11 +350,22 @@ class Engine:
 
     # ---- DLPack hand-over ----
     def features_dlpack(self, mode, capsule):
-        """``iris_features`` into the tensor behind a DLPack capsule (``to_dlpack(t)``)."""
-        L.check(self.lib.iris_features_dlpack(self._ctx, int(mode), L.dlpack_pointer(capsule), self._stream()))
+        """``iris_features`` into the tensor behind a DLPack capsule (``to_dlpack(t)``).  Without an
+        IRIS_OUT_* flag in ``mode`` the flag of the tensor's dtype (bfloat16 / float16) is added."""
+        ptr = L.dlpack_pointer(capsule)
+        mode = int(mode)
+        if not mode & ~L.MODE_MASK:
+            mode |= L.dlpack_out_flag(ptr)
+        L.check(self.lib.iris_features_dlpack(self._ctx, mode, ptr, self._stream()))
 
     def step_dlpack(self, scfg, uniforms, features_capsule, frame_capsule=None, streams=None):
+        """``iris_step`` into DLPack tensors; without an IRIS_OUT_* flag in ``scfg.feature_mode`` the flag
+        of the feature tensor's dtype is added."""
         u = np.ascontiguousarray(uniforms, np.float64)
+        fptr = L.dlpack_pointer(features_capsule)
+        if not scfg.feature_mode & ~L.MODE_MASK:
+            scfg = L.IrisStepConfig(scfg.draw, scfg.stft_filter, scfg.chan_remap, scfg.n_out_chan,
+                                    scfg.feature_mode | L.dlpack_out_flag(fptr))
         g = scfg.draw
         c_out = self.bank_chan
         if scfg.chan_remap == L.REMAP_STEREO_MONO:
@@ -333,7 +374,7 @@ class Engine:
             c_out = int(scfg.n_out_chan)
         self._plan = dict(B=g.batch, T=g.n_frame, V=g.max_voices, c_out=c_out, bytes=0)
         L.check(self.lib.iris_step_dlpack(
-            self._ctx, C.byref(scfg), u.ctypes.data, streams, L.dlpack_pointer(features_capsule),
+            self._ctx, C.byref(scfg), u.ctypes.data, streams, fptr,
             L.dlpack_pointer(frame_capsule) if frame_capsule is not None else None, self._stream()))
 
     # ---- multi-GPU: the count all-reduce (NCCL inside libiris) ----

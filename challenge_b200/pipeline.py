@@ -90,7 +90,7 @@ class IrisDataset:
     def _lower(self, allow_mel=True):
         """Split the stage list into what the fused kernel absorbs and the remainder."""
         fused = dict(frame_labels=False, density_labels=False, augment=False, remap=L.REMAP_NONE, n_out=0, filt=0,
-                     mode=L.FEAT_COMPLEX, n_mels=0, mel_matrix=None)
+                     mode=L.FEAT_COMPLEX, n_mels=0, mel_matrix=None, out_flag=0)
         rest = []
         state = 'pre'       # pre-batch element stages -> post-batch feature stages
         order = {'to_frame_labels': 0, 'density_labels': 0, 'augment': 1, 'stereo_mono': 2, 'merge_aug': 2,
@@ -132,6 +132,8 @@ class IrisDataset:
                 fused['mode'] = L.FEAT_LOGMEL_MINMAX          # trainer.minmax_log_on_mel
             elif state == 'post' and tag and tag[0] == 'log_on_mel' and fused['mode'] == L.FEAT_MEL:
                 fused['mode'] = L.FEAT_LOGMEL
+            elif state == 'post' and tag and tag[0] == 'cast' and fused['out_flag'] == 0:
+                fused['out_flag'] = tag[1]                    # data_utils.cast_features: the kernels store it
             else:
                 rest.append(st)
             i += 1
@@ -168,7 +170,7 @@ class IrisDataset:
                           src['min_ratio'], src['min_noise_ratio'],
                           6 if fused['augment'] else 0, 24, 1 if fused['augment'] else 0, 16, 257,
                           max(fused['n_out'] - 2, 0) if fused['remap'] == L.REMAP_MERGE_AUG else 0)
-        return src['engine'].step_config(cfg, fused['mode'], stft_filter=fused['filt'],
+        return src['engine'].step_config(cfg, fused['mode'] | fused['out_flag'], stft_filter=fused['filt'],
                                          chan_remap=fused['remap'], n_out_chan=fused['n_out'])
 
     def __iter__(self):

@@ -49,6 +49,15 @@ enum {
     IRIS_FEAT_LOGMEL_MINMAX = 5  /* [B,n_mel,T,C'] + minmax + log_on_mel (sj_train.py:119-123)  */
 };
 
+/* Output element type, OR-ed into the mode of iris_features, iris_features_select,
+ * iris_features_dlpack, iris_plan_bytes(_clips) and into iris_step_config.feature_mode.  Without a
+ * flag the features are float32.  With one, the output buffer holds 2-byte elements in the same
+ * layout, equal bit for bit to the float32 features converted with round-to-nearest-even (torch's
+ * .to(torch.bfloat16 / torch.float16); float16 overflow gives +-inf).  All arithmetic stays float32.
+ * Both flags at once, or any other bit above the low 8, is IRIS_ERR_INVALID (as it is for a library
+ * that predates the flags, so callers can detect support). */
+enum { IRIS_OUT_BF16 = 0x100, IRIS_OUT_F16 = 0x200 };
+
 enum { IRIS_REMAP_NONE = 0, IRIS_REMAP_STEREO_MONO = 1, IRIS_REMAP_MERGE_AUG = 2 };
 
 int iris_abi_version(void);
@@ -129,7 +138,9 @@ int iris_plan_upload(iris_ctx* ctx, const iris_plan* plan, iris_stream stream);
 int iris_labels(iris_ctx* ctx, float* d_labels_vtk, float* d_frame_labels, uint8_t* d_keep,
                 iris_stream stream);
 
-/* The fused feature kernel for the uploaded plan; d_out sized per the mode's layout. */
+/* The fused feature kernel for the uploaded plan; d_out sized per the mode's layout, 16-byte aligned.
+ * mode: IRIS_FEAT_* | optional IRIS_OUT_BF16 / IRIS_OUT_F16, in which case d_out points at 2-byte
+ * elements (bfloat16 / float16) in the same layout. */
 int iris_features(iris_ctx* ctx, int mode, float* d_out, iris_stream stream);
 
 /* merge_complex_specs(seperate_noise_voice=True) (pipeline.py:37-38, 82-83, 104-108): the same
@@ -137,7 +148,8 @@ int iris_features(iris_ctx* ctx, int mode, float* d_out, iris_stream stream);
  * masks, remap or filter: these are labels of the 'se' model, sj_train.py:99-105).
  *   IRIS_SELECT_VOICES   only_voice = sum of the accepted voices
  *   IRIS_SELECT_BG_NOISE only_noise = background + noises
- * IRIS_SELECT_ALL is iris_features(). */
+ * IRIS_SELECT_ALL is iris_features().  mode (IRIS_FEAT_COMPLEX for a selection) takes the
+ * IRIS_OUT_* flags as iris_features does, d_out then holding 2-byte elements. */
 enum { IRIS_SELECT_ALL = 0, IRIS_SELECT_VOICES = 1, IRIS_SELECT_BG_NOISE = 2 };
 int iris_features_select(iris_ctx* ctx, int mode, int select, float* d_out, iris_stream stream);
 
@@ -167,8 +179,9 @@ int iris_er_counts_pooled(iris_ctx* ctx, const float* d_y_true, int n_frame, con
                           int n_frame_pred, int batch, int n_classes, float threshold,
                           int32_t* d_triples, float* d_er, iris_stream stream);
 
-/* Algorithmic HBM bytes of the last uploaded plan for `mode` (SURVEY.md 8d): 4 * (samples of
- * every kept source frame range read + output elements); used by bench.py's roofline. */
+/* Algorithmic HBM bytes of the last uploaded plan for `mode` (SURVEY.md 8d): 4 * samples of
+ * every kept source frame range read, plus 4 (2 with an IRIS_OUT_* flag in `mode`) * output
+ * elements; used by bench.py's roofline. */
 int iris_plan_bytes(iris_ctx* ctx, int mode, const uint8_t* host_keep, int64_t* bytes_in,
                     int64_t* bytes_out);
 /* The same for the clips [clip_lo, clip_hi) of the plan. */
@@ -375,7 +388,7 @@ typedef struct iris_step_config {
     int32_t stft_filter;      /* data_utils.stft_filter(k); 0 = off */
     int32_t chan_remap;       /* IRIS_REMAP_* */
     int32_t n_out_chan;       /* channels after remap */
-    int32_t feature_mode;     /* IRIS_FEAT_* */
+    int32_t feature_mode;     /* IRIS_FEAT_* | optional IRIS_OUT_BF16 / IRIS_OUT_F16 */
 } iris_step_config;
 
 typedef void* iris_nccl_comm; /* ncclComm_t */
@@ -383,7 +396,8 @@ typedef void* iris_nccl_comm; /* ncclComm_t */
 typedef struct iris_step_io {
     const double* uniforms;   /* HOST [batch, iris_draw_uniforms_per_clip(&cfg->draw)] */
     iris_shuffle* const* streams; /* [3] (bg, voice, noise) or NULL */
-    float* d_features;        /* DEVICE, layout of cfg->feature_mode */
+    float* d_features;        /* DEVICE, layout of cfg->feature_mode, 16-byte aligned; 2-byte
+                                 elements with an IRIS_OUT_* flag */
     float* d_frame_labels;    /* DEVICE [B,T,K] or NULL (to_frame_labels, data_utils.py:64-70) */
     float* d_labels_vtk;      /* DEVICE [B,V,T,K] or NULL (make_pipeline's label output) */
     uint8_t* d_keep;          /* DEVICE [B,V] or NULL */
@@ -448,8 +462,11 @@ int iris_host_free(iris_ctx* ctx, void* p, size_t bytes);
 /* ---- DLPack hand-over (the exchange format north_star names) ----
  * `managed` points at a DLManagedTensor (dlpack.h ABI: the struct behind the "dltensor"
  * capsule of torch.utils.dlpack.to_dlpack / tf.experimental.dlpack.to_dlpack).  The entry points
- * check device, dtype (float32), contiguity and shape against the plan and then write through
- * data + byte_offset: the tensor stays owned by the producing framework, nothing is copied. */
+ * check device, dtype, contiguity and shape against the plan and then write through
+ * data + byte_offset: the tensor stays owned by the producing framework, nothing is copied.  The
+ * dtype is float32 except for features with an IRIS_OUT_* flag in `mode` / cfg->feature_mode:
+ * bfloat16 (kDLBfloat, 16 bits) for IRIS_OUT_BF16, float16 (kDLFloat, 16 bits) for IRIS_OUT_F16.  A
+ * dtype that does not match the flag is IRIS_ERR_INVALID and nothing is written. */
 int iris_features_dlpack(iris_ctx* ctx, int mode, void* managed, iris_stream stream);
 int iris_labels_dlpack(iris_ctx* ctx, void* managed_vtk, void* managed_frame, iris_stream stream);
 int iris_step_dlpack(iris_ctx* ctx, const iris_step_config* cfg, const double* uniforms,

@@ -15,7 +15,7 @@ extern "C" {
 #endif
 
 enum { kDLCPU = 1, kDLCUDA = 2, kDLCUDAHost = 3, kDLCUDAManaged = 13 };
-enum { kDLInt = 0, kDLUInt = 1, kDLFloat = 2 };
+enum { kDLInt = 0, kDLUInt = 1, kDLFloat = 2, kDLBfloat = 4 };
 
 typedef struct {
     int32_t device_type;
