@@ -127,7 +127,7 @@ int run_labels(iris_ctx* c, float* d_vtk, float* d_frame, uint8_t* d_keep_out, c
     if (feat_hint >= IRIS_FEAT_COMPLEX && feat_hint <= IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode &&
         !getenv("IRIS_NO_LABEL_TILES")) {
         const bool mel = feat_hint >= IRIS_FEAT_MEL;
-        if (!(mel && (c->n_mel == 0 || !c->mel_fusable || c->remap != IRIS_REMAP_NONE)))
+        if (!(mel && (c->n_mel == 0 || !c->mel_fusable)))
             tiles = feature_params(c, feat_hint, IRIS_SELECT_ALL, fp) == IRIS_OK;
     }
     CU(launch_labels(lp, st, tiles ? &fp : nullptr));
@@ -218,7 +218,7 @@ int timed_fused(iris_ctx* c, FusedParams& p, int mode, cudaStream_t st, int out_
 // in place at d_out == p.out), or for bfloat16 / float16 features k_logmel_post_to from the fp32
 // scratch at p.out into d_out
 int run_logmel_minmax(iris_ctx* c, FusedParams& p, void* d_out, cudaStream_t st, int out_type) {
-    const size_t per_clip = size_t(c->n_mel) * c->T * c->C;
+    const size_t per_clip = size_t(c->n_mel) * c->T * p.c_out;
     uint32_t* mm = c->minmax.as<uint32_t>();
     unsigned* done = reinterpret_cast<unsigned*>(mm + 2 * size_t(c->B));
     int rc = timed_fused(c, p, FM_MEL, st, OUT_F32);
@@ -228,9 +228,9 @@ int run_logmel_minmax(iris_ctx* c, FusedParams& p, void* d_out, cudaStream_t st,
     return IRIS_OK;
 }
 
-// fp32 mel scratch [B, n_mel, T, C] of a half-width launch whose last pass converts
+// fp32 mel scratch [B, n_mel, T, c_out] of a half-width launch whose last pass converts
 int mel_scratch(iris_ctx* c, float** out) {
-    CU(c->mel_scratch.reserve(size_t(c->B) * c->n_mel * c->T * c->C * 4));
+    CU(c->mel_scratch.reserve(size_t(c->B) * c->n_mel * c->T * c->c_out * 4));
     *out = c->mel_scratch.as<float>();
     return IRIS_OK;
 }
@@ -268,8 +268,6 @@ int feature_params(iris_ctx* c, int mode, int select, FusedParams& p) {
 // (k_spec.cu), for the mel modes with the projection and the per-clip extrema fused in.
 int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t st, int out_type) {
     const bool mel = mode >= IRIS_FEAT_MEL;
-    if (mel && c->remap != IRIS_REMAP_NONE)
-        return fail(IRIS_ERR_UNSUPPORTED, "mel features with a channel remap run unfused");
     if (mel && c->mel_bins != kBins) return fail(IRIS_ERR_INVALID, "the mel matrix must have 257 rows");
     FusedParams p;
     fill_common(c, p);
@@ -294,8 +292,8 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         CU(launch_specmix(p, mode, nullptr, nullptr, nullptr, st, out_type));
         return IRIS_OK;
     }
-    const size_t per_clip = size_t(c->n_mel) * c->T * c->C;
-    if (specmix_mel_smem(c->C, c->mel_f_n) <= 200 * 1024) {
+    const size_t per_clip = size_t(c->n_mel) * c->T * c->c_out;   // mel channels: after the remap
+    if (specmix_mel_smem(c->c_out, c->mel_f_n) <= 200 * 1024) {
         // fused: mix -> |.| -> mel -> per-clip extrema in one pass; k_logmel_post normalises in L2
         p.out = d_out;
         p.do_log = mode != IRIS_FEAT_MEL;
@@ -318,9 +316,9 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         else if (p.do_minmax) CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
         return IRIS_OK;
     }
-    // many channels: magnitudes through a scratch spectrogram, then the stand-alone kernels (fp32; for
-    // bfloat16 / float16 features the mel goes to a scratch and the last pass converts)
-    CU(c->spec_scratch.reserve(size_t(c->B) * kBins * c->T * 2 * c->C * 4));
+    // many channels: magnitudes through a scratch spectrogram (remapped by store_bin), then the stand-alone
+    // kernels (fp32; for bfloat16 / float16 features the mel goes to a scratch and the last pass converts)
+    CU(c->spec_scratch.reserve(size_t(c->B) * kBins * c->T * 2 * c->c_out * 4));
     p.out = c->spec_scratch.as<float>();
     CU(launch_specmix(p, FM_MAGPHASE, nullptr, nullptr, nullptr, st, OUT_F32));
     float* mel_out = d_out;
@@ -329,7 +327,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         if (rc) return rc;
     }
     CU(launch_mel_project(p.out, c->mel_dense.as<float>(), c->mel_lo.as<int32_t>(), c->mel_len.as<int32_t>(),
-                          mel_out, c->B, kBins, c->T, c->C, c->n_mel, st));
+                          mel_out, c->B, kBins, c->T, c->c_out, c->n_mel, st));
     if (mode == IRIS_FEAT_LOGMEL_MINMAX) {
         int rc = iris_op_minmax(c, 0, mel_out, mel_out, c->B, int64_t(per_clip), 1, st);
         if (rc) return rc;
@@ -1057,8 +1055,6 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
         return fail(IRIS_ERR_UNSUPPORTED,
                     "a mel filter wider than 16 bins (or more than 64 taps over the 32-filter rounds): run "
                     "IRIS_FEAT_MAGPHASE + iris_op_mel instead of the fused mel epilogue");
-    if (mel && c->remap != IRIS_REMAP_NONE)
-        return fail(IRIS_ERR_UNSUPPORTED, "mel features with a channel remap run unfused");
     FusedParams p;
     rc = feature_params(c, mode, select, p);
     if (rc) return rc;
@@ -1212,7 +1208,7 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
         in += samples * 4 * c->C;
     }
     int64_t out;
-    if (mode >= IRIS_FEAT_MEL) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->C * out_elem;
+    if (mode >= IRIS_FEAT_MEL) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->c_out * out_elem;
     else out = int64_t(clip_hi - clip_lo) * kBins * c->T * 2 * c->c_out * out_elem;
     if (bytes_in) *bytes_in = in;
     if (bytes_out) *bytes_out = out;

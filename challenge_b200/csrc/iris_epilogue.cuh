@@ -5,6 +5,21 @@
 
 namespace iris {
 
+// Output channel c >= 2 of a channel remap of a 2-channel clip (data_utils.py:79-82, 100-117) from the
+// real parts r0, r1 of the two input channels and the sum of their imaginary parts: stereo_mono
+// X0 + X1; random_merge_aug (f re0 + sqrt(1 - f) re1, im0 + im1) with fa = f, sf = sqrt(1 - f) of the
+// clip and channel.  Channels 0 and 1 are the inputs themselves.
+__device__ __forceinline__ cpx remap_mix(int remap, float fa, float sf, float r0, float r1, float isum) {
+    if (remap == REMAP_STEREO_MONO) return cpx{r0 + r1, isum};
+    return cpx{fa * r0 + sf * r1, isum};
+}
+// (fa, sf) of output channel c >= 2 of clip b (random_merge_aug; unused by stereo_mono)
+__device__ __forceinline__ float2 remap_coef(const FusedParams& p, int b, int c) {
+    if (p.remap == REMAP_STEREO_MONO) return make_float2(1.f, 1.f);
+    const size_t i = size_t(b) * (p.c_out - 2) + (c - 2);
+    return make_float2(p.merge_f[i], p.merge_sf[i]);
+}
+
 // One (bin f, frame t, channel pair) of the output: (r0, i0) / (r1, i1) are the complex values of
 // channels 2*pair and 2*pair + 1, m the product of the SpecAugment masks of this cell.  OutT: the
 // element type of p.out (iris_common.cuh, store_out*).
@@ -51,12 +66,17 @@ __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, in
             float re, im;
             if (c == 0) { re = r0; im = i0; }
             else if (c == 1) { re = r1; im = i1; }
-            else if (p.remap == REMAP_STEREO_MONO) { re = r0 + r1; im = i0 + i1; }
-            else {
+            // (one branch per remap with the remap a constant: a single remap_mix(p.remap, remap_coef(..))
+            // call moves the registers of the spectrogram-mode k_specmix instances and gives the half
+            // ones a stack frame)
+            else if (p.remap == REMAP_STEREO_MONO) {
+                const cpx z = remap_mix(REMAP_STEREO_MONO, 1.f, 1.f, r0, r1, i0 + i1);
+                re = z.x; im = z.y;
+            } else {
                 const float fa = p.merge_f[size_t(b) * (Co - 2) + (c - 2)];
                 const float sf = p.merge_sf[size_t(b) * (Co - 2) + (c - 2)];
-                re = fa * r0 + sf * r1;
-                im = i0 + i1;
+                const cpx z = remap_mix(REMAP_MERGE_AUG, fa, sf, r0, r1, i0 + i1);
+                re = z.x; im = z.y;
             }
             if (p.filter_k > 0) { re *= filt; im *= filt; }
             float a = re, ph = im;

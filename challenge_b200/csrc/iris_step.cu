@@ -170,7 +170,7 @@ int dl_device_ptr(iris_ctx* c, void* managed, const int64_t* want_shape, int wan
 // mode: the base mode (IRIS_FEAT_*)
 void feature_shape(const iris_ctx* c, int mode, int64_t (&shape)[4]) {
     shape[0] = c->B;
-    if (mode >= IRIS_FEAT_MEL) { shape[1] = c->n_mel; shape[2] = c->T; shape[3] = c->C; }
+    if (mode >= IRIS_FEAT_MEL) { shape[1] = c->n_mel; shape[2] = c->T; shape[3] = c->c_out; }   // after the remap
     else { shape[1] = kBins; shape[2] = c->T; shape[3] = 2 * c->c_out; }
 }
 
@@ -605,7 +605,7 @@ int iris_step_dlpack(iris_ctx* c, const iris_step_config* cfg, const double* uni
     if (cfg->chan_remap == IRIS_REMAP_STEREO_MONO) c_out = 3;
     else if (cfg->chan_remap == IRIS_REMAP_MERGE_AUG) c_out = cfg->n_out_chan;
     int64_t fs[4] = {g.batch, kBins, g.n_frame, 2 * c_out};
-    if (base_mode >= IRIS_FEAT_MEL) { fs[1] = c->n_mel; fs[3] = bg.n_chan; }
+    if (base_mode >= IRIS_FEAT_MEL) { fs[1] = c->n_mel; fs[3] = c_out; }
     iris_step_io io;
     memset(&io, 0, sizeof io);
     io.uniforms = uniforms;

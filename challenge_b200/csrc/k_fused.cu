@@ -169,9 +169,11 @@ __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, 
 // with their switches fixed at compile time (EPI_C2 | EPI_MINMAX or EPI_LOG or neither): no
 // per-round flag branches, no odd-channel selects, C folded into the address arithmetic, the
 // projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.
+// EPI_REMAP: the mel epilogue of a channel remap (stereo_mono / random_merge_aug: 2 input channels, c_out
+// output channels), switches read at run time like EPI == 0.
 // OutT: element type of p.out (float, __nv_bfloat16, __half).  The half instances have no min-max
 // epilogue: the min-max log-mel features are normalised by k_logmel_post, which converts.
-constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4;
+constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4, EPI_REMAP = 8;
 constexpr int kFixFR = 8;   // frames per tile of the fixed mel variants
 __host__ __device__ constexpr int fixed_mel_L(int r) { return r == 0 ? 2 : (r == 1 ? 4 : (r == 2 ? 6 : 0)); }
 template <int MODE, int NJ, int EPI, class OutT>
@@ -181,14 +183,17 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
     // clip; the consumer warps are never more than S <= 3 tiles apart, 8 entries never collide
     __shared__ uint32_t s_mm[8][4];
     constexpr bool kMel = (MODE == FM_MEL);
-    constexpr bool kFix = (EPI != 0);      // switches below are compile-time constants
+    constexpr bool kFix = (EPI & EPI_C2) != 0;   // switches below are compile-time constants
+    constexpr bool kRemap = (EPI == EPI_REMAP);
     static_assert(!kFix || kMel, "fixed epilogues exist for the mel modes only");
+    static_assert(!kRemap || kMel, "the remap epilogue is a mel epilogue");
     constexpr bool kF32 = sizeof(OutT) == 4;
     static_assert(kF32 || (MODE != FM_ACTIVITY && !(EPI & EPI_MINMAX)), "activity flags and the min-max epilogue are fp32 only");
     constexpr int S = slots_of(MODE);      // stage buffers
     const bool do_minmax = !kF32 ? false : kFix ? bool(EPI & EPI_MINMAX) : (p.do_minmax != 0);
     const bool do_lg = kFix ? bool(EPI & EPI_LOG) : (p.do_log && !p.do_minmax);
     const int C = kFix ? 2 : p.C;
+    const int Cm = kRemap ? p.c_out : C;   // channels of the mel output
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
     // fixed variants: 8 frames per tile and the 12 taps of the default mel shape, so that the
@@ -402,7 +407,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
         OutT* clip_out = reinterpret_cast<OutT*>(p.out);   // out[b, 0, 0, 0] of the current clip (mel modes)
         uint32_t zbits = 0;
         int zb_clip = -1;
-        const size_t clip_elems = size_t(p.n_mel) * p.T * C;
+        const size_t clip_elems = size_t(p.n_mel) * p.T * Cm;
         for (int i = 0;; ++i) {
             const TileBlock* tb = reinterpret_cast<const TileBlock*>(sm + OFF_RING + (i & (kRing - 1)) * kTileBlockBytes);
             // ---- gather + mix: v = sum over the stages of this tile of gain * frame ----
@@ -531,7 +536,133 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 const cpx mine = l0 ? u[(16 - jj) & 15] : u[15 - jj];
                 return cpx{__shfl_sync(0xffffffffu, mine.x, partner), __shfl_sync(0xffffffffu, mine.y, partner)};
             };
-            if (kMel) {
+            if (kRemap) {
+                // ---- mel of a channel remap: output pair q = channels (2q, 2q + 1) of c_out.  Pair 0 is the
+                // two input channels; the others are per-bin linear combinations of them (remap_mix), so a
+                // mask or stft_filter zero of a bin zeroes every output channel of it.  Each round of 32
+                // filters is stored as soon as it is summed (no accumulators held across the rounds).
+                //   NJ = 4: the magnitudes of kG = 4 pairs at a time are parked in the exchange rows (128
+                //   float2 per pair, indexed by the bin), from (re ch0, re ch1, im ch0 + im ch1) of the
+                //   lane's 4 bins kept in registers.
+                //   NJ = 8: those 27 registers spill the FFT; the exchange rows hold (re ch0, re ch1, im ch0,
+                //   im ch1) of all 257 bins instead (4112 B) and the projection forms the magnitudes of a
+                //   pair from them tap by tap.
+                if (do_minmax && b != mm_clip) {
+                    if (mm_clip >= 0) flush_minmax();
+                    mm_clip = b;
+                }
+                constexpr int kS = 128;
+                constexpr int kG = NJ == 4 ? 4 : 1;
+                static_assert(4 * 128 * 8 <= kXwBytes && kBins * 16 <= kXwBytes, "exchange rows too small");
+                float2* mg = reinterpret_cast<float2*>(xch);
+                float4* xv = reinterpret_cast<float4*>(xch);
+                const uint32_t* ms = reinterpret_cast<const uint32_t*>(sm + OFF_MSTART) + lane;
+                const int n_op = (Cm + 1) >> 1;
+                float xr0[4], xr1[4], xis[4];   // NJ = 4: re ch0, re ch1, im ch0 + im ch1 of the lane's bins
+                if (do_fft) {   // warp-uniform
+                    auto split = [&](int i, int f, cpx zf, cpx zm) {
+                        const cpx re = cadd(zf, zm);
+                        const cpx im = cadd(cpx{zf.y, -zf.x}, cpx{-zm.y, zm.x});
+                        const bool z = (zbits >> i) & 1u;
+                        if constexpr (NJ == 4) {
+                            const cpx sq = cfma2(im, im, cmul2(re, re));
+                            mg[f] = make_float2(z ? 0.f : sqrt_approx(sq.x), z ? 0.f : sqrt_approx(sq.y));
+                            xr0[i] = z ? 0.f : re.x;
+                            xr1[i] = z ? 0.f : re.y;
+                            xis[i] = z ? 0.f : im.x + im.y;
+                        } else {
+                            xv[f] = z ? make_float4(0.f, 0.f, 0.f, 0.f) : make_float4(re.x, re.y, im.x, im.y);
+                        }
+                    };
+#pragma unroll
+                    for (int jj = 0; jj < NJ; ++jj) split(jj, k1 + 16 * (2 * jj + par), u[jj], mirror(jj));
+                    if (NJ == 8) {
+                        const cpx z8 = u[8];
+                        if (l0) split(8, 256, z8, z8);
+                    }
+                }
+                for (int g0 = 0; g0 < n_op; g0 += kG) {
+                    if (NJ == 4 && do_fft) {
+                        if (g0 > 0) __syncwarp();   // the previous group is projected
+                        for (int k = (g0 == 0 ? 1 : 0); k < kG && g0 + k < n_op; ++k) {
+                            const int ca = 2 * (g0 + k), cb = ca + 1;
+                            const float2 ka = remap_coef(p, b, ca), kb = cb < Cm ? remap_coef(p, b, cb) : ka;
+#pragma unroll
+                            for (int i = 0; i < 4; ++i) {
+                                const cpx za = remap_mix(p.remap, ka.x, ka.y, xr0[i], xr1[i], xis[i]);
+                                const cpx zb = remap_mix(p.remap, kb.x, kb.y, xr0[i], xr1[i], xis[i]);
+                                mg[k * kS + k1 + 16 * (2 * i + par)] =
+                                    make_float2(sqrt_approx(fmaf(za.x, za.x, za.y * za.y)),
+                                                sqrt_approx(fmaf(zb.x, zb.x, zb.y * zb.y)));
+                            }
+                        }
+                    }
+                    if (do_fft) __syncwarp();
+                    for (int k = 0; k < kG && g0 + k < n_op; ++k) {
+                        const int c = 2 * (g0 + k);
+                        const bool has_b = c + 1 < Cm;
+                        // NJ = 8: |.| of channels c, c + 1 of bin f from the parked split values
+                        const float2 ka = c >= 2 ? remap_coef(p, b, c) : make_float2(0.f, 0.f);
+                        const float2 kb = c >= 2 && has_b ? remap_coef(p, b, c + 1) : ka;
+                        auto tap = [&](int f) -> float2 {
+                            if constexpr (NJ == 4) {
+                                return mg[k * kS + f];
+                            } else {
+                                const float4 v = xv[f];
+                                if (c == 0)
+                                    return make_float2(sqrt_approx(fmaf(v.x, v.x, v.z * v.z)),
+                                                       sqrt_approx(fmaf(v.y, v.y, v.w * v.w)));
+                                const cpx za = remap_mix(p.remap, ka.x, ka.y, v.x, v.y, v.z + v.w);
+                                const cpx zb = remap_mix(p.remap, kb.x, kb.y, v.x, v.y, v.z + v.w);
+                                return make_float2(sqrt_approx(fmaf(za.x, za.x, za.y * za.y)),
+                                                   sqrt_approx(fmaf(zb.x, zb.x, zb.y * zb.y)));
+                            }
+                        };
+                        // sparse projection as in the 2-channel epilogue below, then out[b, m, t, c .. c + 1]
+                        const float* wr = reinterpret_cast<const float*>(sm + OFF_MW) + lane;
+                        OutT* o_t = clip_out + t * Cm + c;
+                        const uint32_t row_elems = uint32_t(p.T) * uint32_t(Cm);
+#pragma unroll
+                        for (int r = 0; r < 4; ++r) {
+                            const int L = p.mel_L[r];   // uniform
+                            if (L == 0) break;
+                            cpx sacc{0.f, 0.f};
+                            if (do_fft) {
+                                const int f0 = p.mel_f_lo + int(ms[32 * r] & 0xffffu);
+#pragma unroll
+                                for (int q = 0; q < kMaxFilter; q += 2) {
+                                    if (q >= L) break;
+                                    const float2 x0 = tap(f0 + q), x1 = tap(f0 + q + 1);
+                                    sacc = caxpy(wr[32 * q], cpx{x0.x, x0.y}, sacc);
+                                    sacc = caxpy(wr[32 * q + 32], cpx{x1.x, x1.y}, sacc);
+                                }
+                            }
+                            wr += 32 * L;
+                            const uint32_t mrow = ms[32 * r] >> 16;
+                            if (in_range && mrow != 0xffffu) {
+                                OutT* o = o_t + mrow * row_elems;
+                                float a0 = sacc.x, a1 = sacc.y;
+                                if (do_minmax) {
+                                    mn = fminf(mn, has_b ? fminf(a0, a1) : a0);
+                                    mx = fmaxf(mx, has_b ? fmaxf(a0, a1) : a0);
+                                }
+                                if (do_lg) {
+                                    a0 = __logf(a0 + 1e-8f);
+                                    a1 = __logf(a1 + 1e-8f);
+                                }
+                                // (plain stores: the evict-last hint of the 2-channel epilogue costs
+                                // registers this epilogue does not have)
+                                if ((Cm & 1) == 0) {
+                                    store_out2(o, a0, a1);
+                                } else {
+                                    store_out1(o, a0);
+                                    if (has_b) store_out1(o + 1, a1);
+                                }
+                            }
+                        }
+                    }
+                }
+            } else if (kMel) {
                 if (do_minmax && b != mm_clip) {
                     if (mm_clip >= 0) flush_minmax();
                     mm_clip = b;
@@ -789,7 +920,8 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     const long long n_tiles = (long long)p.B * p.n_pairs * tpc;
     if (n_tiles <= 0) return cudaSuccess;
     if (n_tiles > 0x7fffffffLL || p.max_segs > kMaxStages || p.n_pairs > 127) return cudaErrorInvalidValue;
-    if (mode == FM_MEL && (long long)p.n_mel * p.T * p.C > 0x7fffffffLL) return cudaErrorInvalidValue;   // 32-bit row offsets inside a clip
+    if (mode == FM_MEL && (long long)p.n_mel * p.T * p.c_out > 0x7fffffffLL) return cudaErrorInvalidValue;   // 32-bit row offsets inside a clip
+    if (mode == FM_MEL && p.remap != REMAP_NONE && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
     const size_t smem = fused_smem_bytes(p, mode);
     if (smem > 227 * 1024 - 256) return cudaErrorInvalidValue;   // (128 B of static shared memory: s_mm)
     if (out_type != OUT_F32 && ((out_type != OUT_BF16 && out_type != OUT_F16) || mode == FM_ACTIVITY || p.do_minmax))
@@ -857,7 +989,11 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         case FM_MAGPHASE: IRIS_LAUNCH_OUT(FM_MAGPHASE, 8, 0) break;
         case FM_LOGMAGPHASE: IRIS_LAUNCH_OUT(FM_LOGMAGPHASE, 8, 0) break;
         case FM_MEL:
-            if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
+            // a remap keeps p.C == 2: it must be tested before the fixed 2-channel instances
+            if (p.remap != REMAP_NONE) {
+                if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_REMAP)
+                else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_REMAP)
+            } else if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
             else if (p.C != 2 || p.mel_L[0] != fixed_mel_L(0) || p.mel_L[1] != fixed_mel_L(1) ||
                      p.mel_L[2] != fixed_mel_L(2) || p.mel_L[3] != fixed_mel_L(3) ||
                      FR != kFixFR || p.mel_taps != 12 || getenv("IRIS_NO_FIXED_EPI"))

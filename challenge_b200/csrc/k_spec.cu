@@ -42,8 +42,8 @@ __global__ void k_spec_activity(const float* __restrict__ specs, const int64_t* 
 // bytes (2 channels).  The clip's segments that are kept and overlap the tile are compacted,
 // in the reference's order, into shared memory once per CTA.
 //   spectrogram modes: the cell goes through store_bin (masks, remap, filter, mag / phase).
-//   FM_MEL: |.| of the masked, filtered cell is parked in shared memory [257][32][C]; after the
-//   walk the CTA projects its 32 frames on the mel filters (dense matrix, non-zero rows
+//   FM_MEL: |.| of the masked, filtered cell (every output channel of a remap) is parked in shared
+//   memory [257][32][c_out]; after the walk the CTA projects its 32 frames on the mel filters (dense matrix, non-zero rows
 //   [lo, lo + len) per filter; transforms.py:51-77), stores [n_mel][32 frames] rows of 128 /
 //   256 contiguous bytes and reduces the per-clip extrema for the min-max pass (k_post.cu).
 constexpr int kSpecTile = 32;      // frames per CTA
@@ -64,6 +64,7 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
     const int t = t0 + lane;
     const bool live = t < p.T;
     const int C = p.C, W = 2 * C;
+    const int Cm = p.c_out;   // FM_MEL: channels of the magnitudes (C, or c_out of a channel remap)
     const int g0 = p.seg_ptr[b], g1 = p.seg_ptr[b + 1];
 
     if (warp == 0) {   // ordered compaction of the segments this tile needs
@@ -103,7 +104,7 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
     }
     // FM_MEL: only the bin rows that carry a non-zero mel weight are read at all
     // ([mel_f_lo, mel_f_lo + mel_f_n): bins 4..122 of 257 for the TF default matrix)
-    float* mags = reinterpret_cast<float*>(sm_raw);   // [mel_f_n][32][C]
+    float* mags = reinterpret_cast<float*>(sm_raw);   // [mel_f_n][32][Cm]
     const int f_begin = MODE == FM_MEL ? p.mel_f_lo : 0;
     const int f_end = MODE == FM_MEL ? p.mel_f_lo + p.mel_f_n : kBins;
 
@@ -182,9 +183,19 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                     const float filt = (f >= 1 && f <= p.filter_k) ? 0.f : 1.f;   // data_utils.py:126-136
                     const float mm = m[u] * filt;
                     const float a0 = r0[u] * mm, b0 = i0[u] * mm, a1 = r1[u] * mm, b1 = i1[u] * mm;
-                    float* o = mags + (size_t(f - f_begin) * kSpecTile + lane) * C + 2 * pair;
+                    float* o = mags + (size_t(f - f_begin) * kSpecTile + lane) * Cm + 2 * pair;
                     o[0] = sqrt_approx(fmaf(a0, a0, b0 * b0));   // transforms.py:116
                     if (has1) o[1] = sqrt_approx(fmaf(a1, a1, b1 * b1));
+                    // channel remap (C == 2, one pair): the other output channels from the masked, filtered
+                    // inputs (zeros before the remap are zeros after it; the filter follows it in the
+                    // reference).  Without a remap Cm == C and every channel is an input channel.
+                    if (p.remap != REMAP_NONE) {
+                        for (int c = 2; c < Cm; ++c) {
+                            const float2 k = remap_coef(p, b, c);
+                            const cpx z = remap_mix(p.remap, k.x, k.y, a0, a1, b0 + b1);
+                            o[c] = sqrt_approx(fmaf(z.x, z.x, z.y * z.y));
+                        }
+                    }
                 } else if (live) {
                     store_bin<MODE, OutT>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
                 }
@@ -198,14 +209,14 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
     const bool lg = p.do_log && !p.do_minmax;
     for (int mi = warp; mi < p.n_mel; mi += kSpecWarps) {
         const int f0 = mel_lo[mi] - f_begin, f1 = f0 + mel_len[mi];
-        for (int c = 0; c < C; ++c) {
+        for (int c = 0; c < Cm; ++c) {
             float acc = 0.f;
             for (int f = f0; f < f1; ++f)
-                acc = fmaf(mags[(size_t(f) * kSpecTile + lane) * C + c], __ldg(melW + size_t(f + f_begin) * p.n_mel + mi), acc);
+                acc = fmaf(mags[(size_t(f) * kSpecTile + lane) * Cm + c], __ldg(melW + size_t(f + f_begin) * p.n_mel + mi), acc);
             if (live) {
                 mn = fminf(mn, acc);
                 mx = fmaxf(mx, acc);
-                store_out1(reinterpret_cast<OutT*>(p.out) + ((size_t(b) * p.n_mel + mi) * p.T + t) * C + c,
+                store_out1(reinterpret_cast<OutT*>(p.out) + ((size_t(b) * p.n_mel + mi) * p.T + t) * Cm + c,
                            lg ? __logf(acc + 1e-8f) : acc);
             }
         }
@@ -242,7 +253,8 @@ static cudaError_t launch_specmix_t(const FusedParams& p, int mode, const float*
         case FM_MAGPHASE: k_specmix<FM_MAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
         case FM_LOGMAGPHASE: k_specmix<FM_LOGMAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
         case FM_MEL: {
-            const size_t smem = specmix_mel_smem(p.C, p.mel_f_n);
+            if (p.remap != REMAP_NONE && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
+            const size_t smem = specmix_mel_smem(p.c_out, p.mel_f_n);
             if (smem > 200 * 1024) return cudaErrorInvalidValue;
             static bool attr_set = false;   // per instance
             if (!attr_set) {
@@ -259,7 +271,7 @@ static cudaError_t launch_specmix_t(const FusedParams& p, int mode, const float*
     return cudaGetLastError();
 }
 
-// mode FM_MEL: p.out [B, n_mel, T, C], p.do_log / p.do_minmax / p.minmax as in the fused kernel;
+// mode FM_MEL: p.out [B, n_mel, T, c_out], p.do_log / p.do_minmax / p.minmax as in the fused kernel;
 // melW dense [257, n_mel] with the non-zero rows [lo, lo + len) of every filter.  out_type: OutType
 // of p.out (the min-max mel features are fp32: k_logmel_post normalises them).
 cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,

@@ -233,7 +233,7 @@ class Engine:
     def feature_shape(self, mode):
         pl = self._plan
         if int(mode) & L.MODE_MASK >= L.FEAT_MEL:
-            return (pl['B'], self.n_mel, pl['T'], self.bank_chan)
+            return (pl['B'], self.n_mel, pl['T'], pl['c_out'])   # channels after the remap
         return (pl['B'], 257, pl['T'], 2 * pl['c_out'])
 
     def features(self, mode, out=None, select=L.SELECT_ALL, dtype=None):

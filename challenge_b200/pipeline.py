@@ -121,8 +121,7 @@ class IrisDataset:
                 state = 'post'
             elif state == 'post' and tag and tag[0] == 'magphase' and fused['mode'] == L.FEAT_COMPLEX:
                 fused['mode'] = L.FEAT_MAGPHASE
-            elif state == 'post' and allow_mel and tag and tag[0] == 'mel' and fused['mode'] == L.FEAT_MAGPHASE \
-                    and fused['remap'] == L.REMAP_NONE:
+            elif state == 'post' and allow_mel and tag and tag[0] == 'mel' and fused['mode'] == L.FEAT_MAGPHASE:
                 fused['mode'], fused['n_mels'], fused['mel_matrix'] = L.FEAT_MEL, tag[1], tag[2]
             elif state == 'post' and tag and tag[0] == 'minmax' and fused['mode'] == L.FEAT_MEL \
                     and i + 1 < len(stages) and getattr(stages[i + 1], '_iris_stage', (None,))[0] == 'log_on_mel':

@@ -39,7 +39,10 @@ enum {
 
 enum { IRIS_BANK_BG = 0, IRIS_BANK_VOICE = 1, IRIS_BANK_NOISE = 2 };
 
-/* feature modes of iris_features(); layouts as in the reference */
+/* feature modes of iris_features(); layouts as in the reference.  C' is the channel count after the
+ * plan's channel remap (3 for stereo_mono, n_out_chan for random_merge_aug, else the bank's), in the
+ * spectrogram and the mel layouts alike: a remap is fused in front of the mel projection.  (A library
+ * older than that answers the mel modes of a remapped plan with IRIS_ERR_UNSUPPORTED.) */
 enum {
     IRIS_FEAT_COMPLEX = 0,       /* [B,257,T,2C']  make_pipeline output (pipeline.py:131-133)  */
     IRIS_FEAT_MAGPHASE = 1,      /* [B,257,T,2C']  complex_to_magphase (transforms.py:111-123)  */
