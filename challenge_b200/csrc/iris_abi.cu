@@ -124,9 +124,9 @@ int run_labels(iris_ctx* c, float* d_vtk, float* d_frame, uint8_t* d_keep_out, c
     lp.keep = c->keep.as<uint8_t>();
     FusedParams fp;
     bool tiles = false;
-    if (feat_hint >= IRIS_FEAT_COMPLEX && feat_hint <= IRIS_FEAT_LOGMEL_MINMAX && !c->spec_mode &&
-        !getenv("IRIS_NO_LABEL_TILES")) {
-        const bool mel = feat_hint >= IRIS_FEAT_MEL;
+    if (((feat_hint >= IRIS_FEAT_COMPLEX && feat_hint <= IRIS_FEAT_LOGMEL_MINMAX) || feat_hint == IRIS_FEAT_SE) &&
+        !c->spec_mode && !getenv("IRIS_NO_LABEL_TILES")) {
+        const bool mel = mel_mode(feat_hint);
         if (!(mel && (c->n_mel == 0 || !c->mel_fusable)))
             tiles = feature_params(c, feat_hint, IRIS_SELECT_ALL, fp) == IRIS_OK;
     }
@@ -238,7 +238,7 @@ int mel_scratch(iris_ctx* c, float** out) {
 // FusedParams of a feature launch from waveform banks: everything but the output pointer and the
 // min-max scratch, including the tile-block scratch and its layout (prepare_fused)
 int feature_params(iris_ctx* c, int mode, int select, FusedParams& p) {
-    const bool mel = mode >= IRIS_FEAT_MEL;
+    const bool mel = mel_mode(mode);
     fill_common(c, p);
     p.segs = c->d_segs;
     p.seg_ptr = c->d_seg_ptr;
@@ -257,17 +257,23 @@ int feature_params(iris_ctx* c, int mode, int select, FusedParams& p) {
         p.filter_k = 0; p.remap = IRIS_REMAP_NONE; p.c_out = c->C;
         set_geometry(c, p, c->C, false);
     }
+    if (mode == IRIS_FEAT_SE) {   // two virtual channel pairs over bank pair 0: voices | background + noises
+        if (c->C != 2 || c->remap != IRIS_REMAP_NONE)
+            return fail(IRIS_ERR_UNSUPPORTED, "IRIS_FEAT_SE takes 2-channel plans without a channel remap");
+        p.seg_select = 3;
+        set_geometry(c, p, 4, false);
+    }
     if (mel) {
         p.do_log = mode != IRIS_FEAT_MEL;
         p.do_minmax = mode == IRIS_FEAT_LOGMEL_MINMAX;
     }
-    return prepare_fused(c, p, mel ? FM_MEL : mode, c->max_segs);
+    return prepare_fused(c, p, mel ? FM_MEL : mode == IRIS_FEAT_SE ? FM_SE : mode, c->max_segs);
 }
 
 // Features from spectrogram banks: the mix + per-cell epilogue is one streaming kernel
 // (k_spec.cu), for the mel modes with the projection and the per-clip extrema fused in.
 int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t st, int out_type) {
-    const bool mel = mode >= IRIS_FEAT_MEL;
+    const bool mel = mel_mode(mode);
     if (mel && c->mel_bins != kBins) return fail(IRIS_ERR_INVALID, "the mel matrix must have 257 rows");
     FusedParams p;
     fill_common(c, p);
@@ -289,7 +295,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
     }
     if (!mel) {
         p.out = d_out;
-        CU(launch_specmix(p, mode, nullptr, nullptr, nullptr, st, out_type));
+        CU(launch_specmix(p, mode == IRIS_FEAT_SE ? FM_SE : mode, nullptr, nullptr, nullptr, st, out_type));
         return IRIS_OK;
     }
     const size_t per_clip = size_t(c->n_mel) * c->T * c->c_out;   // mel channels: after the remap
@@ -1033,14 +1039,18 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
     int out_type = OUT_F32;
     if (!split_feature_mode(mode, &mode, &out_type))
         return fail(IRIS_ERR_INVALID, "bad feature mode: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the mode");
+    if (mode == IRIS_FEAT_SE && out_type != OUT_F32)
+        return fail(IRIS_ERR_INVALID, "IRIS_FEAT_SE writes float32 blocks: no IRIS_OUT_* flag");
     if (reinterpret_cast<uintptr_t>(d_out) & 15)
         return fail(IRIS_ERR_INVALID, "the feature buffer must be 16-byte aligned (vector stores)");
     if (select < IRIS_SELECT_ALL || select > IRIS_SELECT_BG_NOISE) return fail(IRIS_ERR_INVALID, "bad segment selection");
     if (select != IRIS_SELECT_ALL && mode != IRIS_FEAT_COMPLEX)
         return fail(IRIS_ERR_INVALID, "only_voice / only_noise are complex spectrograms (pipeline.py:37-38)");
     if (!c->has_plan) return fail(IRIS_ERR_STATE, "no plan uploaded");
-    if (mode < IRIS_FEAT_COMPLEX || mode > IRIS_FEAT_LOGMEL_MINMAX)
+    if ((mode < IRIS_FEAT_COMPLEX || mode > IRIS_FEAT_LOGMEL_MINMAX) && mode != IRIS_FEAT_SE)
         return fail(IRIS_ERR_INVALID, "bad feature mode");
+    if (mode == IRIS_FEAT_SE && (c->C != 2 || c->remap != IRIS_REMAP_NONE))
+        return fail(IRIS_ERR_UNSUPPORTED, "IRIS_FEAT_SE takes 2-channel plans without a channel remap");
     int rc = set_device(c);
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1048,7 +1058,7 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
         rc = run_labels(c, nullptr, nullptr, nullptr, st, select == IRIS_SELECT_ALL ? mode : -1);
         if (rc) return rc;
     }
-    const bool mel = mode >= IRIS_FEAT_MEL;
+    const bool mel = mel_mode(mode);
     if (mel && c->n_mel == 0) return fail(IRIS_ERR_STATE, "iris_set_mel not called");
     if (c->spec_mode) return spec_features(c, mode, select, d_out, st, out_type);
     if (mel && !c->mel_fusable)
@@ -1075,7 +1085,7 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
         rc = p.do_minmax ? run_logmel_minmax(c, p, d_out, st, out_type) : timed_fused(c, p, FM_MEL, st, out_type);
         if (rc) return rc;
     } else {
-        rc = timed_fused(c, p, mode, st, out_type);
+        rc = timed_fused(c, p, mode == IRIS_FEAT_SE ? FM_SE : mode, st, out_type);
     }
     if (rc) return rc;
     return IRIS_OK;
@@ -1191,6 +1201,8 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
     int out_type = OUT_F32;
     if (!split_feature_mode(mode, &mode, &out_type))
         return fail(IRIS_ERR_INVALID, "bad feature mode: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the mode");
+    if (mode == IRIS_FEAT_SE && out_type != OUT_F32)
+        return fail(IRIS_ERR_INVALID, "IRIS_FEAT_SE writes float32 blocks: no IRIS_OUT_* flag");
     const int64_t out_elem = out_type == OUT_F32 ? 4 : 2;
     int64_t in = 0;
     for (size_t i = size_t(c->h_seg_ptr[clip_lo]); i < size_t(c->h_seg_ptr[clip_hi]); ++i) {
@@ -1200,7 +1212,7 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
         // never more than the source holds
         if (c->spec_mode) {   // [257, frames, 2C] cells of the frames the segment covers
             // the mel modes need only the bin rows that carry a non-zero mel weight
-            const int rows = mode >= IRIS_FEAT_MEL ? c->mel_f_n : kBins;
+            const int rows = mel_mode(mode) ? c->mel_f_n : mode == IRIS_FEAT_SE ? kBins - 1 : kBins;
             in += int64_t(s.t_hi - s.t_lo) * rows * 2 * c->C * 4;
             continue;
         }
@@ -1208,7 +1220,8 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
         in += samples * 4 * c->C;
     }
     int64_t out;
-    if (mode >= IRIS_FEAT_MEL) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->c_out * out_elem;
+    if (mode == IRIS_FEAT_SE) out = int64_t(clip_hi - clip_lo) * (kBins - 1) * c->T * 2 * c->C * out_elem;   // C + C/2 + C/2
+    else if (mel_mode(mode)) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->c_out * out_elem;
     else out = int64_t(clip_hi - clip_lo) * kBins * c->T * 2 * c->c_out * out_elem;
     if (bytes_in) *bytes_in = in;
     if (bytes_out) *bytes_out = out;

@@ -32,6 +32,7 @@ enum FusedMode : int {
     FM_LOGMAGPHASE = 2,
     FM_MEL = 3,
     FM_ACTIVITY = 4,
+    FM_SE = 5,   // IRIS_FEAT_SE: x, only_voice, only_noise of the 'se' model (include/iris.h)
 };
 
 enum ChanRemap : int { REMAP_NONE = 0, REMAP_STEREO_MONO = 1, REMAP_MERGE_AUG = 2 };
@@ -97,7 +98,8 @@ struct FusedParams {
     int32_t n_big, n_mid;        // claim schedule (launch_fused): n_big claims of `chunk` tiles, n_mid of
     int32_t chunk_mid, chunk_tail;   // `chunk_mid`, the rest `chunk_tail`
     int32_t seg_select;          // 0: every segment; 1: voices only; 2: background + noises only
-                                 // (only_voice / only_noise of pipeline.py:37-38, 82-83, 104-108)
+                                 // (only_voice / only_noise of pipeline.py:37-38, 82-83, 104-108);
+                                 // 3 (FM_SE): channel pair q of a tile is bank pair 0 restricted as by q + 1
     uint32_t* sched;             // [2] next chunk, CTAs finished; zero between launches
     // outputs
     float* out;             // layout depends on mode

@@ -65,6 +65,9 @@ struct Bank {
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// the IRIS_FEAT_* modes with a mel projection (IRIS_FEAT_SE, numbered after them, has none)
+inline bool mel_mode(int mode) { return mode >= IRIS_FEAT_MEL && mode <= IRIS_FEAT_LOGMEL_MINMAX; }
+
 // mode argument of the feature entry points: IRIS_FEAT_* in the low 8 bits, at most one IRIS_OUT_*
 // flag above them.  false: any other high bit (the base mode is range-checked by the caller).
 inline bool split_feature_mode(int mode, int* base, int* out_type) {

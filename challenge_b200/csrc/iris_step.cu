@@ -566,7 +566,8 @@ int iris_features_dlpack(iris_ctx* c, int mode, void* managed, iris_stream strea
     if (!c->has_plan) return fail(IRIS_ERR_STATE, "no plan uploaded");
     int base = 0, out_type = OUT_F32;
     if (!split_feature_mode(mode, &base, &out_type) || base < IRIS_FEAT_COMPLEX || base > IRIS_FEAT_LOGMEL_MINMAX)
-        return fail(IRIS_ERR_INVALID, "bad feature mode");
+        return fail(IRIS_ERR_INVALID, base == IRIS_FEAT_SE ? "IRIS_FEAT_SE has three output blocks: one DLPack tensor cannot "
+                                                             "describe them (use iris_features)" : "bad feature mode");
     int64_t shape[4];
     feature_shape(c, base, shape);
     float* out = nullptr;
@@ -601,6 +602,8 @@ int iris_step_dlpack(iris_ctx* c, const iris_step_config* cfg, const double* uni
     int base_mode = 0, out_type = OUT_F32;
     if (!split_feature_mode(cfg->feature_mode, &base_mode, &out_type))
         return fail(IRIS_ERR_INVALID, "iris_step_dlpack: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the feature mode");
+    if (base_mode == IRIS_FEAT_SE)
+        return fail(IRIS_ERR_INVALID, "IRIS_FEAT_SE has three output blocks: one DLPack tensor cannot describe them (use iris_step)");
     int c_out = bg.n_chan;
     if (cfg->chan_remap == IRIS_REMAP_STEREO_MONO) c_out = 3;
     else if (cfg->chan_remap == IRIS_REMAP_MERGE_AUG) c_out = cfg->n_out_chan;

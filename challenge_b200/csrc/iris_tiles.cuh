@@ -49,6 +49,9 @@ __host__ __device__ inline long long claim_range(int chunk, int chunk_mid, int c
 // seg_cache / keep_cache / tm_cache / fm_cache: the clip's segments, their keep flags (1 = kept or not a
 // voice) and its mask rectangles staged in shared memory by the caller (k_labels), or null: read them
 // from the plan.
+// SE: the layout of FM_SE (p.seg_select == 3), two virtual channel pairs over bank pair 0: pair 0 takes the
+// kept voices, pair 1 background + noises.  (A compile-time variant: a run-time select spills k_labels.)
+template <bool SE = false>
 __device__ __forceinline__ void build_tile_block(const FusedParams& p, int tile, int per_clip,
                                                  const Seg* seg_cache = nullptr, const uint8_t* keep_cache = nullptr,
                                                  const int32_t* tm_cache = nullptr, const int32_t* fm_cache = nullptr) {
@@ -70,10 +73,12 @@ __device__ __forceinline__ void build_tile_block(const FusedParams& p, int tile,
         const int lo = max(sg.t_lo, t0), hi = min(sg.t_hi, t_end);
         const bool kept = seg_cache ? keep_cache[s - s0] != 0 : !(sg.keep_idx >= 0 && p.keep[sg.keep_idx] == 0);
         if (lo >= hi || !kept) continue;
-        if ((p.seg_select == 1 && sg.keep_idx < 0) || (p.seg_select == 2 && sg.keep_idx >= 0)) continue;
+        if (SE ? ((sg.keep_idx >= 0) != (pair == 0))
+               : ((p.seg_select == 1 && sg.keep_idx < 0) || (p.seg_select == 2 && sg.keep_idx >= 0)))
+            continue;
         if (n < p.max_segs) {
             StageDesc e;
-            e.src = sg.base + size_t(pair) * size_t(sg.pair_stride) + size_t(lo + sg.shift) * 512;
+            e.src = sg.base + size_t(SE ? 0 : pair) * size_t(sg.pair_stride) + size_t(lo + sg.shift) * 512;
             e.j_lo = uint16_t(lo - t0);
             e.j_cnt = uint16_t(hi - lo);
             e.gain = 0.5f * sg.gain;   // exact; folds the 1/2 of the two-channel split

@@ -98,7 +98,8 @@ __global__ void __launch_bounds__(128) k_tiles(const FusedParams p) {
         p.minmax[2 * tile] = 0u;
         p.minmax[2 * tile + 1] = 0u;
     }
-    build_tile_block(p, tile, per_clip);
+    if (p.seg_select == 3) build_tile_block<true>(p, tile, per_clip);
+    else build_tile_block(p, tile, per_clip);
 }
 
 // one (bin, frame, channel pair) of the spectrogram modes without a channel remap:
@@ -768,6 +769,52 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) mxv = fmaxf(mxv, __shfl_xor_sync(0xffffffffu, mxv, o));
                 if (in_range && l0 && mxv > 0.f) p.activity[size_t(b) * p.T + t] = 1;
+            } else if (MODE == FM_SE) {
+                // ---- the 'se' batch (include/iris.h, IRIS_FEAT_SE): the tile's channel pair 0 is the mix of the
+                // kept voices, pair 1 background + noises (build_tile_block, seg_select 3); consecutive tiles of
+                // this CTA, as in the 4-channel combined store below.  Pair 0 parks (Re V0, Re V1) in the staging
+                // area, pair 1 parks (Re N0, Re N1, mask) in its exchange rows; the store phase of pair 1 writes,
+                // for bins 1..256, x = (V + N) * mask * filter, only_voice = Re V0, only_noise = Re N0.  Every
+                // in-range frame runs the FFT: the masks zero x only.
+                float4* stg = reinterpret_cast<float4*>(slots + S * slotB);
+                float4* park = pair == 1 ? reinterpret_cast<float4*>(xch) : stg;
+                if (do_fft) {
+#pragma unroll
+                    for (int jj = 0; jj < 8; ++jj) {
+                        const int f = k1 + 16 * (2 * jj + par);
+                        const cpx zf = u[jj], zm = mirror(jj);
+                        park[pair == 1 ? (f ^ j) : f * FR + (j ^ (f & 7))] =
+                            make_float4(zf.x + zm.x, zf.y + zm.y, ((zbits >> jj) & 1u) ? 0.f : mt, 0.f);
+                    }
+                    if (l0) {
+                        const cpx zf = u[8];
+                        park[pair == 1 ? (256 ^ j) : 256 * FR + j] =
+                            make_float4(zf.x + zf.x, zf.y + zf.y, ((zbits >> 8) & 1u) ? 0.f : mt, 0.f);
+                    }
+                }
+                if (pair == 1) {   // warp-uniform (tile header)
+                    named_bar_sync(1, FR * 32);
+                    const int jt = lane & 7;
+                    const int tt = (hdr.z & 0xffffff) + jt;
+                    if (tt < p.T) {
+                        const size_t cells = size_t(p.B) * 256 * p.T;   // (bin, frame) cells of one block channel
+                        float* ov = p.out + 2 * cells;
+                        float* on = ov + cells;
+                        const unsigned char* x1 = sm + off_xch(mel_taps) + jt * kXwBytes;
+                        for (int f = warp * 4 + (lane >> 3); f < kBins; f += FR * 4) {
+                            if (f == 0) continue;
+                            const float4 v = stg[f * FR + (jt ^ (f & 7))];
+                            const float4 n = *reinterpret_cast<const float4*>(x1 + ((f ^ jt) << 4));
+                            float a0 = (v.x + n.x) * n.z, a1 = (v.y + n.y) * n.z;   // masks by multiplication
+                            if (f <= p.filter_k) { a0 *= 0.f; a1 *= 0.f; }          // data_utils.py:126-136
+                            const size_t c = (size_t(b) * 256 + (f - 1)) * p.T + tt;
+                            *reinterpret_cast<float2*>(p.out + 2 * c) = make_float2(a0, a1);
+                            ov[c] = v.x;
+                            on[c] = n.x;
+                        }
+                    }
+                    named_bar_sync(1, FR * 32);   // staging + exchange rows are read before they are reused
+                }
             } else if (p.stage_out) {
                 // ---- spectrogram modes: every warp parks the 257 x 16 B pieces of its frame in
                 // the staging area, then the 8 warps store bin rows of 8 frames = 128 B each ----
@@ -1003,6 +1050,10 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
             else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2)
             break;
         case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0, float) break;
+        case FM_SE:   // both virtual pairs of a (clip, time) range in one CTA: the combined store
+            if (out_type != OUT_F32 || !p.pair_merge || p.seg_select != 3) return cudaErrorInvalidValue;
+            IRIS_LAUNCH(FM_SE, 8, 0, float)
+            break;
         default: return cudaErrorInvalidValue;
     }
 #undef IRIS_LAUNCH_OUT

@@ -17,6 +17,9 @@ namespace iris {
 // shared memory (one global round trip per clip instead of two per voice).
 // build_tiles: the CTA also writes the tile blocks of its clip (iris_tiles.cuh) for the k_fused
 // launch behind it: the keep flags it has just decided are their only input that is not in the plan.
+// SE: the tile blocks are those of an FM_SE launch (build_tile_block; its own instance, as the run-time
+// choice spills this kernel)
+template <bool SE>
 __global__ void __launch_bounds__(1024) k_labels(const LabelParams p, const int build_tiles,
                                                  const __grid_constant__ FusedParams fp) {
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -119,8 +122,8 @@ __global__ void __launch_bounds__(1024) k_labels(const LabelParams p, const int 
             __syncthreads();
         }
         for (int r = threadIdx.x; r < per_clip; r += blockDim.x)
-            build_tile_block(fp, b * per_clip + r, per_clip, seg_cached ? s_segs : nullptr, seg_cached ? s_kept : nullptr,
-                             seg_cached ? s_tm : nullptr, seg_cached ? s_fm : nullptr);
+            build_tile_block<SE>(fp, b * per_clip + r, per_clip, seg_cached ? s_segs : nullptr, seg_cached ? s_kept : nullptr,
+                                 seg_cached ? s_tm : nullptr, seg_cached ? s_fm : nullptr);
     }
 }
 
@@ -128,11 +131,13 @@ cudaError_t launch_labels(const LabelParams& p, cudaStream_t stream, const Fused
     if (p.B <= 0) return cudaSuccess;
     const size_t smem = (size_t(p.T) * p.K + size_t(p.V) * p.K) * 4 + size_t(p.V) * p.T;
     if (smem > 200 * 1024 || p.V > 64) return cudaErrorInvalidValue;
-    static bool attr_set = false;
-    if (smem > 48 * 1024 && !attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(k_labels, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    const bool se = tiles && tiles->seg_select == 3;
+    static bool attr_set[2] = {false, false};
+    if (smem > 48 * 1024 && !attr_set[se]) {
+        cudaError_t e = cudaFuncSetAttribute(se ? k_labels<true> : k_labels<false>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) return e;
-        attr_set = true;
+        attr_set[se] = true;
     }
     // 1024 threads per clip: one frame per thread, so the sequential per-voice passes are a
     // handful of instructions per warp (256 threads measured 17 us, latency-bound)
@@ -143,7 +148,8 @@ cudaError_t launch_labels(const LabelParams& p, cudaStream_t stream, const Fused
     // several waves and the kernel is latency-bound per CTA, so half-size CTAs (four per SM) finish sooner
     // (1024 clips: step 0.82 -> 0.81 ms; 256 clips: 226.3 vs 226.7 us)
     const int threads = p.B > 296 ? 512 : 1024;
-    k_labels<<<p.B, threads, smem, stream>>>(p, tiles ? 1 : 0, tiles ? *tiles : none);
+    if (se) k_labels<true><<<p.B, threads, smem, stream>>>(p, 1, *tiles);
+    else k_labels<false><<<p.B, threads, smem, stream>>>(p, tiles ? 1 : 0, tiles ? *tiles : none);
     return cudaGetLastError();
 }
 

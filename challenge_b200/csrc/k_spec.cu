@@ -42,6 +42,9 @@ __global__ void k_spec_activity(const float* __restrict__ specs, const int64_t* 
 // bytes (2 channels).  The clip's segments that are kept and overlap the tile are compacted,
 // in the reference's order, into shared memory once per CTA.
 //   spectrogram modes: the cell goes through store_bin (masks, remap, filter, mag / phase).
+//   FM_SE: the 'se' batch (include/iris.h, IRIS_FEAT_SE): besides the mix, the kept voices and background +
+//   noises are summed into their own accumulators (the products and sums of the mix, so the three blocks are
+//   bit-identical to three selected launches); real parts of bins 1..256, masks and filter on x only.
 //   FM_MEL: |.| of the masked, filtered cell (every output channel of a remap) is parked in shared
 //   memory [257][32][c_out]; after the walk the CTA projects its 32 frames on the mel filters (dense matrix, non-zero rows
 //   [lo, lo + len) per filter; transforms.py:51-77), stores [n_mel][32 frames] rows of 128 /
@@ -105,7 +108,7 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
     // FM_MEL: only the bin rows that carry a non-zero mel weight are read at all
     // ([mel_f_lo, mel_f_lo + mel_f_n): bins 4..122 of 257 for the TF default matrix)
     float* mags = reinterpret_cast<float*>(sm_raw);   // [mel_f_n][32][Cm]
-    const int f_begin = MODE == FM_MEL ? p.mel_f_lo : 0;
+    const int f_begin = MODE == FM_MEL ? p.mel_f_lo : (MODE == FM_SE ? 1 : 0);
     const int f_end = MODE == FM_MEL ? p.mel_f_lo + p.mel_f_n : kBins;
 
     // U bin rows per warp iteration: their loads are issued together (the walk is latency-bound
@@ -126,9 +129,10 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
         for (int pair = 0; pair < p.n_pairs; ++pair) {
             const bool has1 = 2 * pair + 1 < C;
             float r0[U], r1[U], i0[U], i1[U];
+            float vr[U], nr[U];   // FM_SE: Re ch0 of the kept voices / of background + noises
 #pragma unroll
-            for (int u = 0; u < U; ++u) { r0[u] = 0.f; r1[u] = 0.f; i0[u] = 0.f; i1[u] = 0.f; }
-            bool first = true;
+            for (int u = 0; u < U; ++u) { r0[u] = 0.f; r1[u] = 0.f; i0[u] = 0.f; i1[u] = 0.f; vr[u] = 0.f; nr[u] = 0.f; }
+            bool first = true, v_first = true, n_first = true;
             if (live) {
                 for (int s = 0; s < n_seg; ++s) {
                     Seg sg;
@@ -173,6 +177,18 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                         }
                     }
                     first = false;
+                    if (MODE == FM_SE) {   // the same products, summed per subset in the same order
+                        const bool voice = sg.keep_idx >= 0;
+                        const bool sf = voice ? v_first : n_first;
+#pragma unroll
+                        for (int u = 0; u < U; ++u) {
+                            const float g = __fmul_rn(sg.gain, x0[u]);
+                            if (voice) vr[u] = sf ? g : __fadd_rn(vr[u], g);
+                            else nr[u] = sf ? g : __fadd_rn(nr[u], g);
+                        }
+                        if (voice) v_first = false;
+                        else n_first = false;
+                    }
                 }
             }
 #pragma unroll
@@ -195,6 +211,18 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                             const cpx z = remap_mix(p.remap, k.x, k.y, a0, a1, b0 + b1);
                             o[c] = sqrt_approx(fmaf(z.x, z.x, z.y * z.y));
                         }
+                    }
+                } else if (MODE == FM_SE) {
+                    if (live) {
+                        // x as store_bin forms it: masks, then the filter, by multiplication
+                        float a0 = r0[u] * m[u], a1 = r1[u] * m[u];
+                        if (f <= p.filter_k) { a0 *= 0.f; a1 *= 0.f; }   // data_utils.py:126-136 (f >= 1)
+                        const size_t cells = size_t(p.B) * 256 * p.T;
+                        const size_t c = (size_t(b) * 256 + (f - 1)) * p.T + t;
+                        float* o = reinterpret_cast<float*>(p.out);
+                        *reinterpret_cast<float2*>(o + 2 * c) = make_float2(a0, a1);
+                        o[2 * cells + c] = vr[u];
+                        o[3 * cells + c] = nr[u];
                     }
                 } else if (live) {
                     store_bin<MODE, OutT>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
@@ -279,6 +307,12 @@ cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, co
     if (p.B <= 0 || p.T <= 0) return cudaSuccess;
     if (p.B > 65535) return cudaErrorInvalidValue;
     if (out_type != OUT_F32 && p.do_minmax) return cudaErrorInvalidValue;
+    if (mode == FM_SE) {   // fp32, 2 channels, no remap; every segment kept (the subsets are split per cell)
+        if (out_type != OUT_F32 || p.C != 2 || p.remap != REMAP_NONE || p.seg_select != 0) return cudaErrorInvalidValue;
+        dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
+        k_specmix<FM_SE, float><<<grid, kSpecWarps * 32, 0, st>>>(p, nullptr, nullptr, nullptr);
+        return cudaGetLastError();
+    }
     switch (out_type) {
         case OUT_F32: return launch_specmix_t<float>(p, mode, melW, mel_lo, mel_len, st);
         case OUT_BF16: return launch_specmix_t<__nv_bfloat16>(p, mode, melW, mel_lo, mel_len, st);

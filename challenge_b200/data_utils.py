@@ -220,6 +220,7 @@ def speech_enhancement_preprocess(x, y=None):
 
 augment._iris_stage = ('augment',)
 to_frame_labels._iris_stage = ('to_frame_labels',)
+speech_enhancement_preprocess._iris_stage = ('se',)
 stereo_mono._iris_stage = ('stereo_mono',)
 minmax._iris_stage = ('minmax',)
 log_on_mel._iris_stage = ('log_on_mel',)

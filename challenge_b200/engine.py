@@ -231,28 +231,57 @@ class Engine:
         return frame, vtk, keep
 
     def feature_shape(self, mode):
+        """Shape of the features of ``mode``; for FEAT_SE the shapes of its three blocks (x, only_voice,
+        only_noise)."""
         pl = self._plan
+        if int(mode) & L.MODE_MASK == L.FEAT_SE:
+            C = self.bank_chan
+            return tuple((pl['B'], 256, pl['T'], c) for c in (C, C // 2, C // 2))
         if int(mode) & L.MODE_MASK >= L.FEAT_MEL:
             return (pl['B'], self.n_mel, pl['T'], pl['c_out'])   # channels after the remap
         return (pl['B'], 257, pl['T'], 2 * pl['c_out'])
+
+    def _feature_buffer(self, mode, out, dtype):
+        """-> (buffer the library writes, what the caller gets).  FEAT_SE: one flat buffer, returned as the
+        contiguous views (x, only_voice, only_noise); ``out`` is then a flat tensor of their total size."""
+        shape = self.feature_shape(mode)
+        if int(mode) & L.MODE_MASK != L.FEAT_SE:
+            if out is None:
+                out = self._empty(shape, dtype)
+            else:
+                assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == dtype
+            return out, out
+        sizes = [int(np.prod(s)) for s in shape]
+        if out is None:
+            out = self._empty((sum(sizes),), dtype)
+        else:
+            assert out.numel() == sum(sizes) and out.is_contiguous() and out.is_cuda and out.dtype == dtype
+        flat = out.view(-1)
+        return out, tuple(v.view(s) for v, s in zip(flat.split(sizes), shape))
 
     def features(self, mode, out=None, select=L.SELECT_ALL, dtype=None):
         """``select``: SELECT_VOICES / SELECT_BG_NOISE give ``only_voice`` / ``only_noise`` of
         ``merge_complex_specs(seperate_noise_voice=True)`` (plain complex spectrograms).  ``dtype``:
         torch.float32 (default), torch.bfloat16 or torch.float16 -- the float32 features rounded to
-        nearest even by the kernel's store; default: the dtype of ``out``, else float32."""
+        nearest even by the kernel's store; default: the dtype of ``out``, else float32.  FEAT_SE returns
+        the tuple (x [B,256,T,C], only_voice [B,256,T,C//2], only_noise [B,256,T,C//2]) of views of one
+        buffer (float32 only)."""
         torch = _torch()
         pl = self._plan
         if dtype is None:
             dtype = out.dtype if out is not None else torch.float32
         mode = int(mode) | out_flag(dtype)
-        shape = self.feature_shape(mode) if select == L.SELECT_ALL else (pl['B'], 257, pl['T'], 2 * self.bank_chan)
-        if out is None:
-            out = self._empty(shape, dtype)
+        if select == L.SELECT_ALL:
+            out, res = self._feature_buffer(mode, out, dtype)
         else:
-            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == dtype
+            shape = (pl['B'], 257, pl['T'], 2 * self.bank_chan)
+            if out is None:
+                out = self._empty(shape, dtype)
+            else:
+                assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == dtype
+            res = out
         L.check(self.lib.iris_features_select(self._ctx, mode, int(select), self._ptr(out), self._stream()))
-        return out
+        return res
 
     # ---- one call per batch (iris_step) ----
     def step_config(self, draw_cfg, mode, stft_filter=0, chan_remap=L.REMAP_NONE, n_out_chan=0, out_dtype=None):
@@ -265,7 +294,8 @@ class Engine:
              triples_send=None, triples_global=None, global_batch=0, threshold=0.5):
         """ONE C call: draws from ``uniforms`` -> plan upload -> labels -> features, plus the metric
         leg (counting, count all-reduce) on the context's side stream when ``y_pred`` is given.
-        -> (features, frame_labels or None).  ``streams``: ``plan.stream_handles(...)``."""
+        -> (features, frame_labels or None); for FEAT_SE the features are the tuple of ``features``.
+        ``streams``: ``plan.stream_handles(...)``."""
         torch = _torch()
         g = scfg.draw
         B, T, V = g.batch, g.n_frame, g.max_voices
@@ -276,11 +306,7 @@ class Engine:
             c_out = int(scfg.n_out_chan)
         self._plan = dict(B=B, T=T, V=V, c_out=c_out, bytes=0)
         mode = scfg.feature_mode
-        shape = self.feature_shape(mode)
-        if out is None:
-            out = self._empty(shape, out_dtype(mode))
-        else:
-            assert tuple(out.shape) == shape and out.is_contiguous() and out.is_cuda and out.dtype == out_dtype(mode)
+        out, res = self._feature_buffer(mode, out, out_dtype(mode))
         if frame is None and want_frame and V > 0:
             frame = self._empty((B, T, self.n_classes))
         u = uniforms if uniforms.flags['C_CONTIGUOUS'] and uniforms.dtype == np.float64 \
@@ -305,7 +331,7 @@ class Engine:
                 io.d_triples_global = triples_global.data_ptr() if triples_global is not None else None
                 io.global_batch = int(global_batch)
         L.check(self.lib.iris_step(self._ctx, C.byref(scfg), C.byref(io), self._stream()))
-        return out, frame
+        return res, frame
 
     def counts_wait(self, lag=0):
         """The current stream waits for the metric leg issued ``lag`` steps ago."""

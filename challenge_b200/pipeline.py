@@ -17,8 +17,10 @@ that ``sj_train.make_dataset`` (sj_train.py:92-130) uses -- ``map``, ``batch``, 
 ``take``, ``repeat``, iteration.  Chaining the drop-in functions in sj_train's order
 (``to_frame_labels``, ``augment``, ``stereo_mono`` | ``random_merge_aug(n)``,
 ``stft_filter(k)``, ``batch``, ``complex_to_magphase``, ``magphase_to_mel(n)``, ``minmax``,
-``log_on_mel``) is recognised and lowered to ONE fused launch per batch; any other callable
-runs after it on the un-fused tensors (the stand-alone kernels), so arbitrary chains work.
+``log_on_mel``) is recognised and lowered to ONE fused launch per batch; so is the 'se' chain
+(``seperate_noise_voice=True``, [``augment``, ``stft_filter(k)``,] ``speech_enhancement_preprocess``,
+``batch``, sj_train.py:99-106) of 2-channel banks.  Any other callable runs after it on the un-fused
+tensors (the stand-alone kernels), so arbitrary chains work.
 """
 import numpy as np
 
@@ -117,6 +119,9 @@ class IrisDataset:
                     fused['remap'], fused['n_out'] = L.REMAP_MERGE_AUG, int(tag[1])
                 elif tag[0] == 'stft_filter':
                     fused['filt'] = int(tag[1])
+            elif state == 'pre' and tag and tag[0] == 'se' and self._se_fusable(fused, last, i):
+                fused['mode'] = L.FEAT_SE      # x, (frame labels, only_voice, only_noise) in one step
+                last = len(order)              # no pre-batch stage is absorbed behind it
             elif state == 'pre' and tag and tag[0] == 'batch':
                 state = 'post'
             elif state == 'post' and tag and tag[0] == 'magphase' and fused['mode'] == L.FEAT_COMPLEX:
@@ -131,19 +136,29 @@ class IrisDataset:
                 fused['mode'] = L.FEAT_LOGMEL_MINMAX          # trainer.minmax_log_on_mel
             elif state == 'post' and tag and tag[0] == 'log_on_mel' and fused['mode'] == L.FEAT_MEL:
                 fused['mode'] = L.FEAT_LOGMEL
-            elif state == 'post' and tag and tag[0] == 'cast' and fused['out_flag'] == 0:
+            elif state == 'post' and tag and tag[0] == 'cast' and fused['out_flag'] == 0 \
+                    and fused['mode'] != L.FEAT_SE:
                 fused['out_flag'] = tag[1]                    # data_utils.cast_features: the kernels store it
             else:
                 rest.append(st)
             i += 1
         return fused, rest
 
+    def _se_fusable(self, fused, last, i):
+        """``speech_enhancement_preprocess`` at stage ``i`` lowers to FEAT_SE: a ``seperate_noise_voice`` source
+        of 2-channel banks, the stage first before ``.batch()`` or behind ``augment`` / ``stft_filter`` only,
+        and, unbatched, the last stage."""
+        src = self._src
+        return bool(src.get('separate')) and src.get('n_chan') == 2 and last in (-1, 1, 3) \
+            and not fused['frame_labels'] and not fused['density_labels'] and fused['remap'] == L.REMAP_NONE \
+            and (self._batch is not None or i + 1 == len(self._stages))
+
     def _prepare(self):
         """Lower the stage list once per iteration: fused step configuration + leftover stages."""
         src = self._src
         eng = src['engine']
         fused, rest = self._lower()
-        if fused['mode'] >= L.FEAT_MEL:
+        if L.FEAT_MEL <= fused['mode'] <= L.FEAT_LOGMEL_MINMAX:
             cur = eng.mel_matrix
             if cur is None or cur.shape != fused['mel_matrix'].shape \
                     or not np.array_equal(cur, fused['mel_matrix']):
@@ -205,16 +220,20 @@ class IrisDataset:
                 b = min(B, elems_left)
                 elems_left -= b
             scfg, n_u = config_for(b)
-            want_vtk = not fused['frame_labels'] or fused['density_labels']
+            se = fused['mode'] == L.FEAT_SE
+            want_frame = fused['frame_labels'] or se
+            want_vtk = not want_frame or fused['density_labels']
             vtk = eng._empty((b, src['max_voices'], src['n_frame'], eng.n_classes)) if want_vtk else None
             # ONE C call: draws -> plan -> labels -> features (include/iris.h iris_step)
             x, frame = eng.step(scfg, O.rng().random((b, n_u)), streams=handles, vtk=vtk,
-                                want_frame=fused['frame_labels'])
+                                want_frame=want_frame)
             y = frame if fused['frame_labels'] else vtk
             if fused['density_labels']:
                 from .trainer import to_density_labels
                 _, y = to_density_labels(None, vtk)
-            if src.get('separate'):   # (label, only_voice, only_noise), pipeline.py:107-108
+            if se:                    # speech_enhancement_preprocess's (x, (frame labels, only_voice, only_noise))
+                x, y = x[0], (frame, x[1], x[2])
+            elif src.get('separate'):   # (label, only_voice, only_noise), pipeline.py:107-108
                 y = (y, eng.features(L.FEAT_COMPLEX, select=L.SELECT_VOICES),
                      eng.features(L.FEAT_COMPLEX, select=L.SELECT_BG_NOISE))
             if pre:
@@ -336,5 +355,6 @@ def make_pipeline(backgrounds,  # a list of background noises  (waveforms [chan,
                   max_voices=int(max_voices), max_noises=int(max_noises) if noises is not None else 0,
                   snr=kwargs.get('snr', -20), min_ratio=kwargs.get('min_ratio', 2 / 3),
                   min_noise_ratio=kwargs.get('min_noise_ratio', 1 / 2), streams=streams,
-                  separate=bool(kwargs.get('seperate_noise_voice', False)), spec_banks=spec_banks)
+                  separate=bool(kwargs.get('seperate_noise_voice', False)), spec_banks=spec_banks,
+                  n_chan=eng.bank_chan)
     return IrisDataset(source)

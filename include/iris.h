@@ -49,8 +49,22 @@ enum {
     IRIS_FEAT_LOG_MAGPHASE = 2,  /* [B,257,T,2C']  + log_magphase (transforms.py:80-86)         */
     IRIS_FEAT_MEL = 3,           /* [B,n_mel,T,C'] magphase_to_mel (transforms.py:51-77)        */
     IRIS_FEAT_LOGMEL = 4,        /* [B,n_mel,T,C'] + log_on_mel ('nominmax', sj_train.py:121)   */
-    IRIS_FEAT_LOGMEL_MINMAX = 5  /* [B,n_mel,T,C'] + minmax + log_on_mel (sj_train.py:119-123)  */
+    IRIS_FEAT_LOGMEL_MINMAX = 5, /* [B,n_mel,T,C'] + minmax + log_on_mel (sj_train.py:119-123)  */
+    IRIS_FEAT_SE = 6             /* the batch of the 'se' model, see below                      */
 };
+
+/* IRIS_FEAT_SE: merge_complex_specs(seperate_noise_voice=True) followed by
+ * speech_enhancement_preprocess (pipeline.py:37-38, 82-83, 104-108; data_utils.py:139-148), the chain of
+ * the 'se' model (sj_train.py:99-106), for a 2-channel plan without a channel remap.  The feature buffer
+ * holds three C-contiguous float32 blocks back to back, each starting 16-byte aligned:
+ *   x          [B,256,T,C]    real parts of bins 1..256 of the mix, after the plan's masks and stft_filter
+ *   only_voice [B,256,T,C/2]  real part of channel 0 of the sum of the kept voices
+ *   only_noise [B,256,T,C/2]  real part of channel 0 of background + noises
+ * (C/2 channels: the reference cuts the two label spectrograms after x was halved.)  Masks and
+ * stft_filter act on x only.  Other channel counts and remapped plans are IRIS_ERR_UNSUPPORTED; an
+ * IRIS_OUT_* flag, a selection other than IRIS_SELECT_ALL and the DLPack entry points are
+ * IRIS_ERR_INVALID (as is the mode itself for a library that predates it, so callers can probe for it).
+ * The frame labels of the batch come from iris_labels / iris_step as for every mode. */
 
 /* Output element type, OR-ed into the mode of iris_features, iris_features_select,
  * iris_features_dlpack, iris_plan_bytes(_clips) and into iris_step_config.feature_mode.  Without a
