@@ -14,7 +14,7 @@ IRIS_OK, IRIS_ERR_INVALID, IRIS_ERR_CUDA, IRIS_ERR_EMPTY_RANGE, IRIS_ERR_STATE, 
 BANK_BG, BANK_VOICE, BANK_NOISE = 0, 1, 2
 FEAT_COMPLEX, FEAT_MAGPHASE, FEAT_LOG_MAGPHASE, FEAT_MEL, FEAT_LOGMEL, FEAT_LOGMEL_MINMAX = range(6)
 FEAT_SE = 6   # x, only_voice, only_noise of the 'se' model: three blocks of one buffer (include/iris.h)
-REMAP_NONE, REMAP_STEREO_MONO, REMAP_MERGE_AUG = 0, 1, 2
+REMAP_NONE, REMAP_STEREO_MONO, REMAP_MERGE_AUG, REMAP_MONO_CHAN = 0, 1, 2, 3
 SELECT_ALL, SELECT_VOICES, SELECT_BG_NOISE = 0, 1, 2
 # output element type, OR-ed into a feature mode (none: float32)
 OUT_BF16, OUT_F16 = 0x100, 0x200

@@ -798,12 +798,15 @@ int iris_plan_upload(iris_ctx* c, const iris_plan* pl, iris_stream stream) {
     const int n_fm = pl->freq_masks ? pl->n_freq_masks : 0;
     if (n_tm < 0 || n_tm > 64) return fail(IRIS_ERR_UNSUPPORTED, "more than 64 time masks");
     if (n_fm < 0 || n_fm > 4) return fail(IRIS_ERR_UNSUPPORTED, "more than 4 frequency masks");
-    int c_out = C;
+    const int c_out = remap_channels(pl->chan_remap, C, pl->n_out_chan);
     if (pl->chan_remap != IRIS_REMAP_NONE) {
         // data_utils.py:104 -- ValueError('This augment can be used in 2 channel audio')
         if (C != 2) return fail(IRIS_ERR_INVALID, "channel remap needs 2-channel audio");
-        c_out = pl->chan_remap == IRIS_REMAP_STEREO_MONO ? 3 : pl->n_out_chan;
-        if (c_out < 3 || c_out > 16) return fail(IRIS_ERR_INVALID, "bad n_out_chan");
+        if (pl->chan_remap == IRIS_REMAP_MONO_CHAN) {
+            if (pl->n_out_chan != 2) return fail(IRIS_ERR_INVALID, "mono_chan: n_out_chan must be 2");
+        } else if (c_out < 3 || c_out > 16) {
+            return fail(IRIS_ERR_INVALID, "bad n_out_chan");
+        }
         if (pl->chan_remap == IRIS_REMAP_MERGE_AUG && !pl->merge_factor)
             return fail(IRIS_ERR_INVALID, "merge_factor NULL");
     }
@@ -1222,7 +1225,7 @@ int iris_plan_bytes_clips(iris_ctx* c, int mode, const uint8_t* host_keep, int c
     int64_t out;
     if (mode == IRIS_FEAT_SE) out = int64_t(clip_hi - clip_lo) * (kBins - 1) * c->T * 2 * c->C * out_elem;   // C + C/2 + C/2
     else if (mel_mode(mode)) out = int64_t(clip_hi - clip_lo) * c->n_mel * c->T * c->c_out * out_elem;
-    else out = int64_t(clip_hi - clip_lo) * kBins * c->T * 2 * c->c_out * out_elem;
+    else out = int64_t(clip_hi - clip_lo) * kBins * c->T * spec_width(mode, c->remap, c->c_out) * out_elem;
     if (bytes_in) *bytes_in = in;
     if (bytes_out) *bytes_out = out;
     return IRIS_OK;

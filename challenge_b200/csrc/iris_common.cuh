@@ -35,7 +35,7 @@ enum FusedMode : int {
     FM_SE = 5,   // IRIS_FEAT_SE: x, only_voice, only_noise of the 'se' model (include/iris.h)
 };
 
-enum ChanRemap : int { REMAP_NONE = 0, REMAP_STEREO_MONO = 1, REMAP_MERGE_AUG = 2 };
+enum ChanRemap : int { REMAP_NONE = 0, REMAP_STEREO_MONO = 1, REMAP_MERGE_AUG = 2, REMAP_MONO_CHAN = 3 };
 
 // element type of the feature output (IRIS_OUT_BF16 / IRIS_OUT_F16 of include/iris.h)
 enum OutType : int { OUT_F32 = 0, OUT_BF16 = 1, OUT_F16 = 2 };
@@ -78,7 +78,7 @@ struct FusedParams {
     int32_t B, T, C;         // clips, frames per clip, input channels
     int32_t n_pairs;         // ceil(C/2): a tile is `fr` frames of one (clip, channel pair)
     int32_t fr;              // frames per tile = consumer warps per CTA
-    int32_t c_out;           // output channels (C unless remapped)
+    int32_t c_out;           // output channels (C unless remapped; 2 pseudo-channels for mono_chan)
     // SpecAugment rectangles (size, offset) per clip; null => none
     const int32_t* tmask;
     int32_t n_tmask;

@@ -68,6 +68,19 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 // the IRIS_FEAT_* modes with a mel projection (IRIS_FEAT_SE, numbered after them, has none)
 inline bool mel_mode(int mode) { return mode >= IRIS_FEAT_MEL && mode <= IRIS_FEAT_LOGMEL_MINMAX; }
 
+// C' of include/iris.h: the channels after a plan's channel remap of n_chan bank channels
+inline int remap_channels(int remap, int n_chan, int n_out_chan) {
+    if (remap == IRIS_REMAP_NONE) return n_chan;
+    if (remap == IRIS_REMAP_STEREO_MONO) return 3;
+    if (remap == IRIS_REMAP_MONO_CHAN) return 2;
+    return n_out_chan;
+}
+// last axis of the spectrogram modes (base mode < IRIS_FEAT_MEL): 2 C', except the 3 columns of mono_chan's
+// complex spectrogram
+inline int spec_width(int mode, int remap, int c_out) {
+    return mode == IRIS_FEAT_COMPLEX && remap == IRIS_REMAP_MONO_CHAN ? 3 : 2 * c_out;
+}
+
 // mode argument of the feature entry points: IRIS_FEAT_* in the low 8 bits, at most one IRIS_OUT_*
 // flag above them.  false: any other high bit (the base mode is range-checked by the caller).
 inline bool split_feature_mode(int mode, int* base, int* out_type) {

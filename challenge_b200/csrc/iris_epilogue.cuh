@@ -1,6 +1,5 @@
 // Per-bin epilogue shared by the fused waveform kernel (k_fused.cu) and the spectrogram-bank
-// mix (k_spec.cu): masks, stft_filter, channel remaps, complex / mag-phase / log-mag-phase output.
-#pragma once
+// mix (k_spec.cu): masks, stft_filter, channel remaps, complex / mag-phase / log-mag-phase output.#pragma once
 #include "iris_common.cuh"
 
 namespace iris {
@@ -22,15 +21,38 @@ __device__ __forceinline__ float2 remap_coef(const FusedParams& p, int b, int c)
 
 // One (bin f, frame t, channel pair) of the output: (r0, i0) / (r1, i1) are the complex values of
 // channels 2*pair and 2*pair + 1, m the product of the SpecAugment masks of this cell.  OutT: the
-// element type of p.out (iris_common.cuh, store_out*).
-template <int MODE, class OutT>
+// element type of p.out (iris_common.cuh, store_out*).  kMono: the plan's remap is mono_chan, whose cells
+// have a layout of their own (a run-time branch for it caps the spectrogram-mode k_specmix instances at 64
+// registers, with spills).
+template <int MODE, class OutT, bool kMono>
 __device__ __forceinline__ void store_bin(const FusedParams& p, int b, int f, int t, int pair,
                                           bool has1, float r0, float i0, float r1, float i1,
                                           float m) {
     // masks are applied by multiplication (transforms.py:40) so zeros keep their sign
     r0 *= m; i0 *= m; r1 *= m; i1 *= m;
     const float filt = (f >= 1 && f <= p.filter_k) ? 0.f : 1.f;   // data_utils.py:126-136
-    if (p.remap == REMAP_NONE) {
+    if constexpr (kMono) {
+        // mono_chan (include/iris.h IRIS_REMAP_MONO_CHAN): the columns [re0 + re1, re0 + im0, re0 + im1] of
+        // the masked inputs, then stft_filter (the reference's order and rounding: the complex spectrogram of
+        // spectrogram banks is bit-identical); magnitude and phase of z_j = (re0 + re1) + i (re0 + im_j)
+        float s = __fadd_rn(r0, r1), y0 = __fadd_rn(r0, i0), y1 = __fadd_rn(r0, i1);
+        if (p.filter_k > 0) { s *= filt; y0 *= filt; y1 *= filt; }
+        const size_t cell = (size_t(b) * kBins + f) * p.T + t;
+        if (MODE == FM_COMPLEX) {
+            OutT* o = reinterpret_cast<OutT*>(p.out) + cell * 3;
+            store_out1(o, s);
+            store_out1(o + 1, y0);
+            store_out1(o + 2, y1);
+        } else {
+            float a0 = sqrt_approx(fmaf(s, s, y0 * y0));
+            float a1 = sqrt_approx(fmaf(s, s, y1 * y1));
+            if (MODE == FM_LOGMAGPHASE) {
+                a0 = __logf(a0 + 1e-8f);
+                a1 = __logf(a1 + 1e-8f);
+            }
+            store_out4(reinterpret_cast<OutT*>(p.out) + cell * 4, make_float4(a0, a1, fast_atan2f(y0, s), fast_atan2f(y1, s)));
+        }
+    } else if (p.remap == REMAP_NONE) {
         const int C = p.C;
         OutT* o = reinterpret_cast<OutT*>(p.out) + ((size_t(b) * kBins + f) * p.T + t) * size_t(2 * C);
         if (p.filter_k > 0) { r0 *= filt; i0 *= filt; r1 *= filt; i1 *= filt; }

@@ -92,9 +92,13 @@ int iris_op_pointwise(iris_ctx* c, int op, const float* x, float* out, int64_t r
     if (rc) return rc;
     if (!x || !out || rows < 0 || width < 1 || op < 0 || op > 4)
         return fail(IRIS_ERR_INVALID, "iris_op_pointwise: bad argument");
-    if (op <= IRIS_PW_MAGPHASE_TO_COMPLEX && (width & 1))
+    // complex_to_magphase of mono_chan's 3 columns: real [..., :1] broadcast against imag [..., 1:]
+    // (transforms.py:111-123) -> rows of 4; every other odd width is an error, as in TF
+    const bool bcast = op == IRIS_PW_COMPLEX_TO_MAGPHASE && width == 3;
+    if (op <= IRIS_PW_MAGPHASE_TO_COMPLEX && (width & 1) && !bcast)
         return fail(IRIS_ERR_INVALID, "iris_op_pointwise: last axis must be 2 * n_chan");
-    CU(launch_pointwise(op, x, out, size_t(rows), width / 2, width, param_i, param_f,
+    if (bcast && x == out) return fail(IRIS_ERR_INVALID, "iris_op_pointwise: rows of 3 -> 4 cannot be in place");
+    CU(launch_pointwise(op, x, out, size_t(rows), bcast ? 2 : width / 2, width, param_i, param_f,
                         static_cast<cudaStream_t>(stream)));
     return IRIS_OK;
 }

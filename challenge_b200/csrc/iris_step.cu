@@ -171,7 +171,7 @@ int dl_device_ptr(iris_ctx* c, void* managed, const int64_t* want_shape, int wan
 void feature_shape(const iris_ctx* c, int mode, int64_t (&shape)[4]) {
     shape[0] = c->B;
     if (mode >= IRIS_FEAT_MEL) { shape[1] = c->n_mel; shape[2] = c->T; shape[3] = c->c_out; }   // after the remap
-    else { shape[1] = kBins; shape[2] = c->T; shape[3] = 2 * c->c_out; }
+    else { shape[1] = kBins; shape[2] = c->T; shape[3] = spec_width(mode, c->remap, c->c_out); }
 }
 
 }  // namespace
@@ -604,10 +604,8 @@ int iris_step_dlpack(iris_ctx* c, const iris_step_config* cfg, const double* uni
         return fail(IRIS_ERR_INVALID, "iris_step_dlpack: at most one of IRIS_OUT_BF16 / IRIS_OUT_F16 above the feature mode");
     if (base_mode == IRIS_FEAT_SE)
         return fail(IRIS_ERR_INVALID, "IRIS_FEAT_SE has three output blocks: one DLPack tensor cannot describe them (use iris_step)");
-    int c_out = bg.n_chan;
-    if (cfg->chan_remap == IRIS_REMAP_STEREO_MONO) c_out = 3;
-    else if (cfg->chan_remap == IRIS_REMAP_MERGE_AUG) c_out = cfg->n_out_chan;
-    int64_t fs[4] = {g.batch, kBins, g.n_frame, 2 * c_out};
+    const int c_out = remap_channels(cfg->chan_remap, bg.n_chan, cfg->n_out_chan);
+    int64_t fs[4] = {g.batch, kBins, g.n_frame, spec_width(base_mode, cfg->chan_remap, c_out)};
     if (base_mode >= IRIS_FEAT_MEL) { fs[1] = c->n_mel; fs[3] = c_out; }
     iris_step_io io;
     memset(&io, 0, sizeof io);

@@ -172,9 +172,11 @@ __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, 
 // projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.
 // EPI_REMAP: the mel epilogue of a channel remap (stereo_mono / random_merge_aug: 2 input channels, c_out
 // output channels), switches read at run time like EPI == 0.
+// EPI_MONO, alone or on top of the 2-channel variants above: mono_chan (include/iris.h IRIS_REMAP_MONO_CHAN)
+// keeps two channels, so it is the 2-channel epilogue with (re0 + re1, re0 + im_j) formed before |.|.
 // OutT: element type of p.out (float, __nv_bfloat16, __half).  The half instances have no min-max
 // epilogue: the min-max log-mel features are normalised by k_logmel_post, which converts.
-constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4, EPI_REMAP = 8;
+constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4, EPI_REMAP = 8, EPI_MONO = 16;
 constexpr int kFixFR = 8;   // frames per tile of the fixed mel variants
 __host__ __device__ constexpr int fixed_mel_L(int r) { return r == 0 ? 2 : (r == 1 ? 4 : (r == 2 ? 6 : 0)); }
 template <int MODE, int NJ, int EPI, class OutT>
@@ -188,6 +190,8 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
     constexpr bool kRemap = (EPI == EPI_REMAP);
     static_assert(!kFix || kMel, "fixed epilogues exist for the mel modes only");
     static_assert(!kRemap || kMel, "the remap epilogue is a mel epilogue");
+    constexpr bool kMono = (EPI & EPI_MONO) != 0;
+    static_assert(!kMono || kMel, "the mono_chan epilogue is a mel epilogue");
     constexpr bool kF32 = sizeof(OutT) == 4;
     static_assert(kF32 || (MODE != FM_ACTIVITY && !(EPI & EPI_MINMAX)), "activity flags and the min-max epilogue are fp32 only");
     constexpr int S = slots_of(MODE);      // stage buffers
@@ -679,8 +683,13 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 if (do_fft) {   // warp-uniform
                     auto emit = [&](int f, int bit, cpx zf, cpx zm) {
                         // (re ch0, re ch1) and (im ch0, im ch1) of the split, as packed pairs
-                        const cpx re = cadd(zf, zm);
-                        const cpx im = cadd(cpx{zf.y, -zf.x}, cpx{-zm.y, zm.x});
+                        cpx re = cadd(zf, zm);
+                        cpx im = cadd(cpx{zf.y, -zf.x}, cpx{-zm.y, zm.x});
+                        if constexpr (kMono) {   // z_j = (re0 + re1) + i (re0 + im_j); a masked bin is 0 either way
+                            const float s = re.x + re.y;
+                            im = cpx{re.x + im.x, re.x + im.y};
+                            re = cpx{s, s};
+                        }
                         const cpx sq = cfma2(im, im, cmul2(re, re));
                         float m0 = sqrt_approx(sq.x);
                         float m1 = sqrt_approx(sq.y);
@@ -740,7 +749,8 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                                 a1 = __logf(a1 + 1e-8f);
                             }
                             if ((C & 1) == 0) {
-                                if constexpr (kF32) {
+                                // (mono_chan with NJ = 8: plain stores, the hint's registers spill)
+                                if constexpr (kF32 && !(kMono && NJ == 8)) {
                                     if (keep_l2) st_f2_hint(o, a0, a1, pol_keep);
                                     else store_out2(o, a0, a1);
                                 } else {
@@ -876,17 +886,20 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 named_bar_sync(1, FR * 32);   // the pieces are read before the next tile overwrites them
             } else if (do_fft) {
                 // channel remaps: stft_filter is applied by store_bin (it follows the remap)
+                const bool mono = p.remap == REMAP_MONO_CHAN;
+                auto store = [&](int f, float r0, float i0, float r1, float i1, float m) {
+                    if (mono) store_bin<MODE, OutT, true>(p, b, f, t, pair, has1, r0, i0, r1, i1, m);
+                    else store_bin<MODE, OutT, false>(p, b, f, t, pair, has1, r0, i0, r1, i1, m);
+                };
 #pragma unroll
                 for (int jj = 0; jj < 8; ++jj) {
                     const int f = k1 + 16 * (2 * jj + par);
                     const cpx zf = u[jj], zm = mirror(jj);
-                    store_bin<MODE, OutT>(p, b, f, t, pair, has1, zf.x + zm.x, zf.y - zm.y, zf.y + zm.y,
-                                    zm.x - zf.x, ((zbits >> jj) & 1u) ? 0.f : mt);
+                    store(f, zf.x + zm.x, zf.y - zm.y, zf.y + zm.y, zm.x - zf.x, ((zbits >> jj) & 1u) ? 0.f : mt);
                 }
                 if (l0) {
                     const cpx zf = u[8];
-                    store_bin<MODE, OutT>(p, b, 256, t, pair, has1, zf.x + zf.x, zf.y - zf.y, zf.y + zf.y,
-                                    zf.x - zf.x, ((zbits >> 8) & 1u) ? 0.f : mt);
+                    store(256, zf.x + zf.x, zf.y - zf.y, zf.y + zf.y, zf.x - zf.x, ((zbits >> 8) & 1u) ? 0.f : mt);
                 }
             }
         }
@@ -968,7 +981,9 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     if (n_tiles <= 0) return cudaSuccess;
     if (n_tiles > 0x7fffffffLL || p.max_segs > kMaxStages || p.n_pairs > 127) return cudaErrorInvalidValue;
     if (mode == FM_MEL && (long long)p.n_mel * p.T * p.c_out > 0x7fffffffLL) return cudaErrorInvalidValue;   // 32-bit row offsets inside a clip
-    if (mode == FM_MEL && p.remap != REMAP_NONE && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
+    if (mode == FM_MEL && p.remap != REMAP_NONE &&
+        (p.C != 2 || (p.remap == REMAP_MONO_CHAN ? p.c_out != 2 : p.c_out < 3)))
+        return cudaErrorInvalidValue;
     const size_t smem = fused_smem_bytes(p, mode);
     if (smem > 227 * 1024 - 256) return cudaErrorInvalidValue;   // (128 B of static shared memory: s_mm)
     if (out_type != OUT_F32 && ((out_type != OUT_BF16 && out_type != OUT_F16) || mode == FM_ACTIVITY || p.do_minmax))
@@ -1035,20 +1050,28 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         case FM_COMPLEX: IRIS_LAUNCH_OUT(FM_COMPLEX, 8, 0) break;
         case FM_MAGPHASE: IRIS_LAUNCH_OUT(FM_MAGPHASE, 8, 0) break;
         case FM_LOGMAGPHASE: IRIS_LAUNCH_OUT(FM_LOGMAGPHASE, 8, 0) break;
-        case FM_MEL:
+        case FM_MEL: {
+            const bool fixed = p.C == 2 && p.mel_L[0] == fixed_mel_L(0) && p.mel_L[1] == fixed_mel_L(1) &&
+                               p.mel_L[2] == fixed_mel_L(2) && p.mel_L[3] == fixed_mel_L(3) && FR == kFixFR &&
+                               p.mel_taps == 12 && !getenv("IRIS_NO_FIXED_EPI");
+            // the 2-channel choice; X = 0, or EPI_MONO for mono_chan
+#define IRIS_LAUNCH_MEL2(X)                                                                     \
+    {                                                                                           \
+        if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, X)                         \
+        else if (!fixed) IRIS_LAUNCH_OUT(FM_MEL, 4, X)                                          \
+        else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX | X, float)            \
+        else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | EPI_LOG | X)                     \
+        else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | X)                                             \
+    }
             // a remap keeps p.C == 2: it must be tested before the fixed 2-channel instances
-            if (p.remap != REMAP_NONE) {
+            if (p.remap == REMAP_MONO_CHAN) IRIS_LAUNCH_MEL2(EPI_MONO)
+            else if (p.remap != REMAP_NONE) {
                 if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_REMAP)
                 else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_REMAP)
-            } else if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
-            else if (p.C != 2 || p.mel_L[0] != fixed_mel_L(0) || p.mel_L[1] != fixed_mel_L(1) ||
-                     p.mel_L[2] != fixed_mel_L(2) || p.mel_L[3] != fixed_mel_L(3) ||
-                     FR != kFixFR || p.mel_taps != 12 || getenv("IRIS_NO_FIXED_EPI"))
-                IRIS_LAUNCH_OUT(FM_MEL, 4, 0)
-            else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX, float)
-            else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | EPI_LOG)
-            else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2)
+            } else IRIS_LAUNCH_MEL2(0)
+#undef IRIS_LAUNCH_MEL2
             break;
+        }
         case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0, float) break;
         case FM_SE:   // both virtual pairs of a (clip, time) range in one CTA: the combined store
             if (out_type != OUT_F32 || !p.pair_merge || p.seg_select != 3) return cudaErrorInvalidValue;

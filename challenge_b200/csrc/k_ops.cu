@@ -43,7 +43,8 @@ __global__ void __launch_bounds__(kOpThreads) k_axis_shift(const float* __restri
 }
 
 // rows of [2C]: first C = real / magnitude, last C = imag / phase
-//   OP 0: complex_to_magphase (transforms.py:111-123)
+//   OP 0: complex_to_magphase (transforms.py:111-123); an odd input width (3, C = 2) is mono_chan's
+//         [real, imag0, imag1], the real column broadcast, into rows of 2C = 4
 //   OP 1: magphase_to_complex (transforms.py:126-134)
 //   OP 2: log_magphase        (transforms.py:80-86): log(x + 1e-8) on the first n_log columns
 //   OP 3: log_on_mel          (data_utils.py:50-55):  log(x + 1e-8) everywhere
@@ -57,7 +58,7 @@ __global__ void __launch_bounds__(kOpThreads) k_pointwise(const float* __restric
         for (size_t i = blockIdx.x * size_t(kOpThreads) + threadIdx.x; i < n;
              i += size_t(gridDim.x) * kOpThreads) {
             const size_t r = i / C, c = i - r * C;
-            const float a = x[r * width + c], b = x[r * width + C + c];
+            const float a = x[r * width + ((width & 1) ? 0 : c)], b = x[r * width + (width - C) + c];
             float u, v;
             if (OP == 0) {
                 u = sqrtf(__fadd_rn(__fmul_rn(a, a), __fmul_rn(b, b)));   // sqrt(real**2 + img**2)
@@ -66,8 +67,8 @@ __global__ void __launch_bounds__(kOpThreads) k_pointwise(const float* __restric
                 u = a * cosf(b);
                 v = a * sinf(b);
             }
-            out[r * width + c] = u;
-            out[r * width + C + c] = v;
+            out[r * 2 * C + c] = u;
+            out[r * 2 * C + C + c] = v;
         }
     } else {
         const size_t n = rows * size_t(width);

@@ -53,8 +53,10 @@ constexpr int kSpecTile = 32;      // frames per CTA
 constexpr int kSpecWarps = 8;
 constexpr int kSpecMaxSegs = 48;   // staged segments per tile; more fall back to the global list
 
-template <int MODE, class OutT>
-__global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_constant__ FusedParams p,
+// kMono: the spectrogram modes of a mono_chan plan (store_bin<.., true>).  Their minimum of 2 CTAs per SM keeps
+// ptxas from its own choice of 64 registers with spills for the COMPLEX instance (0 = no minimum, as before).
+template <int MODE, class OutT, bool kMono = false>
+__global__ void __launch_bounds__(kSpecWarps * 32, kMono ? 2 : 0) k_specmix(const __grid_constant__ FusedParams p,
                                                             const float* __restrict__ melW,
                                                             const int32_t* __restrict__ mel_lo,
                                                             const int32_t* __restrict__ mel_len) {
@@ -200,6 +202,14 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                     const float mm = m[u] * filt;
                     const float a0 = r0[u] * mm, b0 = i0[u] * mm, a1 = r1[u] * mm, b1 = i1[u] * mm;
                     float* o = mags + (size_t(f - f_begin) * kSpecTile + lane) * Cm + 2 * pair;
+                    if (p.remap == REMAP_MONO_CHAN) {
+                        // z_j = (re0 + re1) + i (re0 + im_j) (include/iris.h): the sums of the masked,
+                        // filtered inputs (a bin the filter zeroes has |z_j| = 0 either way)
+                        const float s = __fadd_rn(a0, a1), y0 = __fadd_rn(a0, b0), y1 = __fadd_rn(a0, b1);
+                        o[0] = sqrt_approx(fmaf(s, s, y0 * y0));
+                        o[1] = sqrt_approx(fmaf(s, s, y1 * y1));
+                        continue;
+                    }
                     o[0] = sqrt_approx(fmaf(a0, a0, b0 * b0));   // transforms.py:116
                     if (has1) o[1] = sqrt_approx(fmaf(a1, a1, b1 * b1));
                     // channel remap (C == 2, one pair): the other output channels from the masked, filtered
@@ -225,7 +235,7 @@ __global__ void __launch_bounds__(kSpecWarps * 32) k_specmix(const __grid_consta
                         o[3 * cells + c] = nr[u];
                     }
                 } else if (live) {
-                    store_bin<MODE, OutT>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
+                    store_bin<MODE, OutT, kMono>(p, b, f, t, pair, has1, r0[u], i0[u], r1[u], i1[u], m[u]);
                 }
             }
         }
@@ -276,12 +286,23 @@ static cudaError_t launch_specmix_t(const FusedParams& p, int mode, const float*
                                     const int32_t* mel_len, cudaStream_t st) {
     dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
     const int threads = kSpecWarps * 32;
+    const bool mono = p.remap == REMAP_MONO_CHAN;   // the spectrogram modes of mono_chan: instances of their own
+    if (mono && (p.C != 2 || p.c_out != 2)) return cudaErrorInvalidValue;
     switch (mode) {
-        case FM_COMPLEX: k_specmix<FM_COMPLEX, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
-        case FM_MAGPHASE: k_specmix<FM_MAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
-        case FM_LOGMAGPHASE: k_specmix<FM_LOGMAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr); break;
+        case FM_COMPLEX:
+            if (mono) k_specmix<FM_COMPLEX, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            else k_specmix<FM_COMPLEX, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            break;
+        case FM_MAGPHASE:
+            if (mono) k_specmix<FM_MAGPHASE, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            else k_specmix<FM_MAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            break;
+        case FM_LOGMAGPHASE:
+            if (mono) k_specmix<FM_LOGMAGPHASE, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            else k_specmix<FM_LOGMAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
+            break;
         case FM_MEL: {
-            if (p.remap != REMAP_NONE && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
+            if (p.remap != REMAP_NONE && !mono && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
             const size_t smem = specmix_mel_smem(p.c_out, p.mel_f_n);
             if (smem > 200 * 1024) return cudaErrorInvalidValue;
             static bool attr_set = false;   // per instance

@@ -222,5 +222,6 @@ augment._iris_stage = ('augment',)
 to_frame_labels._iris_stage = ('to_frame_labels',)
 speech_enhancement_preprocess._iris_stage = ('se',)
 stereo_mono._iris_stage = ('stereo_mono',)
+mono_chan._iris_stage = ('mono_chan',)
 minmax._iris_stage = ('minmax',)
 log_on_mel._iris_stage = ('log_on_mel',)

@@ -207,14 +207,16 @@ class Engine:
         p.chan_remap = int(chan_remap)
         p.n_out_chan = int(n_out_chan)
         L.check(self.lib.iris_plan_upload(self._ctx, C.byref(p), self._stream()))
-        c_out = self.bank_chan
-        if chan_remap == L.REMAP_STEREO_MONO:
-            c_out = 3
-        elif chan_remap == L.REMAP_MERGE_AUG:
-            c_out = int(n_out_chan)
-        self._plan = dict(B=int(d.batch), T=int(d.n_frame), V=int(d.max_voices), c_out=c_out,
+        self._plan = dict(B=int(d.batch), T=int(d.n_frame), V=int(d.max_voices), remap=int(chan_remap),
+                          c_out=self._remap_channels(chan_remap, n_out_chan),
                           bytes=sum(v.nbytes for v in keep.values() if v is not None))
         return self._plan
+
+    def _remap_channels(self, chan_remap, n_out_chan):
+        """C' of include/iris.h: the channels after a channel remap of the banks' channels."""
+        if chan_remap == L.REMAP_NONE:
+            return self.bank_chan
+        return {L.REMAP_STEREO_MONO: 3, L.REMAP_MONO_CHAN: 2}.get(chan_remap, int(n_out_chan))
 
     def labels(self, want_vtk=False, want_keep=True):
         """-> (frame_labels [B,T,K], labels [B,V,T,K] or None, keep [B,V] uint8 or None)."""
@@ -239,6 +241,8 @@ class Engine:
             return tuple((pl['B'], 256, pl['T'], c) for c in (C, C // 2, C // 2))
         if int(mode) & L.MODE_MASK >= L.FEAT_MEL:
             return (pl['B'], self.n_mel, pl['T'], pl['c_out'])   # channels after the remap
+        if int(mode) & L.MODE_MASK == L.FEAT_COMPLEX and pl['remap'] == L.REMAP_MONO_CHAN:
+            return (pl['B'], 257, pl['T'], 3)                    # mono_chan's own columns
         return (pl['B'], 257, pl['T'], 2 * pl['c_out'])
 
     def _feature_buffer(self, mode, out, dtype):
@@ -299,12 +303,8 @@ class Engine:
         torch = _torch()
         g = scfg.draw
         B, T, V = g.batch, g.n_frame, g.max_voices
-        c_out = self.bank_chan
-        if scfg.chan_remap == L.REMAP_STEREO_MONO:
-            c_out = 3
-        elif scfg.chan_remap == L.REMAP_MERGE_AUG:
-            c_out = int(scfg.n_out_chan)
-        self._plan = dict(B=B, T=T, V=V, c_out=c_out, bytes=0)
+        self._plan = dict(B=B, T=T, V=V, remap=int(scfg.chan_remap),
+                          c_out=self._remap_channels(scfg.chan_remap, scfg.n_out_chan), bytes=0)
         mode = scfg.feature_mode
         out, res = self._feature_buffer(mode, out, out_dtype(mode))
         if frame is None and want_frame and V > 0:
@@ -393,12 +393,8 @@ class Engine:
             scfg = L.IrisStepConfig(scfg.draw, scfg.stft_filter, scfg.chan_remap, scfg.n_out_chan,
                                     scfg.feature_mode | L.dlpack_out_flag(fptr))
         g = scfg.draw
-        c_out = self.bank_chan
-        if scfg.chan_remap == L.REMAP_STEREO_MONO:
-            c_out = 3
-        elif scfg.chan_remap == L.REMAP_MERGE_AUG:
-            c_out = int(scfg.n_out_chan)
-        self._plan = dict(B=g.batch, T=g.n_frame, V=g.max_voices, c_out=c_out, bytes=0)
+        self._plan = dict(B=g.batch, T=g.n_frame, V=g.max_voices, remap=int(scfg.chan_remap),
+                          c_out=self._remap_channels(scfg.chan_remap, scfg.n_out_chan), bytes=0)
         L.check(self.lib.iris_step_dlpack(
             self._ctx, C.byref(scfg), u.ctypes.data, streams, fptr,
             L.dlpack_pointer(frame_capsule) if frame_capsule is not None else None, self._stream()))

@@ -15,9 +15,10 @@ The host only draws the randomness of a whole batch in the reference's draw orde
 ``make_pipeline`` returns an :class:`IrisDataset` with the slice of the ``tf.data`` surface
 that ``sj_train.make_dataset`` (sj_train.py:92-130) uses -- ``map``, ``batch``, ``prefetch``,
 ``take``, ``repeat``, iteration.  Chaining the drop-in functions in sj_train's order
-(``to_frame_labels``, ``augment``, ``stereo_mono`` | ``random_merge_aug(n)``,
+(``to_frame_labels``, ``augment``, ``stereo_mono`` | ``random_merge_aug(n)`` | ``mono_chan``,
 ``stft_filter(k)``, ``batch``, ``complex_to_magphase``, ``magphase_to_mel(n)``, ``minmax``,
-``log_on_mel``) is recognised and lowered to ONE fused launch per batch; so is the 'se' chain
+``log_on_mel``) is recognised and lowered to ONE fused launch per batch (``mono_chan`` of 2-channel
+banks only); so is the 'se' chain
 (``seperate_noise_voice=True``, [``augment``, ``stft_filter(k)``,] ``speech_enhancement_preprocess``,
 ``batch``, sj_train.py:99-106) of 2-channel banks.  Any other callable runs after it on the un-fused
 tensors (the stand-alone kernels), so arbitrary chains work.
@@ -96,7 +97,7 @@ class IrisDataset:
         rest = []
         state = 'pre'       # pre-batch element stages -> post-batch feature stages
         order = {'to_frame_labels': 0, 'density_labels': 0, 'augment': 1, 'stereo_mono': 2, 'merge_aug': 2,
-                 'stft_filter': 3}
+                 'mono_chan': 2, 'stft_filter': 3}
         last = -1
         stages = list(self._stages)
         i = 0
@@ -105,7 +106,8 @@ class IrisDataset:
             tag = getattr(st, '_iris_stage', None) if callable(st) else st
             if rest:
                 rest.append(st)
-            elif state == 'pre' and tag and tag[0] in order and order[tag[0]] > last:
+            elif state == 'pre' and tag and tag[0] in order and order[tag[0]] > last \
+                    and (tag[0] != 'mono_chan' or self._src.get('n_chan') == 2):
                 last = order[tag[0]]
                 if tag[0] == 'to_frame_labels':
                     fused['frame_labels'] = True
@@ -117,6 +119,8 @@ class IrisDataset:
                     fused['remap'], fused['n_out'] = L.REMAP_STEREO_MONO, 3
                 elif tag[0] == 'merge_aug':
                     fused['remap'], fused['n_out'] = L.REMAP_MERGE_AUG, int(tag[1])
+                elif tag[0] == 'mono_chan':                 # 2-channel banks only (IRIS_REMAP_MONO_CHAN)
+                    fused['remap'], fused['n_out'] = L.REMAP_MONO_CHAN, 2
                 elif tag[0] == 'stft_filter':
                     fused['filt'] = int(tag[1])
             elif state == 'pre' and tag and tag[0] == 'se' and self._se_fusable(fused, last, i):

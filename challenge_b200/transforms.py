@@ -123,8 +123,9 @@ def minmax_norm_magphase(specs, labels=None):
 def complex_to_magphase(complex_tensor, y=None):
     """transforms.py:111-123."""
     x = O.dev(complex_tensor)
-    out = O.empty(x.shape)
     width = int(x.shape[-1])
+    # mono_chan's [re, im0, im1]: TF broadcasts re against both imaginary columns -> [mag0, mag1, ph0, ph1]
+    out = O.empty(tuple(x.shape[:-1]) + (4 if width == 3 else width,))
     O.call('iris_op_pointwise', L.PW_C2MP, O.ptr(x), O.ptr(out), x.numel() // width, width, 0, 0.0)
     if y is None:
         return out

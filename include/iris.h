@@ -40,9 +40,10 @@ enum {
 enum { IRIS_BANK_BG = 0, IRIS_BANK_VOICE = 1, IRIS_BANK_NOISE = 2 };
 
 /* feature modes of iris_features(); layouts as in the reference.  C' is the channel count after the
- * plan's channel remap (3 for stereo_mono, n_out_chan for random_merge_aug, else the bank's), in the
- * spectrogram and the mel layouts alike: a remap is fused in front of the mel projection.  (A library
- * older than that answers the mel modes of a remapped plan with IRIS_ERR_UNSUPPORTED.) */
+ * plan's channel remap (3 for stereo_mono, n_out_chan for random_merge_aug, 2 for mono_chan, else the
+ * bank's), in the spectrogram and the mel layouts alike: a remap is fused in front of the mel projection.
+ * (A library older than that answers the mel modes of a remapped plan with IRIS_ERR_UNSUPPORTED.)  One
+ * exception: IRIS_FEAT_COMPLEX of a mono_chan plan is [B,257,T,3], see IRIS_REMAP_MONO_CHAN. */
 enum {
     IRIS_FEAT_COMPLEX = 0,       /* [B,257,T,2C']  make_pipeline output (pipeline.py:131-133)  */
     IRIS_FEAT_MAGPHASE = 1,      /* [B,257,T,2C']  complex_to_magphase (transforms.py:111-123)  */
@@ -75,7 +76,14 @@ enum {
  * that predates the flags, so callers can detect support). */
 enum { IRIS_OUT_BF16 = 0x100, IRIS_OUT_F16 = 0x200 };
 
-enum { IRIS_REMAP_NONE = 0, IRIS_REMAP_STEREO_MONO = 1, IRIS_REMAP_MERGE_AUG = 2 };
+enum { IRIS_REMAP_NONE = 0, IRIS_REMAP_STEREO_MONO = 1, IRIS_REMAP_MERGE_AUG = 2, IRIS_REMAP_MONO_CHAN = 3 };
+/* IRIS_REMAP_MONO_CHAN: data_utils.mono_chan (data_utils.py:73-76) of a 2-channel plan, n_out_chan = 2.  Its
+ * broadcast quirk x[..., :1] + x[..., 1:] makes the complex spectrogram the 3 columns [re0 + re1, re0 + im0,
+ * re0 + im1] (IRIS_FEAT_COMPLEX: [B,257,T,3]); complex_to_magphase then broadcasts the one real column
+ * against the two imaginary ones (transforms.py:111-123), so every later mode sees C' = 2 pseudo-channels
+ * z_j = (re0 + re1) + i (re0 + im_j): magnitude + phase [B,257,T,4], mel [B,n_mel,T,2].  Masks act on the
+ * inputs, stft_filter on the sums.  A library without it answers the plan with IRIS_ERR_INVALID (n_out_chan
+ * below 3), so callers can probe for it. */
 
 int iris_abi_version(void);
 const char* iris_last_error(void);
@@ -139,7 +147,7 @@ typedef struct iris_plan {
     const int32_t* freq_masks;   /* [B,n_freq_masks,2] (size, offset) or NULL              */
     int32_t stft_filter;         /* zero bins 1..k (data_utils.py:126-136); 0 = off        */
     int32_t chan_remap;          /* IRIS_REMAP_*  (data_utils.py:79-82, 100-117)           */
-    int32_t n_out_chan;          /* channels after remap (3 for stereo_mono)               */
+    int32_t n_out_chan;          /* channels after remap (3 for stereo_mono, 2 for mono_chan) */
     const float* merge_factor;   /* [B, n_out_chan-2] U(0.1, 0.9), REMAP_MERGE_AUG only    */
 } iris_plan;
 
@@ -241,7 +249,9 @@ int iris_op_random_shift(iris_ctx* ctx, const float* d_x, float* d_out, int64_t 
                          int64_t n_axis, int64_t inner, int width, int offset, iris_stream stream);
 /* Row-wise stages on [rows, 2*n_chan] (first half real / magnitude, second imag / phase). */
 enum {
-    IRIS_PW_COMPLEX_TO_MAGPHASE = 0, /* transforms.py:111-123 */
+    IRIS_PW_COMPLEX_TO_MAGPHASE = 0, /* transforms.py:111-123; width 3 (mono_chan's [re, im0, im1]) is
+                                        TF's broadcast of re against both: rows of 4 (out must NOT
+                                        alias x), other odd widths are IRIS_ERR_INVALID */
     IRIS_PW_MAGPHASE_TO_COMPLEX = 1, /* transforms.py:126-134 */
     IRIS_PW_LOG_MAGPHASE = 2,        /* transforms.py:80-86; `param_i` = n_chan argument      */
     IRIS_PW_LOG_ON_MEL = 3,          /* data_utils.py:50-55; any shape, pass width = 1        */
