@@ -11,6 +11,7 @@ from oracle import data_utils as D
 from oracle import metrics as M
 from oracle import pipeline as P
 from oracle import transforms as T
+from oracle.f64 import synth_index_level as _synth_index_level
 
 KATS = json.load(open(os.path.join(os.path.dirname(__file__), 'golden', 'reference_kats.json')))
 
@@ -234,60 +235,6 @@ def test_oracle_resampler_is_pinned_to_torchaudio(orig, n):
     ref = ta.functional.resample(torch.from_numpy(wav), orig, 16000).numpy()
     assert got.shape == ref.shape
     assert np.abs(got - ref).max() <= 1e-4 * np.abs(ref).max()
-
-
-def _synth_index_level(bg, voices, vlabels, noises, d, b, K=3):
-    """Independent restatement of sample synthesis from the INDEX-LEVEL semantics (SURVEY.md appendix
-    A.2), frame by frame in float64, sharing no code with oracle/pipeline.py (which pads, slices and
-    adds whole tensors like the reference does): out[f,t] = BG[f,(t+o_b) mod bgT] + sum over kept
-    voices of g_v X_v[f, t+off_v-s_v] + sum over noises; labels and keep flags by the same indices."""
-    T = d.n_frame
-    V, M = d.max_voices, d.max_noises
-    BG = bg[int(d.bg_id[b])].astype(np.float64)
-    bgT = BG.shape[1]
-    out = np.empty((BG.shape[0], T, BG.shape[2]), np.float64)
-    for t in range(T):
-        out[:, t] = BG[:, (t + int(d.bg_offset[b])) % bgT]
-    label = np.zeros((V, T, K), np.float64)
-    keep = [0] * V
-    if V:
-        ids = [int(i) for i in d.voice_id[b]]
-        vP = max(voices[i].shape[1] for i in ids)                      # padded_batch: the group's longest
-        pad = T - int(np.int32(np.float32(d.min_ratio) * np.float32(vP)))
-        s = pad if pad > 0 else 0
-        nv = int(d.n_voices[b]) if V > 1 else 1
-        L = np.zeros((T, K), np.float64)
-        for v in range(nv):
-            X = voices[ids[v]].astype(np.float64)
-            kT = X.shape[1]
-            act = (voices[ids[v]].max(axis=(0, 2)) > 0)
-            cand = np.zeros((T, K), np.float64)
-            src = [t + int(d.voice_offset[b][v]) - s for t in range(T)]
-            for t, k in enumerate(src):
-                if 0 <= k < kT and act[k]:
-                    cand[t] = np.asarray(vlabels[ids[v]], np.float64)
-            ok = not ((L + cand) >= 2).any()
-            keep[v] = int(ok)
-            if ok:
-                g = float(d.voice_gain[b][v])
-                for t, k in enumerate(src):
-                    if 0 <= k < kT:
-                        out[:, t] += g * X[:, k]
-                L += cand
-                label[v] = cand
-    if M:
-        ids = [int(i) for i in d.noise_id[b]]
-        nP = max(noises[i].shape[1] for i in ids)
-        pad = T - int(np.int32(np.float32(d.min_noise_ratio) * np.float32(nP)))
-        s = pad if pad > 0 else 0
-        for n in range(int(d.n_noises[b])):
-            X = noises[ids[n]].astype(np.float64)
-            g = float(d.noise_gain[b][n])
-            for t in range(T):
-                k = t + int(d.noise_offset[b][n]) - s
-                if 0 <= k < X.shape[1]:
-                    out[:, t] += g * X[:, k]
-    return out, label, keep
 
 
 def test_merge_complex_specs_against_an_index_level_restatement():
