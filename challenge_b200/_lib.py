@@ -80,6 +80,8 @@ SIGNATURES = {
     'iris_set_mel': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     'iris_bank_register': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    'iris_bank_register_audio': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     'iris_specbank_register': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     'iris_bank_info': (C.c_int, [C.c_void_p, C.c_int, _i32p, _i32p, C.c_void_p]),
@@ -172,6 +174,8 @@ SIGNATURES = {
     'iris_plan_upload_bytes': (C.c_int64, [C.c_void_p]),
     'iris_max_segments': (C.c_int, []),
 }
+# symbols added under IRIS_ABI_VERSION 2 that an older library lacks (callers probe with hasattr)
+OPTIONAL = {'iris_bank_register_audio'}
 PW_C2MP, PW_MP2C, PW_LOG_MAGPHASE, PW_LOG_ON_MEL, PW_MULTIPLY = range(5)
 MAP_MONO_CHAN, MAP_STEREO_MONO, MAP_MERGE_AUG = range(3)
 
@@ -189,6 +193,8 @@ def load():
             '`python -m challenge_b200.build` (needs nvcc).  There is no CPU fallback.')
     lib = C.CDLL(LIB_PATH)
     for name, (res, args) in SIGNATURES.items():
+        if name in OPTIONAL and not hasattr(lib, name):
+            continue
         fn = getattr(lib, name)
         fn.restype = res
         fn.argtypes = args

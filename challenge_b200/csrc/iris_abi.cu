@@ -589,17 +589,16 @@ int iris_set_mel(iris_ctx* c, int n_mel, int n_bins, const float* w) {
     return IRIS_OK;
 }
 
-int iris_bank_register(iris_ctx* c, int kind, int n_items, int n_chan, const float* wav,
-                       const int64_t* offsets, const float* labels, int n_classes, int normalize,
-                       iris_stream stream) {
-    if (!c || !wav || !offsets) return fail(IRIS_ERR_INVALID, "NULL argument");
-    if (kind < 0 || kind > 2) return fail(IRIS_ERR_INVALID, "bad bank kind");
-    if (n_items < 1 || n_chan < 1) return fail(IRIS_ERR_INVALID, "empty bank");
-    if (kind == IRIS_BANK_VOICE && (!labels || n_classes < 1))
-        return fail(IRIS_ERR_INVALID, "voice bank needs labels [n_items, n_classes]");
-    int rc = set_device(c);
-    if (rc) return rc;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+}  // extern "C"
+
+namespace {
+
+// Registration of a waveform bank from 16 kHz audio, shared by iris_bank_register and
+// iris_bank_register_audio.  bank_layout: checks the items of `offsets` (host, cumulative per-channel
+// 16 kHz samples) and lays out their frames; bank_fill: from the packed items in `wav16` (device, item i
+// at n_chan * (offsets[i] - offsets[0])), normalize + reflect-padded pair layout (k_bank_prepare) and,
+// for the voice bank, the activity pass.  Synchronises the stream and releases wav16.
+int bank_layout(iris_ctx* c, int kind, int n_items, int n_chan, const int64_t* offsets, int n_classes) {
     Bank& b = c->banks[kind];
     b.ready = false;
     b.spec = false;
@@ -621,24 +620,27 @@ int iris_bank_register(iris_ctx* c, int kind, int n_items, int n_chan, const flo
         b.pad_offsets[i + 1] = b.pad_offsets[i] + 256 * (kT + 1);
     }
     if (n_chan > 32) return fail(IRIS_ERR_UNSUPPORTED, "more than 32 channels");
+    return IRIS_OK;
+}
+
+int bank_fill(iris_ctx* c, int kind, DevBuf& wav16, const float* labels, int normalize, cudaStream_t st) {
+    Bank& b = c->banks[kind];
+    const int n_items = b.n_items, n_chan = b.n_chan, n_classes = b.n_classes;
     const int n_pairs = (n_chan + 1) / 2;
-    const size_t wav_floats = size_t(offsets[n_items]) * n_chan;
     const size_t pad_floats = size_t(b.pad_offsets[n_items]) * n_pairs * 2;
-    DevBuf raw, d_off;
-    CU(raw.reserve(wav_floats * 4));
+    DevBuf d_off;
     CU(d_off.reserve(size_t(n_items + 1) * 16));
     CU(b.padded.reserve(pad_floats * 4));
     CU(b.d_n_frames.reserve(size_t(n_items) * 4));
-    CU(cudaMemcpyAsync(raw.p, wav + size_t(offsets[0]) * n_chan, wav_floats * 4, cudaMemcpyDefault, st));
     std::vector<int64_t> rel(n_items + 1);
-    for (int i = 0; i <= n_items; ++i) rel[i] = offsets[i] - offsets[0];
+    for (int i = 0; i <= n_items; ++i) rel[i] = b.offsets[i] - b.offsets[0];
     int64_t* d_o = d_off.as<int64_t>();
     CU(cudaMemcpyAsync(d_o, rel.data(), size_t(n_items + 1) * 8, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(d_o + n_items + 1, b.pad_offsets.data(), size_t(n_items + 1) * 8,
                        cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(b.d_n_frames.p, b.n_frames.data(), size_t(n_items) * 4,
                        cudaMemcpyHostToDevice, st));
-    CU(launch_bank_prepare(raw.as<float>(), d_o, d_o + n_items + 1, n_items, n_chan, normalize,
+    CU(launch_bank_prepare(wav16.as<float>(), d_o, d_o + n_items + 1, n_items, n_chan, normalize,
                            b.padded.as<float>(), st));
     if (kind == IRIS_BANK_VOICE) {
         CU(b.labels.reserve(size_t(n_items) * n_classes * 4));
@@ -677,7 +679,7 @@ int iris_bank_register(iris_ctx* c, int kind, int n_items, int n_chan, const flo
         p.T = b.max_frames;
         set_geometry(c, p, n_chan, false);
         p.activity = b.activity.as<uint8_t>();
-        rc = run_fused(c, p, FM_ACTIVITY, 1, st);
+        const int rc = run_fused(c, p, FM_ACTIVITY, 1, st);
         c->tile_sig.valid = false;   // the segment list of this pass is freed below
         if (rc) return rc;
         b.h_activity.resize(act_bytes);
@@ -686,12 +688,78 @@ int iris_bank_register(iris_ctx* c, int kind, int n_items, int n_chan, const flo
         d_segs.release();
     }
     CU(cudaStreamSynchronize(st));
-    raw.release();
+    wav16.release();
     d_off.release();
     b.ready = true;
     c->has_plan = false;
     return IRIS_OK;
 }
+
+}  // namespace
+
+extern "C" {
+
+int iris_bank_register(iris_ctx* c, int kind, int n_items, int n_chan, const float* wav,
+                       const int64_t* offsets, const float* labels, int n_classes, int normalize,
+                       iris_stream stream) {
+    if (!c || !wav || !offsets) return fail(IRIS_ERR_INVALID, "NULL argument");
+    if (kind < 0 || kind > 2) return fail(IRIS_ERR_INVALID, "bad bank kind");
+    if (n_items < 1 || n_chan < 1) return fail(IRIS_ERR_INVALID, "empty bank");
+    if (kind == IRIS_BANK_VOICE && (!labels || n_classes < 1))
+        return fail(IRIS_ERR_INVALID, "voice bank needs labels [n_items, n_classes]");
+    int rc = set_device(c);
+    if (rc) return rc;
+    rc = bank_layout(c, kind, n_items, n_chan, offsets, n_classes);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t wav_floats = size_t(offsets[n_items] - offsets[0]) * n_chan;
+    DevBuf raw;
+    CU(raw.reserve(wav_floats * 4));
+    CU(cudaMemcpyAsync(raw.p, wav + size_t(offsets[0]) * n_chan, wav_floats * 4, cudaMemcpyDefault, st));
+    return bank_fill(c, kind, raw, labels, normalize, st);
+}
+
+int iris_bank_register_audio(iris_ctx* c, int kind, int n_items, int n_chan, const float* wav,
+                             const int64_t* offsets, const int32_t* sample_rates, const float* labels,
+                             int n_classes, int normalize, iris_stream stream) {
+    if (!c || !wav || !offsets || !sample_rates) return fail(IRIS_ERR_INVALID, "NULL argument");
+    if (kind < 0 || kind > 2) return fail(IRIS_ERR_INVALID, "bad bank kind");
+    if (n_items < 1 || n_chan < 1) return fail(IRIS_ERR_INVALID, "empty bank");
+    if (kind == IRIS_BANK_VOICE && (!labels || n_classes < 1))
+        return fail(IRIS_ERR_INVALID, "voice bank needs labels [n_items, n_classes]");
+    for (int i = 0; i < n_items; ++i)
+        if (sample_rates[i] < 1 || offsets[i + 1] < offsets[i])
+            return fail(IRIS_ERR_INVALID, "iris_bank_register_audio: bad argument");
+    int rc = set_device(c);
+    if (rc) return rc;
+    std::vector<int64_t> n_in(n_items);
+    for (int i = 0; i < n_items; ++i) n_in[i] = offsets[i + 1] - offsets[i];
+    ResamplePlan plan;
+    rc = resample_plan("iris_bank_register_audio", n_items, n_chan, n_in.data(), sample_rates, 16000, &plan);
+    if (rc) return rc;
+    std::vector<int64_t> off16(n_items + 1, 0);   // the items' 16 kHz lengths, cumulative
+    for (int i = 0; i < n_items; ++i) off16[i + 1] = off16[i] + plan.n_out[i];
+    rc = bank_layout(c, kind, n_items, n_chan, off16.data(), n_classes);
+    if (rc) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t raw_floats = size_t(offsets[n_items] - offsets[0]) * n_chan;
+    DevBuf raw, pcm16, blob;
+    CU(raw.reserve(raw_floats * 4));
+    CU(cudaMemcpyAsync(raw.p, wav + size_t(offsets[0]) * n_chan, raw_floats * 4, cudaMemcpyDefault, st));
+    if (plan.copy_only)   // every item is 16 kHz: registered as iris_bank_register registers it
+        return bank_fill(c, kind, raw, labels, normalize, st);
+    // one copy of every item descriptor and filter table, one resample launch for the whole bank
+    CU(blob.reserve(plan.blob.size()));
+    CU(cudaMemcpyAsync(blob.p, plan.blob.data(), plan.blob.size(), cudaMemcpyHostToDevice, st));
+    CU(pcm16.reserve(size_t(off16[n_items]) * n_chan * 4));
+    CU(launch_resample(raw.as<float>(), pcm16.as<float>(), n_chan, blob.as<char>(), n_items, plan.n_ctas,
+                       plan.chunk, plan.smem_floats, st));
+    rc = bank_fill(c, kind, pcm16, labels, normalize, st);   // synchronises the stream
+    raw.release();
+    blob.release();
+    return rc;
+}
+
 
 int iris_specbank_register(iris_ctx* c, int kind, int n_items, int n_freq, int n_chan2, const float* specs,
                            const int64_t* frame_offsets, const float* labels, int n_classes,

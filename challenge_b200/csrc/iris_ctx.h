@@ -81,6 +81,21 @@ inline int spec_width(int mode, int remap, int c_out) {
     return mode == IRIS_FEAT_COMPLEX && remap == IRIS_REMAP_MONO_CHAN ? 3 : 2 * c_out;
 }
 
+// One k_resample launch (iris_ops_abi.cu: resample_plan): item i is [n_chan, n_in[i]] at orig[i] Hz, packed
+// back to back in the input, its [n_chan, n_out[i]] result back to back in the output.  `blob` is what goes
+// to the device in one copy: the ResampleItem array, then the Kaldi filter table of every distinct rate pair
+// (built once per pair).
+struct ResamplePlan {
+    std::vector<char> blob;
+    std::vector<int64_t> n_out;
+    long long n_ctas = 0;
+    int chunk = 0, smem_floats = 0;
+    bool copy_only = true;   // every item is at the target rate
+};
+// Rates must be >= 1.  A rate pair whose table exceeds 32 MB is IRIS_ERR_UNSUPPORTED ("<who>: ...").
+int resample_plan(const char* who, int n_items, int n_chan, const int64_t* n_in, const int32_t* orig,
+                  int new_freq, ResamplePlan* plan);
+
 // mode argument of the feature entry points: IRIS_FEAT_* in the low 8 bits, at most one IRIS_OUT_*
 // flag above them.  false: any other high bit (the base mode is range-checked by the caller).
 inline bool split_feature_mode(int mode, int* base, int* out_type) {

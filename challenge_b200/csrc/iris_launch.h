@@ -89,10 +89,18 @@ cudaError_t launch_phase_vocoder(const float* x, float* out, int F, int T, int C
 cudaError_t launch_sum_pool2(const float* y, float* out, int B, int T, int K, float scale, cudaStream_t st);
 cudaError_t launch_density_labels(const float* y, float* out, size_t outer, int V, int TK, cudaStream_t st);
 
-// k_resample.cu -- kaldi.resample_waveform (data_utils.py:20-21)
-cudaError_t launch_resample(const float* wav, float* out, int n_chan, long long n_in, long long n_out,
-                            int u_in, int u_out, int W, const int32_t* first, const float* weights,
-                            cudaStream_t st);
+// k_resample.cu -- kaldi.resample_waveform (data_utils.py:20-21) of a list of items.  The device blob
+// of a launch starts with its ResampleItem array; the filter tables follow.
+struct ResampleItem {
+    long long in_off, out_off;   // float offsets of the item's [n_chan, n_in] / [n_chan, n_out] blocks
+    long long n_in, n_out;       // samples per channel
+    long long table;             // byte offset in the blob of first[u_out] (int32), weights[u_out * W]; -1: copy
+    long long cta0;              // first CTA of the item (it has ceil(n_out / chunk))
+    int u_in, u_out, W, pad;
+};
+// smem_floats: the largest table of the launch that is staged in shared memory (0: none)
+cudaError_t launch_resample(const float* wav, float* out, int n_chan, const char* d_blob, int n_items,
+                            long long n_ctas, int chunk, int smem_floats, cudaStream_t st);
 
 // k_spec.cu -- spectrogram-format banks (the reference's pickled [257, t, 2C] lists)
 cudaError_t launch_spec_activity(const float* specs, const int64_t* frame_off, int n_items, int F, int W,

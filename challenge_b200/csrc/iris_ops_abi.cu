@@ -352,9 +352,121 @@ int iris_op_phase_vocoder(iris_ctx* c, const float* x, float* out, int n_freq, i
     return IRIS_OK;
 }
 
+}  // extern "C"
+
 // torchaudio.compliance.kaldi.resample_waveform (data_utils.py:20-21): Kaldi's LinearResample.
 // The per-phase window starts and windowed-sinc weights are computed here in float32 in the
 // port's op order (kaldi.py::_get_LR_indices_and_weights), the FIR runs in k_resample.cu.
+namespace iris {
+namespace {
+
+// The filter bank of orig -> new_freq: first[u_out] window starts, then weights[u_out * W], appended to
+// `blob`.  false: it would exceed 32 MB (nothing appended).
+bool append_kaldi_table(int orig_freq, int new_freq, std::vector<char>& blob, int* u_in, int* u_out, int* W) {
+    int g = orig_freq;
+    for (int b = new_freq; b;) { const int t = g % b; g = b; b = t; }
+    *u_in = orig_freq / g;
+    *u_out = new_freq / g;
+    const int uo = *u_out;
+    const int min_freq = orig_freq < new_freq ? orig_freq : new_freq;
+    const double cutoff = 0.99 * 0.5 * min_freq;              // lowpass_cutoff
+    const double width = 6.0 / (2.0 * cutoff);                // window_width, lowpass_filter_width = 6
+    const float ww = float(width), fo = float(orig_freq), fn = float(new_freq);
+    std::vector<int32_t> first(uo);
+    std::vector<float> mn(uo);
+    int w_max = 0;
+    for (int i = 0; i < uo; ++i) {
+        const float t = float(i) / fn;
+        mn[i] = ceilf((t - ww) * fo);
+        const float mx = floorf((t + ww) * fo);
+        first[i] = int32_t(mn[i]);
+        w_max = std::max(w_max, int(mx - mn[i] + 1.f));
+    }
+    *W = w_max;
+    if (size_t(uo) * w_max > (8u << 20)) return false;
+    std::vector<float> wt(size_t(uo) * w_max);
+    const float cw = float(2 * M_PI * cutoff / 6.0), cs = float(2 * M_PI * cutoff), pi = float(M_PI);
+    for (int i = 0; i < uo; ++i) {
+        const float t = float(i) / fn;
+        for (int j = 0; j < w_max; ++j) {
+            const float dt = (mn[i] + float(j)) / fo - t;
+            float w = 0.f;
+            if (fabsf(dt) < ww) w = 0.5f * (1.f + cosf(cw * dt));     // raised-cosine window
+            if (dt != 0.f) w *= sinf(cs * dt) / (pi * dt);              // sinc
+            else w *= float(2 * cutoff);
+            wt[size_t(i) * w_max + j] = w / fo;
+        }
+    }
+    const size_t at = align_up(blob.size(), 16);
+    blob.resize(at + size_t(uo) * 4 + wt.size() * 4);
+    memcpy(blob.data() + at, first.data(), size_t(uo) * 4);
+    memcpy(blob.data() + at + size_t(uo) * 4, wt.data(), wt.size() * 4);
+    return true;
+}
+
+}  // namespace
+
+int resample_plan(const char* who, int n_items, int n_chan, const int64_t* n_in, const int32_t* orig,
+                  int new_freq, ResamplePlan* plan) {
+    std::vector<ResampleItem> items(n_items);
+    std::vector<int32_t> rates;           // distinct rate pairs orig -> new_freq, in order of appearance
+    std::vector<ResampleItem> tabs;       // their table, u_in, u_out, W
+    std::vector<char>& blob = plan->blob;
+    blob.assign(size_t(n_items) * sizeof(ResampleItem), 0);
+    plan->n_out.assign(n_items, 0);
+    plan->copy_only = true;
+    plan->smem_floats = 0;
+    long long in_off = 0, out_off = 0, total = 0;
+    for (int i = 0; i < n_items; ++i) {
+        ResampleItem& it = items[i];
+        it.in_off = in_off;
+        it.out_off = out_off;
+        it.n_in = n_in[i];
+        it.n_out = orig[i] == new_freq ? n_in[i] : iris_resample_len(n_in[i], orig[i], new_freq);
+        it.table = -1;
+        it.u_in = it.u_out = it.W = 1;
+        if (orig[i] != new_freq) {
+            plan->copy_only = false;
+            size_t r = std::find(rates.begin(), rates.end(), orig[i]) - rates.begin();
+            if (r == rates.size()) {
+                ResampleItem t{};
+                t.table = (long long)align_up(blob.size(), 16);
+                if (!append_kaldi_table(orig[i], new_freq, blob, &t.u_in, &t.u_out, &t.W))
+                    return fail(IRIS_ERR_UNSUPPORTED, std::string(who) + ": rate pair needs a filter bank above 32 MB");
+                if (size_t(t.u_out) * t.W * 4 <= 96 * 1024)      // staged in shared memory
+                    plan->smem_floats = std::max(plan->smem_floats, t.u_out * t.W);
+                rates.push_back(orig[i]);
+                tabs.push_back(t);
+            }
+            it.table = tabs[r].table;
+            it.u_in = tabs[r].u_in;
+            it.u_out = tabs[r].u_out;
+            it.W = tabs[r].W;
+        }
+        plan->n_out[i] = it.n_out;
+        in_off += it.n_in * n_chan;
+        out_off += it.n_out * n_chan;
+        total += it.n_out;
+    }
+    // outputs per CTA: 4096 amortise a table load over 4096 * n_chan outputs; smaller inputs get smaller
+    // chunks so that the launch still spreads over the GPU (256: one output per thread)
+    int chunk = 4096;
+    while (chunk > 256 && total / chunk < 1024) chunk >>= 1;
+    long long cta = 0;
+    for (ResampleItem& it : items) {
+        it.cta0 = cta;
+        cta += (it.n_out + chunk - 1) / chunk;
+    }
+    if (cta >= (1ll << 31)) return fail(IRIS_ERR_UNSUPPORTED, std::string(who) + ": more than 2^31 CTAs of output");
+    memcpy(blob.data(), items.data(), items.size() * sizeof(ResampleItem));
+    plan->chunk = chunk;
+    plan->n_ctas = cta;
+    return IRIS_OK;
+}
+
+}  // namespace iris
+
+extern "C" {
 int64_t iris_resample_len(int64_t n_in, int orig_freq, int new_freq) {
     if (n_in <= 0 || orig_freq <= 0 || new_freq <= 0) return 0;
     // kaldi.py::_get_num_LR_output_samples: outputs whose time lies in [0, n_in / orig_freq)
@@ -379,48 +491,18 @@ int iris_resample(iris_ctx* c, const float* wav, int n_chan, int64_t n_in, int o
         CU(cudaMemcpyAsync(d_out, wav, size_t(n_in) * n_chan * 4, cudaMemcpyDefault, st));
         return IRIS_OK;
     }
-    int g = orig_freq;
-    for (int b = new_freq; b;) { const int t = g % b; g = b; b = t; }
-    const int u_in = orig_freq / g, u_out = new_freq / g;
-    const int min_freq = orig_freq < new_freq ? orig_freq : new_freq;
-    const double cutoff = 0.99 * 0.5 * min_freq;              // lowpass_cutoff
-    const double width = 6.0 / (2.0 * cutoff);                // window_width, lowpass_filter_width = 6
-    const float ww = float(width), fo = float(orig_freq), fn = float(new_freq);
-    std::vector<int32_t> first(u_out);
-    std::vector<float> mn(u_out);
-    int W = 0;
-    for (int i = 0; i < u_out; ++i) {
-        const float t = float(i) / fn;
-        mn[i] = ceilf((t - ww) * fo);
-        const float mx = floorf((t + ww) * fo);
-        first[i] = int32_t(mn[i]);
-        W = std::max(W, int(mx - mn[i] + 1.f));
-    }
-    if (size_t(u_out) * W > (8u << 20)) return fail(IRIS_ERR_UNSUPPORTED, "iris_resample: rate pair needs a filter bank above 32 MB");
-    std::vector<float> wt(size_t(u_out) * W);
-    const float cw = float(2 * M_PI * cutoff / 6.0), cs = float(2 * M_PI * cutoff), pi = float(M_PI);
-    for (int i = 0; i < u_out; ++i) {
-        const float t = float(i) / fn;
-        for (int j = 0; j < W; ++j) {
-            const float dt = (mn[i] + float(j)) / fo - t;
-            float w = 0.f;
-            if (fabsf(dt) < ww) w = 0.5f * (1.f + cosf(cw * dt));     // raised-cosine window
-            if (dt != 0.f) w *= sinf(cs * dt) / (pi * dt);              // sinc
-            else w *= float(2 * cutoff);
-            wt[size_t(i) * W + j] = w / fo;
-        }
-    }
-    const int64_t n_out = iris_resample_len(n_in, orig_freq, new_freq);
-    const size_t tab = size_t(u_out) * 4 + wt.size() * 4, raw = size_t(n_in) * n_chan * 4;
+    ResamplePlan plan;
+    const int32_t rate = orig_freq;
+    rc = resample_plan("iris_resample", 1, n_chan, &n_in, &rate, new_freq, &plan);
+    if (rc) return rc;
+    const size_t tab = plan.blob.size(), raw = size_t(n_in) * n_chan * 4;
     CU(c->spec_scratch.reserve(align_up(tab, 256) + raw));
     char* base = c->spec_scratch.as<char>();
-    CU(cudaMemcpyAsync(base, first.data(), size_t(u_out) * 4, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(base + size_t(u_out) * 4, wt.data(), wt.size() * 4, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(base, plan.blob.data(), tab, cudaMemcpyHostToDevice, st));
     float* d_wav = reinterpret_cast<float*>(base + align_up(tab, 256));
     CU(cudaMemcpyAsync(d_wav, wav, raw, cudaMemcpyDefault, st));
-    CU(cudaStreamSynchronize(st));   // the host tables are on the stack of this call
-    CU(launch_resample(d_wav, d_out, n_chan, n_in, n_out, u_in, u_out, W,
-                       reinterpret_cast<const int32_t*>(base), reinterpret_cast<const float*>(base + size_t(u_out) * 4), st));
+    CU(cudaStreamSynchronize(st));   // the host blob is freed when this call returns
+    CU(launch_resample(d_wav, d_out, n_chan, base, 1, plan.n_ctas, plan.chunk, plan.smem_floats, st));
     return IRIS_OK;
 }
 }  // extern "C"

@@ -60,6 +60,35 @@ def default_mel_matrix(num_mel_bins=80, num_spectrogram_bins=257, sample_rate=16
     return np.pad(w.astype(np.float32), [[1, 0], [0, 0]])
 
 
+def bank_item(item):
+    """One waveform-bank item -> (float32 ``[C, N]`` array, sample rate): ``(waveform, sample_rate)``, the
+    in-memory form ``load_wav`` takes, or a plain array, which is 16 kHz audio."""
+    if isinstance(item, tuple):
+        wav, rate = item
+        return np.ascontiguousarray(wav, np.float32), int(rate)
+    return np.ascontiguousarray(item, np.float32), 16000
+
+
+def is_spec_bank(items):
+    """Whether bank ``items`` are spectrograms ``[257, t, 2C]`` rather than waveforms (arrays ``[C, N]`` or
+    ``(waveform, sample_rate)`` tuples)."""
+    return not isinstance(items[0], tuple) and np.asarray(items[0]).ndim == 3
+
+
+def pack_waveforms(items):
+    """Waveform-bank items (see :func:`bank_item`) -> (packed float32 samples, offsets int64 ``[n + 1]`` of the
+    per-channel sample counts at each item's own rate, sample rates int32 ``[n]``, channels): the arguments
+    of ``iris_bank_register(_audio)``."""
+    waves, rates = zip(*(bank_item(x) for x in items))
+    n_chan = waves[0].shape[0]
+    assert all(w.ndim == 2 and w.shape[0] == n_chan for w in waves), \
+        'each waveform must be [chan, samples]'
+    offsets = np.zeros(len(waves) + 1, np.int64)
+    offsets[1:] = np.cumsum([w.shape[1] for w in waves])
+    packed = np.concatenate([w.reshape(-1) for w in waves])
+    return packed, offsets, np.asarray(rates, np.int32), n_chan
+
+
 class Engine:
     """One engine (= one ``iris_ctx``) per CUDA device."""
 
@@ -143,28 +172,33 @@ class Engine:
         return frames
 
     def register_bank(self, kind, waveforms, labels=None, normalize=True):
-        """``waveforms``: list of float32 ``[C, N_i]`` arrays (the audio load_wav reads,
-        data_utils.py:19).  ``labels``: ``[n_items, K]`` one-hot rows (voice bank)."""
-        if np.asarray(waveforms[0]).ndim == 3:
+        """``waveforms``: list of float32 ``[C, N_i]`` arrays of 16 kHz audio or ``(waveform, sample_rate)``
+        tuples at any rate, mixed freely (the audio load_wav reads, data_utils.py:19-22; items not at 16 kHz
+        are resampled on the device with load_wav's filter), or spectrograms ``[257, t, 2C]``
+        (:meth:`register_spec_bank`).  ``labels``: ``[n_items, K]`` one-hot rows (voice bank)."""
+        if is_spec_bank(waveforms):
             return self.register_spec_bank(kind, waveforms, labels=labels)
-        waves = [np.ascontiguousarray(w, np.float32) for w in waveforms]
-        n_chan = waves[0].shape[0]
-        assert all(w.ndim == 2 and w.shape[0] == n_chan for w in waves), \
-            'each waveform must be [chan, samples]'
-        offsets = np.zeros(len(waves) + 1, np.int64)
-        offsets[1:] = np.cumsum([w.shape[1] for w in waves])
-        packed = np.concatenate([w.reshape(-1) for w in waves])
+        packed, offsets, rates, n_chan = pack_waveforms(waveforms)
+        n = len(rates)
         lab = None
         n_classes = 0
         if labels is not None:
             lab = np.ascontiguousarray(labels, np.float32)
-            assert lab.shape[0] == len(waves)
+            assert lab.shape[0] == n
             n_classes = lab.shape[1]
-        L.check(self.lib.iris_bank_register(
-            self._ctx, kind, len(waves), n_chan, packed.ctypes.data, offsets.ctypes.data,
-            lab.ctypes.data if lab is not None else None, n_classes, int(bool(normalize)),
-            self._stream()))
-        frames = np.zeros(len(waves), np.int32)
+        lab_p = lab.ctypes.data if lab is not None else None
+        if (rates == 16000).all():
+            L.check(self.lib.iris_bank_register(
+                self._ctx, kind, n, n_chan, packed.ctypes.data, offsets.ctypes.data, lab_p, n_classes,
+                int(bool(normalize)), self._stream()))
+        else:
+            if not hasattr(self.lib, 'iris_bank_register_audio'):
+                raise NotImplementedError('this libiris predates iris_bank_register_audio: resample the items '
+                                          'to 16 kHz first')
+            L.check(self.lib.iris_bank_register_audio(
+                self._ctx, kind, n, n_chan, packed.ctypes.data, offsets.ctypes.data, rates.ctypes.data, lab_p,
+                n_classes, int(bool(normalize)), self._stream()))
+        frames = np.zeros(n, np.int32)
         L.check(self.lib.iris_bank_info(self._ctx, kind, None, None, frames.ctypes.data))
         self.bank_frames[kind] = frames
         self.bank_chan = n_chan

@@ -27,14 +27,14 @@ import numpy as np
 
 from . import _lib as L
 from . import _ops as O
-from .engine import Engine, get_engine
+from .engine import Engine, get_engine, is_spec_bank
 from .plan import ShuffleStream, draw_batch, draw_config, stream_handles, uniforms_per_clip
 
 AUTOTUNE = -1   # tf.data.experimental.AUTOTUNE stand-in for .prefetch()
 
 
 def _is_waveform_bank(items):
-    return np.asarray(items[0]).ndim == 2
+    return isinstance(items[0], tuple) or np.asarray(items[0]).ndim == 2
 
 
 class IrisDataset:
@@ -284,7 +284,7 @@ def merge_complex_specs(background, voices_and_labels, noises=None, n_frame=300,
         labels: (n_voices, time, n_classes)
     '''
     voices, labels = voices_and_labels
-    if np.asarray(background).ndim not in (2, 3):
+    if not isinstance(background, tuple) and np.asarray(background).ndim not in (2, 3):
         raise ValueError('background must be a spectrogram [freq, time, chan2] or a waveform [chan, samples]')
     if t_axis != 1:
         raise NotImplementedError('merge_complex_specs: t_axis must be 1 (the only value the reference uses)')
@@ -328,7 +328,7 @@ def make_pipeline(backgrounds,  # a list of background noises  (waveforms [chan,
     (pipeline.py:113-175; kwargs = merge_complex_specs' min_ratio / min_noise_ratio / snr)
     '''
     # pipeline.py:136 asserts 3-D spectrograms; waveform banks [chan, samples] are accepted too
-    assert len(np.asarray(backgrounds[0]).shape) in (2, 3), 'each spec must be a 3D-tensor'
+    assert _is_waveform_bank(backgrounds) or is_spec_bank(backgrounds), 'each spec must be a 3D-tensor'
     assert len(voices) == len(labels)
     assert len(np.asarray(labels[0]).shape) == 1 and np.asarray(labels[0]).shape[0] == n_classes, \
         'labels must be in the form of [n_samples, n_classes]'

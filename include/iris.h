@@ -116,6 +116,17 @@ int iris_specbank_register(iris_ctx* ctx, int kind, int n_items, int n_freq, int
 int iris_bank_register(iris_ctx* ctx, int kind, int n_items, int n_chan, const float* packed_wav,
                        const int64_t* offsets, const float* labels, int n_classes, int normalize,
                        iris_stream stream);
+/* The same from audio at any sample rate, as load_wav reads it (data_utils.py:19-22): item i is
+ * [n_chan, len_i] at sample_rates[i] Hz (host, >= 1), packed and counted by `offsets` as above.  Every
+ * item not at 16 kHz is resampled to 16 kHz with iris_resample's filter (Kaldi LinearResample) by one
+ * device pass over the bank; the 16 kHz items are then registered exactly as iris_bank_register
+ * registers them (normalize over the resampled item, layout, activity), so iris_bank_info reports the
+ * frames of the iris_resample_len lengths and a bank whose rates are all 16000 is registered bit for
+ * bit as by iris_bank_register.  A rate pair whose filter bank exceeds 32 MB is IRIS_ERR_UNSUPPORTED.
+ * Added under IRIS_ABI_VERSION 2: callers probe for the symbol. */
+int iris_bank_register_audio(iris_ctx* ctx, int kind, int n_items, int n_chan, const float* packed_wav,
+                             const int64_t* offsets, const int32_t* sample_rates, const float* labels,
+                             int n_classes, int normalize, iris_stream stream);
 int iris_bank_info(iris_ctx* ctx, int kind, int32_t* n_items, int32_t* n_chan,
                    int32_t* n_frames /* [n_items] or NULL */);
 int iris_bank_activity(iris_ctx* ctx, int item, uint8_t* host_out /* [n_frames[item]] */);
