@@ -143,6 +143,7 @@ int prepare_fused(iris_ctx* c, FusedParams& p, int mode, int max_segs) {
     p.max_segs = max_segs < 1 ? 1 : max_segs;
     p.stage_out = fused_stages_output(mode, p.remap, p.fr) ? 1 : 0;
     p.fm_bits = (mode == FM_MEL && p.mel_f_lo + p.mel_f_n <= 128) ? 1 : 0;   // = the NJ == 4 kernels
+    p.plane = fused_reads_plane(p, mode) ? 1 : 0;
     p.pair_merge = p.stage_out && p.C == 4 ? 1 : 0;
     int stride = 0;
     const size_t bytes = fused_tile_bytes(p, &stride);
@@ -164,7 +165,7 @@ bool tile_sig_matches(const iris_ctx* c, const FusedParams& p) {
     const iris_ctx::TileSig& g = c->tile_sig;
     return g.valid && g.segs == p.segs && g.keep == p.keep && g.B == p.B && g.T == p.T && g.fm_bits == p.fm_bits && g.seg_select == p.seg_select && g.fr == p.fr &&
            g.n_pairs == p.n_pairs && g.max_segs == p.max_segs && g.stride == p.tile_stride &&
-           g.masks == ((p.tmask ? 1 : 0) | (p.fmask ? 2 : 0)) && g.filter_k == p.filter_k;
+           g.masks == ((p.tmask ? 1 : 0) | (p.fmask ? 2 : 0)) && g.filter_k == p.filter_k && g.plane == p.plane;
 }
 void tile_sig_set(iris_ctx* c, const FusedParams& p) {
     iris_ctx::TileSig& g = c->tile_sig;
@@ -174,6 +175,7 @@ void tile_sig_set(iris_ctx* c, const FusedParams& p) {
     g.max_segs = p.max_segs; g.stride = p.tile_stride;
     g.masks = (p.tmask ? 1 : 0) | (p.fmask ? 2 : 0);
     g.filter_k = p.filter_k;
+    g.plane = p.plane;
 }
 
 // k_tiles + k_fused over the whole batch; k_tiles is skipped when the tile blocks of this plan
@@ -266,6 +268,21 @@ int feature_params(iris_ctx* c, int mode, int select, FusedParams& p) {
     if (mel) {
         p.do_log = mode != IRIS_FEAT_MEL;
         p.do_minmax = mode == IRIS_FEAT_LOGMEL_MINMAX;
+        // the bin planes of the plan's banks, for the launches that read them (fused_reads_plane)
+        bool planes = c->C == 2;
+        int k = 0;
+        for (int kind : {IRIS_BANK_BG, IRIS_BANK_VOICE, IRIS_BANK_NOISE}) {
+            const Bank& bk = c->banks[kind];
+            const bool used = kind == IRIS_BANK_BG || (kind == IRIS_BANK_VOICE ? c->V > 0 : c->M > 0);
+            if (!used) continue;
+            if (!bk.ready || bk.spec || bk.n_chan != 2 || !bk.plane.p) { planes = false; break; }
+            p.pl_wave[k] = bk.padded.as<float>();
+            p.pl_floats[k] = int64_t(bk.plane_floats);
+            p.pl_delta[k] = (int64_t(uintptr_t(bk.plane.p)) - int64_t(uintptr_t(bk.padded.p))) / 4;
+            ++k;
+        }
+        if (!planes)
+            for (int i = 0; i < 3; ++i) { p.pl_wave[i] = nullptr; p.pl_floats[i] = 0; p.pl_delta[i] = 0; }
     }
     return prepare_fused(c, p, mel ? FM_MEL : mode == IRIS_FEAT_SE ? FM_SE : mode, c->max_segs);
 }
@@ -397,7 +414,7 @@ int iris_ctx_destroy(iris_ctx* c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (auto& b : c->banks) {
-        b.padded.release(); b.activity.release(); b.labels.release(); b.d_n_frames.release();
+        b.padded.release(); b.activity.release(); b.labels.release(); b.d_n_frames.release(); b.plane.release();
     }
     for (auto& pb : c->plan_blobs) pb.release();
     if (c->copy) {
@@ -642,14 +659,11 @@ int bank_fill(iris_ctx* c, int kind, DevBuf& wav16, const float* labels, int nor
                        cudaMemcpyHostToDevice, st));
     CU(launch_bank_prepare(wav16.as<float>(), d_o, d_o + n_items + 1, n_items, n_chan, normalize,
                            b.padded.as<float>(), st));
-    if (kind == IRIS_BANK_VOICE) {
-        CU(b.labels.reserve(size_t(n_items) * n_classes * 4));
-        CU(cudaMemcpyAsync(b.labels.p, labels, size_t(n_items) * n_classes * 4,
-                           cudaMemcpyHostToDevice, st));
-        // activity: one STFT pass over every voice, frame active iff any coefficient > 0
-        const size_t act_bytes = size_t(n_items) * b.max_frames;
-        CU(b.activity.reserve(act_bytes));
-        CU(cudaMemsetAsync(b.activity.p, 0, act_bytes, st));
+    b.plane_floats = 0;
+    if (n_chan != 2) b.plane.release();
+    if (kind == IRIS_BANK_VOICE || n_chan == 2) {
+        // the STFT passes over the bank: one segment per item, gain 1 (the split of the packed two-channel
+        // FFT then gives X itself)
         std::vector<Seg> segs(n_items);
         std::vector<int32_t> ptr(n_items + 1);
         for (int i = 0; i < n_items; ++i) {
@@ -678,12 +692,31 @@ int bank_fill(iris_ctx* c, int kind, DevBuf& wav16, const float* labels, int nor
         p.B = n_items;
         p.T = b.max_frames;
         set_geometry(c, p, n_chan, false);
-        p.activity = b.activity.as<uint8_t>();
-        const int rc = run_fused(c, p, FM_ACTIVITY, 1, st);
-        c->tile_sig.valid = false;   // the segment list of this pass is freed below
-        if (rc) return rc;
-        b.h_activity.resize(act_bytes);
-        CU(cudaMemcpyAsync(b.h_activity.data(), b.activity.p, act_bytes, cudaMemcpyDeviceToHost, st));
+        if (n_chan == 2) {
+            // the bin plane: bins 0..127 of every frame, the rows behind an item's last frame zero
+            CU(b.plane.reserve(pad_floats * 4));
+            CU(cudaMemsetAsync(b.plane.p, 0, pad_floats * 4, st));
+            p.pl_delta[0] = (int64_t(uintptr_t(b.plane.p)) - int64_t(uintptr_t(b.padded.p))) / 4;
+            const int rc = run_fused(c, p, FM_PLANE, 1, st);
+            c->tile_sig.valid = false;   // the segment list of this pass is freed below
+            if (rc) return rc;
+            b.plane_floats = pad_floats;
+        }
+        if (kind == IRIS_BANK_VOICE) {
+            CU(b.labels.reserve(size_t(n_items) * n_classes * 4));
+            CU(cudaMemcpyAsync(b.labels.p, labels, size_t(n_items) * n_classes * 4,
+                               cudaMemcpyHostToDevice, st));
+            // activity: frame active iff any coefficient > 0
+            const size_t act_bytes = size_t(n_items) * b.max_frames;
+            CU(b.activity.reserve(act_bytes));
+            CU(cudaMemsetAsync(b.activity.p, 0, act_bytes, st));
+            p.activity = b.activity.as<uint8_t>();
+            const int rc = run_fused(c, p, FM_ACTIVITY, 1, st);
+            c->tile_sig.valid = false;
+            if (rc) return rc;
+            b.h_activity.resize(act_bytes);
+            CU(cudaMemcpyAsync(b.h_activity.data(), b.activity.p, act_bytes, cudaMemcpyDeviceToHost, st));
+        }
         CU(cudaStreamSynchronize(st));
         d_segs.release();
     }
@@ -778,6 +811,8 @@ int iris_specbank_register(iris_ctx* c, int kind, int n_items, int n_freq, int n
     Bank& b = c->banks[kind];
     b.ready = false;
     b.spec = true;
+    b.plane.release();   // spectrogram banks have none (k_specmix reads their bins directly)
+    b.plane_floats = 0;
     b.n_items = n_items;
     b.n_chan = n_chan2 / 2;
     b.n_classes = n_classes;

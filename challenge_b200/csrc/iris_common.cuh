@@ -33,6 +33,7 @@ enum FusedMode : int {
     FM_MEL = 3,
     FM_ACTIVITY = 4,
     FM_SE = 5,   // IRIS_FEAT_SE: x, only_voice, only_noise of the 'se' model (include/iris.h)
+    FM_PLANE = 6,   // bank registration: bins 0..127 of every frame into the bank's STFT bin plane
 };
 
 enum ChanRemap : int { REMAP_NONE = 0, REMAP_STEREO_MONO = 1, REMAP_MERGE_AUG = 2, REMAP_MONO_CHAN = 3 };
@@ -119,6 +120,13 @@ struct FusedParams {
     int32_t mel_L[4];
     const uint32_t* mel_info;  // [n_mel] first tap, relative to mel_f_lo
     const float* mel_w;        // [mel_taps][32]
+    // 2-channel mel from the STFT bin planes of the banks (Bank::plane, k_fused EPI_PLANE): a stage whose
+    // source row s lies in bank k's waveform [pl_wave[k], pl_wave[k] + pl_floats[k]) is read from the
+    // plane row s + pl_delta[k], with the full gain (the plane holds X, not the packed two-channel FFT)
+    int32_t plane;
+    const float* pl_wave[3];
+    int64_t pl_floats[3];
+    int64_t pl_delta[3];    // FM_PLANE (the pass that builds a plane): pl_delta[0] is its own bank's
     // tables (fftwarp.cuh)
     const float4* tw1;      // [8][32] {W512^(n2*2q), W512^(n2*(2q+1))}
     const float4* ts;       // [8][2]  {t(2m), t(2m+1)}, t(i) = par ? W32^i : 1

@@ -60,6 +60,11 @@ struct Bank {
     std::vector<int32_t> n_frames;
     int max_frames = 0;
     DevBuf padded, activity, labels, d_n_frames;
+    // 2-channel waveform banks: the STFT bin plane, the geometry of `padded` (one 2 KB row per frame: bins
+    // 0..127 of frame h as {re0, re1, im0, im1}; the item's last row is zero), read by the mel launches
+    // (fused_reads_plane); `plane_floats` of it are in use
+    DevBuf plane;
+    size_t plane_floats = 0;
     std::vector<uint8_t> h_activity;   // host mirror (voice bank)
 };
 
@@ -139,6 +144,7 @@ struct iris_ctx {
         const void *segs = nullptr, *keep = nullptr;   // the plan (a plan upload invalidates as well)
         int B = 0, T = 0;
         int fm_bits = 0, seg_select = 0, fr = 0, n_pairs = 0, max_segs = 0, stride = 0, masks = 0, filter_k = 0;
+        int plane = 0;   // the stages point into the bin planes (full gains) or into the waveforms (halved)
     } tile_sig;
     int feat_hint = -1;   // feature mode of the last feature launch: what k_labels builds tile blocks for
     cudaEvent_t ev_after_fused = nullptr;   // recorded (once) right behind the next k_fused launch (iris_step)

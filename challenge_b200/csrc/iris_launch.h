@@ -12,6 +12,7 @@ struct FusedParams;
 cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream, bool build_tiles,
                          int out_type);
 size_t fused_smem_bytes(const FusedParams& p, int mode);
+bool fused_reads_plane(const FusedParams& p, int mode);   // FusedParams::plane of a launch
 void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge, int32_t out[5]);
 int fused_max_segments();      // mixing segments one clip may have
 bool fused_stages_output(int mode, int remap, int fr);   // FusedParams::stage_out for a launch

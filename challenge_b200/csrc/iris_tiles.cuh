@@ -79,9 +79,17 @@ __device__ __forceinline__ void build_tile_block(const FusedParams& p, int tile,
         if (n < p.max_segs) {
             StageDesc e;
             e.src = sg.base + size_t(SE ? 0 : pair) * size_t(sg.pair_stride) + size_t(lo + sg.shift) * 512;
+            if (!SE && p.plane) {
+                // the same row of the source's bin plane (one 2 KB row per frame, the waveform's geometry)
+#pragma unroll
+                for (int k = 0; k < 3; ++k)
+                    if (uint64_t(e.src) - uint64_t(p.pl_wave[k]) < uint64_t(p.pl_floats[k]) * 4u)
+                        e.src = reinterpret_cast<const float*>(uint64_t(e.src) + uint64_t(p.pl_delta[k]) * 4u);
+            }
             e.j_lo = uint16_t(lo - t0);
             e.j_cnt = uint16_t(hi - lo);
-            e.gain = 0.5f * sg.gain;   // exact; folds the 1/2 of the two-channel split
+            // exact; the waveform path folds the 1/2 of the two-channel split, a plane holds X itself
+            e.gain = (!SE && p.plane) ? sg.gain : 0.5f * sg.gain;
             d[n++] = e;
         }
     }

@@ -20,7 +20,8 @@
 //  * Tiles are claimed in chunks of consecutive tiles that shrink towards the end of the launch
 //    (fused_schedule): the first claim of a CTA is its block index, the later ones come from a global
 //    counter.  The producer warp copies the TileBlock of each tile into a shared-memory descriptor
-//    ring and fetches every stage -- (j_cnt + 1) contiguous 2 KB rows of the pair-interleaved bank --
+//    ring and fetches every stage -- (j_cnt + 1) contiguous 2 KB rows of the pair-interleaved bank, or
+//    j_cnt rows of the bank's STFT bin plane for the 2-channel mel launches that read it (EPI_PLANE) --
 //    with ONE cp.async.bulk (TMA 1-D) into a ring of 3 (mel) or 2 (spectrogram modes) stage buffers:
 //    full[slot] completes when the bytes have landed, empty[slot] when all FR consumer warps have
 //    read the slot.
@@ -72,7 +73,9 @@ __host__ __device__ inline uint32_t slot_bytes(int fr) { return uint32_t(fr + 1)
 // stage buffers per CTA: the modes that write whole spectrograms trade one stage buffer for
 // the store staging area below
 constexpr int kMelSlots = 3;
-__host__ __device__ constexpr int slots_of(int mode) { return (mode == FM_MEL || mode == FM_ACTIVITY) ? kMelSlots : 2; }
+__host__ __device__ constexpr int slots_of(int mode) {
+    return (mode == FM_MEL || mode == FM_ACTIVITY || mode == FM_PLANE) ? kMelSlots : 2;
+}
 // staging of a tile's [257 bins][FR frames] x 16 B output pieces (16-byte columns XOR-swizzled
 // by the bin so that both the per-frame writes and the per-bin reads are conflict-free)
 __host__ __device__ inline uint32_t stage_bytes(int fr) { return uint32_t(kBins) * uint32_t(fr) * 16u; }
@@ -82,7 +85,7 @@ __host__ __device__ inline uint32_t smem_total(int mel_taps, int fr, int mode, b
 // spectrogram modes without a channel remap (16 B per (bin, frame, pair)) store through the
 // staging area; 8 frames per tile give 128-byte rows
 __host__ __device__ inline bool stages_output(int mode, int remap, int fr) {
-    return mode != FM_MEL && mode != FM_ACTIVITY && remap == REMAP_NONE && fr == 8;
+    return mode != FM_MEL && mode != FM_ACTIVITY && mode != FM_PLANE && remap == REMAP_NONE && fr == 8;
 }
 
 // ---- pre-kernel: one thread per tile builds its TileBlock (launches without a k_labels pass in
@@ -169,14 +172,21 @@ __device__ __forceinline__ void store_piece(const FusedParams& p, int b, int f, 
 // rounds of 32, which is tf.signal.linear_to_mel_weight_matrix(80, 257, 16000), transforms.py:55 --
 // with their switches fixed at compile time (EPI_C2 | EPI_MINMAX or EPI_LOG or neither): no
 // per-round flag branches, no odd-channel selects, C folded into the address arithmetic, the
-// projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.
+// projection loops unrolled to their 12 taps.  Measured: plain mel 202 -> 190 us.  (Those instances now exist
+// with EPI_PLANE only: the 2-channel launches with bins below 128 read the bin planes.)
 // EPI_REMAP: the mel epilogue of a channel remap (stereo_mono / random_merge_aug: 2 input channels, c_out
 // output channels), switches read at run time like EPI == 0.
 // EPI_MONO, alone or on top of the 2-channel variants above: mono_chan (include/iris.h IRIS_REMAP_MONO_CHAN)
 // keeps two channels, so it is the 2-channel epilogue with (re0 + re1, re0 + im_j) formed before |.|.
+// EPI_PLANE (NJ = 4, 2 channels, no remap or mono_chan): no FFT.  A stage is j_cnt rows of the sources' STFT
+// bin planes (Bank::plane: bins 0..127 of one frame per 2 KB row, {re0, re1, im0, im1} per bin); lane l mixes
+// bins l + 32 q in registers, product then sum as pipeline.merge_complex_specs rounds, and the magnitudes go to
+// the same projection, extrema, log and store code as the FFT path.  With EPI_C2 the fixed-shape instance,
+// without it the generic one (IRIS_NO_FIXED_EPI); both do the same arithmetic in the same order.
 // OutT: element type of p.out (float, __nv_bfloat16, __half).  The half instances have no min-max
 // epilogue: the min-max log-mel features are normalised by k_logmel_post, which converts.
-constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4, EPI_REMAP = 8, EPI_MONO = 16;
+// MODE FM_PLANE (NJ = 4) is the registration pass that writes a bank's plane from its waveform.
+constexpr int EPI_MINMAX = 1, EPI_LOG = 2, EPI_C2 = 4, EPI_REMAP = 8, EPI_MONO = 16, EPI_PLANE = 32;
 constexpr int kFixFR = 8;   // frames per tile of the fixed mel variants
 __host__ __device__ constexpr int fixed_mel_L(int r) { return r == 0 ? 2 : (r == 1 ? 4 : (r == 2 ? 6 : 0)); }
 template <int MODE, int NJ, int EPI, class OutT>
@@ -188,6 +198,8 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
     constexpr bool kMel = (MODE == FM_MEL);
     constexpr bool kFix = (EPI & EPI_C2) != 0;   // switches below are compile-time constants
     constexpr bool kRemap = (EPI == EPI_REMAP);
+    constexpr bool kPlane = (EPI & EPI_PLANE) != 0;
+    static_assert(!kPlane || (kMel && NJ == 4), "the plane epilogue is the 2-channel mel epilogue of bins below 128");
     static_assert(!kFix || kMel, "fixed epilogues exist for the mel modes only");
     static_assert(!kRemap || kMel, "the remap epilogue is a mel epilogue");
     constexpr bool kMono = (EPI & EPI_MONO) != 0;
@@ -296,7 +308,9 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                         if (d.j_cnt == 0) {
                             mbar_arrive(&full[slot]);
                         } else {
-                            const uint32_t bytes = (uint32_t(d.j_cnt) + 1u) * 2048u;
+                            // frames j_lo .. j_lo + j_cnt - 1: their plane rows, or the j_cnt + 1 waveform
+                            // rows they span
+                            const uint32_t bytes = (uint32_t(d.j_cnt) + (kPlane ? 0u : 1u)) * 2048u;
                             mbar_arrive_expect_tx(&full[slot], bytes);
                             bulk_g2s_hint(slots + slot * slotB + uint32_t(d.j_lo) * 2048u, d.src, bytes, &full[slot], pol_stream);
                         }
@@ -415,8 +429,40 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
         const size_t clip_elems = size_t(p.n_mel) * p.T * Cm;
         for (int i = 0;; ++i) {
             const TileBlock* tb = reinterpret_cast<const TileBlock*>(sm + OFF_RING + (i & (kRing - 1)) * kTileBlockBytes);
-            // ---- gather + mix: v = sum over the stages of this tile of gain * frame ----
+            int4 hdr;
+            float4 z[4];   // EPI_PLANE: the mixed {re0, re1, im0, im1} of bins lane + 32 q
             cpx v[16];
+            if constexpr (kPlane) {
+                // ---- mix of the stored bins: z = sum over the stages of gain * X, product then sum ----
+                mbar_wait_parked(&full[slot], phase);   // also publishes the TileBlock of this tile
+                hdr = *reinterpret_cast<const int4*>(tb);
+                if (hdr.x == 0) break;                  // end marker
+                // a time-masked frame and one behind the clip's end are not read (they still release
+                // every slot of the tile)
+                const bool live = int(hdr.z & 0xffffff) + j < p.T && !((uint32_t(hdr.w) >> j) & 1u);
+#pragma unroll
+                for (int q = 0; q < 4; ++q) z[q] = make_float4(0.f, 0.f, 0.f, 0.f);
+                for (int e = 0; e < hdr.x; ++e) {
+                    if (e > 0) mbar_wait_parked(&full[slot], phase);
+                    const uint2 dd = *reinterpret_cast<const uint2*>(&tb->d[e].j_lo);   // j_lo | j_cnt << 16, gain
+                    if (live && unsigned(j - int(dd.x & 0xffffu)) < (dd.x >> 16)) {
+                        const float g = __uint_as_float(dd.y);
+                        const float4* src = reinterpret_cast<const float4*>(slots + slot * slotB + j * 2048) + lane;
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            const float4 x = src[32 * q];
+                            z[q].x = __fadd_rn(z[q].x, __fmul_rn(g, x.x));
+                            z[q].y = __fadd_rn(z[q].y, __fmul_rn(g, x.y));
+                            z[q].z = __fadd_rn(z[q].z, __fmul_rn(g, x.z));
+                            z[q].w = __fadd_rn(z[q].w, __fmul_rn(g, x.w));
+                        }
+                    }
+                    __syncwarp();
+                    mbar_arrive_if(&empty[slot], l0);
+                    if (++slot == S) { slot = 0; phase ^= 1u; }
+                }
+            } else {
+            // ---- gather + mix: v = sum over the stages of this tile of gain * frame ----
             mbar_wait_parked(&full[slot], phase);           // also publishes the TileBlock of this tile
             // the rows of the first stage are requested before the tile header is looked at (the end
             // marker's rows are stale but finite): the header's load-to-use latency hides behind them
@@ -428,7 +474,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                     v[q] = cpx{x.x, x.y};
                 }
             }
-            const int4 hdr = *reinterpret_cast<const int4*>(tb);
+            hdr = *reinterpret_cast<const int4*>(tb);
             const int n_st = hdr.x;
             if (n_st == 0) break;                    // end marker
             // (skipping the row reads of time-masked frames -- ~11 % of the frames -- was measured on
@@ -461,6 +507,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 mbar_arrive_if(&empty[slot], l0);
                 if (++slot == S) { slot = 0; phase ^= 1u; }
             }
+            }
 
             const int b = hdr.y;
             const int pair = kFix ? 0 : (hdr.z >> 24);
@@ -480,7 +527,11 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                 if (kMel) clip_out = reinterpret_cast<OutT*>(p.out) + size_t(b) * clip_elems;
                 zbits = 0;
                 const int4 fmv = *reinterpret_cast<const int4*>(tb->fm);
-                if (kMel && NJ == 4) {
+                if (kPlane) {
+                    // the same bitmap; the lane holds bin lane + 32 q, bit `lane` of word q
+                    zbits = ((uint32_t(fmv.x) >> lane) & 1u) | (((uint32_t(fmv.y) >> lane) & 1u) << 1) |
+                            (((uint32_t(fmv.z) >> lane) & 1u) << 2) | (((uint32_t(fmv.w) >> lane) & 1u) << 3);
+                } else if (kMel && NJ == 4) {
                     // k_tiles left a bitmap of the zeroed bins 0..127 (p.fm_bits): bin
                     // k1 + 16 par + 32 jj is bit k1 + 16 par of word jj
                     const int sh = k1 + 16 * par;
@@ -503,7 +554,7 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
             }
 
             cpx u[16];
-            if (do_fft) {
+            if (!kPlane && do_fft) {
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
                     const float wq = w8[32 * q];
@@ -696,11 +747,28 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                         if ((zbits >> bit) & 1u) { m0 = 0.f; m1 = 0.f; }   // |x| * 0 == +0
                         mg[f] = make_float2(m0, m1);
                     };
+                    if constexpr (kPlane) {
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            cpx re{z[q].x, z[q].y}, im{z[q].z, z[q].w};
+                            if constexpr (kMono) {
+                                const float s = re.x + re.y;
+                                im = cpx{re.x + im.x, re.x + im.y};
+                                re = cpx{s, s};
+                            }
+                            const cpx sq = cfma2(im, im, cmul2(re, re));
+                            float m0 = sqrt_approx(sq.x);
+                            float m1 = sqrt_approx(sq.y);
+                            if ((zbits >> q) & 1u) { m0 = 0.f; m1 = 0.f; }
+                            mg[lane + 32 * q] = make_float2(m0, m1);
+                        }
+                    } else {
 #pragma unroll
                     for (int jj = 0; jj < NJ; ++jj) emit(k1 + 16 * (2 * jj + par), jj, u[jj], mirror(jj));
                     if (NJ == 8) {
                         const cpx z8 = u[8];
                         if (l0) emit(256, 8, z8, z8);
+                    }
                     }
                     __syncwarp();
                     // sparse mel projection (transforms.py:51-77): the filter of slot (r, lane) reads
@@ -761,6 +829,19 @@ __global__ void __maxnreg__(kMaxRegs) k_fused(const __grid_constant__ FusedParam
                                 if (has1) store_out1(o + 1, a1);
                             }
                         }
+                    }
+                }
+            } else if (MODE == FM_PLANE) {
+                // bins 0..127 of frame t of item b into row t of its plane (pl_delta[0] floats behind its
+                // waveform): with the stage gain 1/2 the split values are X itself.  One segment per item
+                // (bank_fill); frames past the item's end keep the zeros the plane was cleared to.
+                const Seg sg = p.segs[p.seg_ptr[b]];
+                if (do_fft && t < sg.t_hi) {
+                    float4* row = reinterpret_cast<float4*>(const_cast<float*>(sg.base) + p.pl_delta[0] + size_t(t) * 512);
+#pragma unroll
+                    for (int jj = 0; jj < 4; ++jj) {
+                        const cpx zf = u[jj], zm = mirror(jj);
+                        row[k1 + 16 * (2 * jj + par)] = make_float4(zf.x + zm.x, zf.y + zm.y, zf.y - zm.y, zm.x - zf.x);
                     }
                 }
             } else if (MODE == FM_ACTIVITY) {
@@ -968,6 +1049,16 @@ void fused_debug_schedule(long long n_tiles, int grid, int chunk, int pair_merge
     out[0] = p.chunk; out[1] = p.chunk_mid; out[2] = p.chunk_tail; out[3] = p.n_big; out[4] = p.n_mid;
 }
 
+// The one rule for which launches read the banks' STFT bin planes instead of transforming the waveform: the
+// mel modes of 2-channel waveform banks (the caller has filled pl_wave / pl_floats / pl_delta: every
+// 2-channel waveform bank has a plane) whose channels stay two (no remap, or mono_chan) and whose mel support
+// ends below bin 128 -- the bins a plane row holds.  prepare_fused sets p.plane from it, so that the tile
+// blocks (k_tiles, k_labels) point into the planes.
+bool fused_reads_plane(const FusedParams& p, int mode) {
+    return mode == FM_MEL && p.C == 2 && (p.remap == REMAP_NONE || p.remap == REMAP_MONO_CHAN) &&
+           p.mel_f_lo + p.mel_f_n <= 128 && p.seg_select == 0 && p.pl_wave[0] != nullptr;
+}
+
 // p.tile_blocks (fused_tile_bytes) is provided by the caller; build_tiles: k_tiles builds them first
 // (otherwise the kernel in front -- k_labels -- has built them and triggers early).  out_type: OutType
 // of p.out; FM_ACTIVITY and the min-max epilogue write fp32 only.
@@ -1051,28 +1142,42 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
         case FM_MAGPHASE: IRIS_LAUNCH_OUT(FM_MAGPHASE, 8, 0) break;
         case FM_LOGMAGPHASE: IRIS_LAUNCH_OUT(FM_LOGMAGPHASE, 8, 0) break;
         case FM_MEL: {
-            const bool fixed = p.C == 2 && p.mel_L[0] == fixed_mel_L(0) && p.mel_L[1] == fixed_mel_L(1) &&
-                               p.mel_L[2] == fixed_mel_L(2) && p.mel_L[3] == fixed_mel_L(3) && FR == kFixFR &&
-                               p.mel_taps == 12 && !getenv("IRIS_NO_FIXED_EPI");
-            // the 2-channel choice; X = 0, or EPI_MONO for mono_chan
-#define IRIS_LAUNCH_MEL2(X)                                                                     \
+            // p.plane (fused_reads_plane): 2 channels, no remap or mono_chan, support below bin 128 -- the mix of
+            // the banks' stored bins, fixed-shape or generic instance.  Otherwise the FFT path: NJ = 8 for a
+            // support reaching bin 128, NJ = 4 for C != 2 and the stereo_mono / random_merge_aug remaps.
+            if (p.plane != (fused_reads_plane(p, mode) ? 1 : 0)) return cudaErrorInvalidValue;
+            const bool nj8 = p.mel_f_lo + p.mel_f_n > 128;
+            if (p.plane) {
+                const bool fixed = p.mel_L[0] == fixed_mel_L(0) && p.mel_L[1] == fixed_mel_L(1) &&
+                                   p.mel_L[2] == fixed_mel_L(2) && p.mel_L[3] == fixed_mel_L(3) && FR == kFixFR &&
+                                   p.mel_taps == 12 && !getenv("IRIS_NO_FIXED_EPI");
+                // X = 0, or EPI_MONO for mono_chan
+#define IRIS_LAUNCH_PLANE(X)                                                                    \
     {                                                                                           \
-        if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, X)                         \
-        else if (!fixed) IRIS_LAUNCH_OUT(FM_MEL, 4, X)                                          \
-        else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_C2 | EPI_MINMAX | X, float)            \
-        else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | EPI_LOG | X)                     \
-        else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_C2 | X)                                             \
+        if (!fixed) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | X)                                   \
+        else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_PLANE | EPI_C2 | EPI_MINMAX | X, float) \
+        else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | EPI_C2 | EPI_LOG | X)         \
+        else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | EPI_C2 | X)                                 \
     }
-            // a remap keeps p.C == 2: it must be tested before the fixed 2-channel instances
-            if (p.remap == REMAP_MONO_CHAN) IRIS_LAUNCH_MEL2(EPI_MONO)
-            else if (p.remap != REMAP_NONE) {
-                if (p.mel_f_lo + p.mel_f_n > 128) IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_REMAP)
+                if (p.remap == REMAP_MONO_CHAN) IRIS_LAUNCH_PLANE(EPI_MONO)
+                else IRIS_LAUNCH_PLANE(0)
+#undef IRIS_LAUNCH_PLANE
+            } else if (p.remap == REMAP_MONO_CHAN) {
+                if (!nj8) return cudaErrorInvalidValue;   // bins below 128 only: the plane path
+                IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_MONO)
+            } else if (p.remap != REMAP_NONE) {
+                if (nj8) IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_REMAP)
                 else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_REMAP)
-            } else IRIS_LAUNCH_MEL2(0)
-#undef IRIS_LAUNCH_MEL2
+            } else if (nj8) {
+                IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
+            } else {
+                if (p.C == 2) return cudaErrorInvalidValue;   // the plane path
+                IRIS_LAUNCH_OUT(FM_MEL, 4, 0)
+            }
             break;
         }
         case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0, float) break;
+        case FM_PLANE: IRIS_LAUNCH(FM_PLANE, 4, 0, float) break;
         case FM_SE:   // both virtual pairs of a (clip, time) range in one CTA: the combined store
             if (out_type != OUT_F32 || !p.pair_merge || p.seg_select != 3) return cudaErrorInvalidValue;
             IRIS_LAUNCH(FM_SE, 8, 0, float)
