@@ -92,6 +92,8 @@ SIGNATURES = {
     'iris_features_select': (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     'iris_stft': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int, C.c_void_p,
                             C.c_void_p]),
+    'iris_istft': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_void_p,
+                             C.c_void_p]),
     'iris_metric_counts': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                      C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p]),
@@ -175,7 +177,7 @@ SIGNATURES = {
     'iris_max_segments': (C.c_int, []),
 }
 # symbols added under IRIS_ABI_VERSION 2 that an older library lacks (callers probe with hasattr)
-OPTIONAL = {'iris_bank_register_audio'}
+OPTIONAL = {'iris_bank_register_audio', 'iris_istft'}
 PW_C2MP, PW_MP2C, PW_LOG_MAGPHASE, PW_LOG_ON_MEL, PW_MULTIPLY = range(5)
 MAP_MONO_CHAN, MAP_STEREO_MONO, MAP_MERGE_AUG = range(3)
 

@@ -12,7 +12,7 @@ CSRC = os.path.join(HERE, 'csrc')
 OBJ = os.path.join(HERE, 'build')
 LIB = os.path.join(HERE, 'libiris.so')
 SOURCES = ['iris_abi.cu', 'k_fused.cu', 'k_post.cu', 'k_bank.cu', 'k_labels.cu', 'k_metrics.cu',
-           'k_ops.cu', 'k_eval.cu', 'k_spec.cu', 'k_resample.cu', 'iris_ops_abi.cu', 'iris_step.cu']
+           'k_ops.cu', 'k_eval.cu', 'k_spec.cu', 'k_resample.cu', 'k_istft.cu', 'iris_ops_abi.cu', 'iris_step.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17',
               '--expt-relaxed-constexpr', '-Xcompiler', '-fPIC']
 

@@ -103,6 +103,10 @@ struct ResampleItem {
 cudaError_t launch_resample(const float* wav, float* out, int n_chan, const char* d_blob, int n_items,
                             long long n_ctas, int chunk, int smem_floats, cudaStream_t st);
 
+// k_istft.cu -- torch.istft of [B,257,T,2C] spectrograms into [B,C,L] (L >= 1); tw1: the ctx's warp FFT twiddles
+cudaError_t launch_istft(const float* spec, float* out, int B, int T, int C, long long L, const float4* tw1,
+                         cudaStream_t st);
+
 // k_spec.cu -- spectrogram-format banks (the reference's pickled [257, t, 2C] lists)
 cudaError_t launch_spec_activity(const float* specs, const int64_t* frame_off, int n_items, int F, int W,
                                  int max_frames, uint8_t* activity, cudaStream_t st);

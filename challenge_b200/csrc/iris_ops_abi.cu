@@ -352,6 +352,25 @@ int iris_op_phase_vocoder(iris_ctx* c, const float* x, float* out, int n_freq, i
     return IRIS_OK;
 }
 
+// torch.istft of load_wav's STFT (k_istft.cu)
+int iris_istft(iris_ctx* c, const float* spec, int batch, int n_frames, int n_chan, int64_t length, float* out,
+               iris_stream stream) {
+    int rc = begin(c);
+    if (rc) return rc;
+    if (!spec || !out || batch < 1 || n_frames < 1 || n_chan < 1)
+        return fail(IRIS_ERR_INVALID, "iris_istft: bad argument");
+    if (reinterpret_cast<uintptr_t>(spec) & 15)
+        return fail(IRIS_ERR_INVALID, "iris_istft: the spectrogram must be 16-byte aligned (vector loads)");
+    const int64_t L = length > 0 ? length : int64_t(kHop) * (n_frames - 1);
+    if (L == 0)
+        return fail(IRIS_ERR_INVALID, "iris_istft: a single frame has no samples at the default length; pass length > 0");
+    if (batch > 65535) return fail(IRIS_ERR_UNSUPPORTED, "iris_istft: more than 65535 items");
+    if (n_chan > 32) return fail(IRIS_ERR_UNSUPPORTED, "iris_istft: more than 32 channels");
+    if (L > 0x7fffffffll) return fail(IRIS_ERR_UNSUPPORTED, "iris_istft: length above 2^31 - 1 samples");
+    CU(launch_istft(spec, out, batch, n_frames, n_chan, L, c->tw.as<float4>(), static_cast<cudaStream_t>(stream)));
+    return IRIS_OK;
+}
+
 }  // extern "C"
 
 // torchaudio.compliance.kaldi.resample_waveform (data_utils.py:20-21): Kaldi's LinearResample.

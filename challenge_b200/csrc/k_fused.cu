@@ -107,21 +107,6 @@ __global__ void __launch_bounds__(128) k_tiles(const FusedParams p) {
 
 // one (bin, frame, channel pair) of the spectrogram modes without a channel remap:
 // {first-half ch0, ch1, second-half ch0, ch1} = (re, re, im, im) or (|.|, |.|, phase, phase)
-// W32^(2m), W32^(2m+1) as (cos, sin) of -2 pi i / 32, handed to f as compile-time constants
-template <class F>
-__device__ __forceinline__ void constexpr_for_pair(int m, F f) {
-    switch (m) {   // m is a constant of an unrolled loop: the switch folds away
-        case 0: f(1.f, 0.f, float(cx_cos2pi(1, 32)), -float(cx_sin2pi(1, 32))); break;
-        case 1: f(float(cx_cos2pi(2, 32)), -float(cx_sin2pi(2, 32)), float(cx_cos2pi(3, 32)), -float(cx_sin2pi(3, 32))); break;
-        case 2: f(float(cx_cos2pi(4, 32)), -float(cx_sin2pi(4, 32)), float(cx_cos2pi(5, 32)), -float(cx_sin2pi(5, 32))); break;
-        case 3: f(float(cx_cos2pi(6, 32)), -float(cx_sin2pi(6, 32)), float(cx_cos2pi(7, 32)), -float(cx_sin2pi(7, 32))); break;
-        case 4: f(float(cx_cos2pi(8, 32)), -float(cx_sin2pi(8, 32)), float(cx_cos2pi(9, 32)), -float(cx_sin2pi(9, 32))); break;
-        case 5: f(float(cx_cos2pi(10, 32)), -float(cx_sin2pi(10, 32)), float(cx_cos2pi(11, 32)), -float(cx_sin2pi(11, 32))); break;
-        case 6: f(float(cx_cos2pi(12, 32)), -float(cx_sin2pi(12, 32)), float(cx_cos2pi(13, 32)), -float(cx_sin2pi(13, 32))); break;
-        default: f(float(cx_cos2pi(14, 32)), -float(cx_sin2pi(14, 32)), float(cx_cos2pi(15, 32)), -float(cx_sin2pi(15, 32))); break;
-    }
-}
-
 template <int MODE>
 __device__ __forceinline__ float4 make_piece(const FusedParams& p, int f, float r0, float i0, float r1,
                                              float i1, float m) {

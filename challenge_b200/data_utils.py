@@ -202,6 +202,26 @@ def cast_features(dtype):
     return _cast_features
 
 
+def to_waveform(x, y=None, *, length=None):
+    """Not a reference function: complex spectrograms back to audio, ``[257, T, 2C]`` -> ``[C, L]`` or
+    ``[B, 257, T, 2C]`` -> ``[B, C, L]`` (``iris_istft``: ``torch.istft`` with ``load_wav``'s STFT parameters,
+    ``L = 256 (T - 1)`` unless ``length`` is given).  The inverse of ``load_wav`` up to its normalisation.
+    As a dataset stage (``.map(to_waveform)``) it converts ``x`` and, for a ``seperate_noise_voice=True``
+    source, the ``only_voice`` / ``only_noise`` members of ``y = (labels, only_voice, only_noise)``; labels
+    pass through."""
+    from .engine import istft_shape
+    parts = [x] + ([y[1], y[2]] if isinstance(y, tuple) and len(y) == 3 else [])
+    for p in parts:   # shapes are checked before anything reaches the device
+        istft_shape(np.shape(p), length)
+    eng = get_engine()
+    x = eng.istft(x, length)
+    if y is None:
+        return x
+    if isinstance(y, tuple) and len(y) == 3:
+        y = (y[0], eng.istft(y[1], length), eng.istft(y[2], length))
+    return x, y
+
+
 def speech_enhancement_preprocess(x, y=None):
     """
     :param y: ([..., n_voices, n_frames, n_classes], ..., ...)

@@ -89,6 +89,23 @@ def pack_waveforms(items):
     return packed, offsets, np.asarray(rates, np.int32), n_chan
 
 
+def istft_shape(shape, length=None):
+    """Spectrogram shape ``[257, T, 2C]`` or ``[B, 257, T, 2C]`` and ``length`` (None: ``256 (T - 1)``) ->
+    (B, T, C, L) of ``Engine.istft``; ValueError for anything else."""
+    shape = tuple(int(s) for s in shape)
+    if len(shape) not in (3, 4) or shape[-3] != 257 or shape[-1] < 2 or shape[-1] % 2 or shape[-2] < 1 \
+            or (len(shape) == 4 and shape[0] < 1):
+        raise ValueError('istft takes [257, T, 2C] or [B, 257, T, 2C] spectrograms (T >= 1), not %s' % (shape,))
+    T = shape[-2]
+    if length is None:
+        length = 256 * (T - 1)
+        if length == 0:
+            raise ValueError('a single frame has no samples at the default length: pass length')
+    elif int(length) < 1:
+        raise ValueError('length must be positive, not %r' % (length,))
+    return (shape[0] if len(shape) == 4 else 1), T, shape[-1] // 2, int(length)
+
+
 class Engine:
     """One engine (= one ``iris_ctx``) per CUDA device."""
 
@@ -507,6 +524,20 @@ class Engine:
         L.check(self.lib.iris_stft(self._ctx, C.c_void_p(ptr), n_chan, n, int(bool(normalize)),
                                    self._ptr(out), self._stream()))
         return out
+
+    def istft(self, spec, length=None):
+        """The inverse of :meth:`stft` without its normalisation: ``torch.istft(n_fft=512, hop_length=256,
+        window=torch.hann_window(512), center=True, length=length)`` of every channel of ``[257, T, 2C]`` ->
+        ``[C, L]`` or ``[B, 257, T, 2C]`` -> ``[B, C, L]`` (device float32); ``L = 256 (T - 1)`` without a
+        ``length``."""
+        torch = _torch()
+        B, T, n_chan, n = istft_shape(np.shape(spec), length)
+        x = torch.as_tensor(spec).to(device=self.device, dtype=torch.float32).contiguous()
+        if x.data_ptr() % 16:   # a view into a larger tensor: the kernel reads 16-byte cells
+            x = x.clone()
+        out = self._empty((B, n_chan, n))
+        L.check(self.lib.iris_istft(self._ctx, self._ptr(x), B, T, n_chan, n, self._ptr(out), self._stream()))
+        return out if len(np.shape(spec)) == 4 else out[0]
 
     def resample(self, wav, orig_freq, new_freq=16000):
         """``torchaudio.compliance.kaldi.resample_waveform`` (data_utils.py:20-21) on an in-memory

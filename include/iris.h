@@ -194,6 +194,21 @@ int iris_features_select(iris_ctx* ctx, int mode, int select, float* d_out, iris
 int iris_stft(iris_ctx* ctx, const float* wav, int n_chan, int64_t n_samples, int normalize,
               float* d_out, iris_stream stream);
 
+/* The inverse: torch.istft(X, n_fft=512, hop_length=256, window=torch.hann_window(512) (periodic),
+ * center=True, normalized=False, onesided=True, length) of every channel.
+ *   d_spec [batch, 257, n_frames, 2*n_chan] device float32 in the layout iris_stft writes (real parts of
+ *          the channels, then their imaginary parts), 16-byte aligned; the imaginary parts of bins 0 and
+ *          256 are ignored, as torch's C2R transform ignores them
+ *   d_out  [batch, n_chan, L] device float32, L = length, or 256 * (n_frames - 1) for length <= 0.  A
+ *          length past 256 * (n_frames - 1) gets the last frame's second half (over its window-square
+ *          envelope, as torch computes it) and then zeros.
+ * Deterministic: every output sample is the sum of its two frames in a fixed order.  Bad pointers or
+ * shapes and an empty default output (n_frames = 1 without a length) are IRIS_ERR_INVALID; batch above
+ * 65535, n_chan above 32 and L above 2^31 - 1 are IRIS_ERR_UNSUPPORTED.  Added under IRIS_ABI_VERSION 2:
+ * callers probe for the symbol. */
+int iris_istft(iris_ctx* ctx, const float* d_spec, int batch, int n_frames, int n_chan, int64_t length,
+               float* d_out, iris_stream stream);
+
 /* metrics.er_score(smoothing=False) integer core (metrics.py:217-266) and tfa F1Score
  * micro counts (metrics.py:290-298) for y_true, y_pred [B,T,K] device floats.
  *   d_triples : [B,3] int32  (n_true, n_pred, correct)
