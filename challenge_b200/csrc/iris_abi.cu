@@ -632,6 +632,9 @@ int bank_layout(iris_ctx* c, int kind, int n_items, int n_chan, const int64_t* o
             return fail(IRIS_ERR_INVALID,
                         "source shorter than 257 samples (reflect padding needs pad < length)");
         const int64_t kT = 1 + n / kHop;
+        if (n_chan > 2 && 2 * 256 * (kT + 1) > INT32_MAX)
+            return fail(IRIS_ERR_UNSUPPORTED,
+                        "a source of 3 or more channels longer than 1073741311 samples (pair stride above 2^31 - 1)");
         b.n_frames[i] = int32_t(kT);
         if (kT > b.max_frames) b.max_frames = int(kT);
         b.pad_offsets[i + 1] = b.pad_offsets[i] + 256 * (kT + 1);
@@ -1207,6 +1210,10 @@ int iris_stft(iris_ctx* c, const float* wav, int n_chan, int64_t n, int normaliz
     const int64_t kT = 1 + n / kHop, plen = 256 * (kT + 1);
     if (n_chan > 32) return fail(IRIS_ERR_UNSUPPORTED, "more than 32 channels");
     const int n_pairs = (n_chan + 1) / 2;
+    // Seg::pair_stride (floats between pair planes) is an int32_t; only a second pair plane uses it
+    if (n_pairs > 1 && 2 * plen > INT32_MAX)
+        return fail(IRIS_ERR_UNSUPPORTED, "iris_stft: 3 or more channels of more than 1073741311 samples "
+                                          "(pair stride above 2^31 - 1)");
     CU(c->stft_pad.reserve((size_t(plen) * n_pairs * 2 + size_t(n) * n_chan) * 4));
     CU(c->stft_small.reserve(256));
     float* P = c->stft_pad.as<float>();
