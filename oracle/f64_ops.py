@@ -1,7 +1,7 @@
 """Float64 values and per-cell error bounds of the stand-alone drop-in operations (TEST INFRASTRUCTURE ONLY).
 
 The functions of ``challenge_b200.{data_utils,transforms,metrics,trainer}`` run one stand-alone kernel each
-(k_ops.cu, k_resample.cu, the STFT of ``iris_stft``).  Their inputs are exact float32 values, so the error a correct
+(k_ops.cu, k_resample.cu, the STFT of ``iris_stft``, the inverse STFT of ``iris_istft``).  Their inputs are exact float32 values, so the error a correct
 float32 implementation may make in an output cell is a forward-error bound of the operation's own arithmetic,
 computed here next to the float64 value from the size of the terms that went into that cell:
 
@@ -14,7 +14,8 @@ one rounding        u * |value|, plus TINY = 2^-149 where a product may land in 
 Operations whose result is decided by selections, 0 / 1 factors and a fixed order of float32 operations are
 given as the float32 computation itself, in the kernel's order (``*_f32``): the kernel must match it bit for bit.
 
-Only ``load_wav`` / ``Engine.stft`` uses a calibrated constant: the 'complex' cell of oracle/f64.py with its own
+Only ``load_wav`` / ``Engine.stft`` and the inverse (``to_waveform`` / ``Engine.istft``, KAPPA_ISTFT and SUB_ISTFT
+below) use calibrated constants.  The former is the 'complex' cell of oracle/f64.py with its own
 KAPPA_LOAD, 4x the largest ratio |oracle - f64| / (u S_pair) the float32 oracle (float32 normalisation, torchaudio
 FFT) reaches on the signals of tests/test_f64_ops_host.py, which re-measures it.  It is larger than oracle/f64.py's
 KAPPA_C: these signals put exact-zero stretches, a -100 dB tail and pure DC / Nyquist tones into single frames,
@@ -49,6 +50,15 @@ A_TAB = 11
 # 'zeros' signal at a frame that straddles an exact-zero stretch); KAPPA_LOAD = 4x, as oracle/f64.py's kappas
 MEASURED_RATIO_LOAD = 5.1
 KAPPA_LOAD = 4 * MEASURED_RATIO_LOAD
+# to_waveform: largest |float32 torch.istft - f64| / (u S) over tests/test_istft_host.py istft_cases (4.51, the
+# 'clicks' signal, C = 3: a frame whose energy sits in a few samples); KAPPA_ISTFT = 4x, the same rule.  SUB_ISTFT:
+# 4x the largest |float32 model of k_istft - f64| / (2^-149 G) on bins around 1e-40 and 1e-43 (0.997), where the
+# samples are subnormal and their rounding is absolute; torch.istft cannot calibrate that one, its x w / w^2 rounds
+# x w at the subnormal spacing before dividing by w^2 (1.1e4 times this bound past the last frame's centre)
+MEASURED_RATIO_ISTFT = 4.6
+KAPPA_ISTFT = 4 * MEASURED_RATIO_ISTFT
+MEASURED_SUB_ISTFT = 1.0
+SUB_ISTFT = 4 * MEASURED_SUB_ISTFT
 
 
 def gamma(n):
@@ -122,6 +132,89 @@ def stft_value_bound(wav, normalize=True, frames=None, kappa=KAPPA_LOAD):
     val = np.concatenate([X.real, X.imag], 0).transpose(1, 2, 0)
     s = kappa * U * f64.pair_scale(np.abs(X).transpose(1, 2, 0), False)
     return val, np.concatenate([s, s], -1) + f64.R_OUT * U * np.abs(val)
+
+
+# ---- to_waveform / Engine.istft (iris_istft: k_istft) ----
+def istft_f64(spec, length=None):
+    """torch.istft(n_fft=512, hop_length=256, periodic Hann, center=True, length) in float64 on the CPU of
+    ``[.., 257, T, 2C]`` spectrograms in load_wav's layout (real parts, then imaginary parts) -> ``[.., C, L]``."""
+    import warnings
+    import torch
+    x = torch.as_tensor(np.asarray(spec, np.float64))
+    C = x.shape[-1] // 2
+    z = torch.complex(x[..., :C], x[..., C:]).movedim(-1, -3)          # [.., C, 257, T]
+    lead = z.shape[:-2]
+    with warnings.catch_warnings():   # a length past the last frame is padded with zeros on purpose
+        warnings.simplefilter('ignore', UserWarning)
+        y = torch.istft(z.reshape(-1, 257, z.shape[-1]), 512, 256, window=torch.hann_window(512, dtype=torch.float64),
+                        center=True, length=length)
+    return y.reshape(*lead, y.shape[-1]).numpy()
+
+
+def istft_weights(T, L):
+    """The overlap-add weight of each covering frame, per output sample s = 256 h + r (r < 256) of ``L``:
+    -> (hi [L], lo [L], h [L]).  Frame h contributes with ``hi`` (w[r + 256] / env[r] where frame h + 1 also covers
+    s, 1 / w[r + 256] past the last frame's centre), frame h + 1 with ``lo`` (w[r] / env[r]); env[r] = w[r]^2 +
+    w[r + 256]^2, w the periodic Hann window.  Both are 0 from s = 256 T on, where no frame covers s."""
+    w = 0.5 - 0.5 * np.cos(2 * np.pi * np.arange(512) / 512)
+    s = np.arange(L)
+    h, r = s // 256, s % 256
+    env = w[r] ** 2 + w[r + 256] ** 2
+    two = h + 1 < T
+    hi = np.where(two, w[r + 256] / env, np.where(h < T, 1 / w[r + 256], 0.0))
+    lo = np.where(two, w[r] / env, 0.0)
+    return hi, lo, h
+
+
+def istft_frame_norms(spec):
+    """``[.., 257, T, 2C]`` -> ``[.., C, T]``: per channel, the L2 norm over bins 0 .. 256 of both channels of its
+    channel pair (the complex FFT ``z = X_a + i X_b`` the kernel inverts), without the imaginary parts of bins 0
+    and 256, which the inverse ignores."""
+    x = np.asarray(spec, np.float64)
+    C = x.shape[-1] // 2
+    sq = x * x
+    sq[..., [0, 256], :, C:] = 0
+    e = sq[..., :C] + sq[..., C:]                                        # [.., 257, T, C]
+    e = e.sum(-3)                                                        # [.., T, C]
+    out = np.empty_like(e)
+    for c0 in range(0, C, 2):
+        out[..., c0:c0 + 2] = np.sqrt(e[..., c0:c0 + 2].sum(-1, keepdims=True))
+    return np.swapaxes(out, -1, -2)
+
+
+def istft_spread(per_frame, T, L):
+    """Sum over the (at most two) frames covering each sample of the frame's weight times ``per_frame [.., T]``
+    -> ``[.., L]``."""
+    hi, lo, h = istft_weights(T, L)
+    p = np.concatenate([per_frame, np.zeros(per_frame.shape[:-1] + (2,))], -1)
+    hh = np.minimum(h, T)
+    return hi * p[..., hh] + lo * p[..., hh + 1]
+
+
+def istft_value_bound(spec, length=None):
+    """to_waveform of ``[.., 257, T, 2C]`` -> (value, bound) ``[.., C, L]``.  The bound is KAPPA_ISTFT u S(s) +
+    R_OUT u |value| + SUB_ISTFT 2^-149 G(s): S(s) sums, over the frames covering sample s, the frame's weight
+    (istft_weights) times its channel pair's norm (istft_frame_norms) over sqrt(512); G(s) sums the weights of the
+    covering frames whose pair is not all zero (rounding in the subnormal range, where u |x| no longer bounds it).
+    A sample no frame covers, or only all-zero frames, has a bound of 0: it must be exactly 0."""
+    x = np.asarray(spec, np.float64)
+    T = x.shape[-2]
+    L = 256 * (T - 1) if length is None else int(length)
+    val = istft_f64(x, L)
+    nrm = istft_frame_norms(x)
+    S = istft_spread(nrm / math.sqrt(512), T, L)
+    G = istft_spread((nrm > 0).astype(np.float64), T, L)
+    return val, KAPPA_ISTFT * U * S + f64.R_OUT * U * np.abs(val) + SUB_ISTFT * TINY * G
+
+
+def istft_carry(bound_spec, T, L):
+    """How far an error of the spectrum, at most ``bound_spec [.., 257, T, 2C]`` per cell, moves the exact inverse
+    -> ``[.., C, L]``: per frame and channel (|d0| + |d256| + 2 sum_{k=1}^{255} (|dRe_k| + |dIm_k|)) / 512 (the
+    real inverse FFT; the imaginary parts of bins 0 and 256 are ignored), times the overlap-add weights."""
+    b = np.asarray(bound_spec, np.float64)
+    C = b.shape[-1] // 2
+    e = b[..., 0, :, :C] + b[..., 256, :, :C] + 2 * (b[..., 1:256, :, :C] + b[..., 1:256, :, C:]).sum(-3)
+    return istft_spread(np.swapaxes(e, -1, -2) / 512, T, L)
 
 
 # ---- resample (k_resample) ----

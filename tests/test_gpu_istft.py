@@ -3,19 +3,27 @@ float64 on the CPU: random spectra and real STFTs over channels, batch, frame co
 imaginary parts of DC and Nyquist, load_wav round trips, the pipeline batch and the 'se' triple as audio,
 phase_vocoder output, argument errors and determinism.
 
-The bound is per element (test_istft_host.istft_ratio): |got - ref| <= TOL * peak * g, with peak the largest
-sample of the frames' float64 inverse FFTs and g = sum w / sum w^2 over the frames covering the sample (at most 2
-where two frames overlap, 1 / w past the last frame's centre, where torch divides by a single window square).
-TOL holds with margin: on a B200 the largest ratio measured was 2.2e-7 for the istft alone and 2.7e-7 for the
-load_wav round trips, which add the forward STFT's own float32 error.  Each test prints the ratio it measured."""
+The bound is per sample, oracle/f64_ops.py istft_value_bound (tests/test_gpu_istft_f64.py has the edge shapes and
+quiet inputs): the covering frames' overlap-add weights times their channel pair's norm, so that every item, pair
+and channel is held to its own frames; the load_wav round trips add what the forward STFT's bound moves the exact
+inverse (istft_carry).  Each test prints the largest ratio error / bound it measured, which must be <= 1."""
 import numpy as np
 import pytest
 
-from test_istft_host import frame_peak, istft_f64, istft_ratio
+from oracle import f64, f64_ops as F
+from test_gpu_istft_f64 import round_trip_value_bound
 
 pytestmark = pytest.mark.gpu
 
-TOL = 1e-6
+
+def istft_ratio(got, spec, length=None):
+    """Largest |got - value| / bound of istft_value_bound; samples no frame covers must be exactly +0."""
+    val, bnd = F.istft_value_bound(spec, length)
+    got = np.asarray(got)
+    T = np.shape(spec)[-2]
+    z = got[..., 256 * T:]
+    assert not (np.any(z != 0) or np.signbit(z).any()), 'not +0 from 256 T on'
+    return f64.worst(F.ratio(got, val, bnd))[0]
 
 
 def _np(t):
@@ -44,7 +52,7 @@ def test_random_spectra(engine, C, B, T):
         if B == 1:
             assert np.array_equal(_np(engine.istft(x[0], length)), got[0])
     print('C=%d B=%d T=%d ratio %.3g' % (C, B, T, worst))
-    assert worst <= TOL
+    assert worst <= 1
     if T == 1:
         with pytest.raises(ValueError):
             engine.istft(x)
@@ -60,7 +68,7 @@ def test_real_stfts(engine, C):
         for length in (None, n):
             r = istft_ratio(_np(engine.istft(spec, length)), spec, length)
             print('C=%d n=%d length=%s ratio %.3g' % (C, n, length, r))
-            assert r <= TOL
+            assert r <= 1
 
 
 def test_dc_and_nyquist_imaginary_parts_are_ignored(engine):
@@ -70,7 +78,7 @@ def test_dc_and_nyquist_imaginary_parts_are_ignored(engine):
     z[:, [0, 256], :, 3:] = 0.0
     a, b = _np(engine.istft(x, 40 * 256)), _np(engine.istft(z, 40 * 256))
     assert np.array_equal(a, b)
-    assert istft_ratio(a, z, 40 * 256) <= TOL
+    assert istft_ratio(a, z, 40 * 256) <= 1
 
 
 @pytest.mark.parametrize('n', [256 * 250, 256 * 250 + 1, 256 * 250 + 255, 40000 - 17])
@@ -78,16 +86,14 @@ def test_dc_and_nyquist_imaginary_parts_are_ignored(engine):
 def test_round_trip_through_load_wav(engine, n, C):
     """to_waveform(load_wav(w)) gives back normalize(w) (float64): the whole clip with length=n."""
     from challenge_b200 import data_utils as D
-    from oracle import f64
     w = np.random.default_rng(n + C).standard_normal((C, n)).astype(np.float32)
     spec = D.load_wav(w)
     length = None if n % 256 == 0 else n
     got = _np(D.to_waveform(spec, length=length))
-    ref = f64.normalize_f64(w)
     assert got.shape == (C, n)
-    r = istft_ratio(got, f64.spec_f64(w), length, ref=ref)
+    r = f64.worst(F.ratio(got, *round_trip_value_bound(w, _np(spec))))[0]
     print('round trip C=%d n=%d ratio %.3g' % (C, n, r))
-    assert r <= TOL
+    assert r <= 1
 
 
 def _pipeline(separate, wave):
@@ -108,8 +114,8 @@ def _pipeline(separate, wave):
 @pytest.mark.parametrize('separate', [False, True])
 def test_pipeline_batch_as_audio(engine, separate):
     """make_pipeline(...).map(to_frame_labels).map(augment).map(stft_filter(3)).batch(8).map(to_waveform): the audio
-    is the float64 inverse of the COMPLEX batch of the same seed and the labels are bit-identical.  With
-    seperate_noise_voice=True, only_voice and only_noise become audio too."""
+    is the float64 inverse of the COMPLEX batch of the same seed, each item within the bound of its own frames, and
+    the labels are bit-identical.  With seperate_noise_voice=True, only_voice and only_noise become audio too."""
     plain, wave = _pipeline(separate, False), _pipeline(separate, True)
     for (x, y), (xw, yw) in zip(plain, wave):
         assert tuple(xw.shape) == (8, 2, 256 * 119)
@@ -122,8 +128,8 @@ def test_pipeline_batch_as_audio(engine, separate):
         for got, spec in pairs:
             spec = _np(spec)
             r = istft_ratio(_np(got), spec)
-            print('separate=%d ratio %.3g (peak %.3g)' % (separate, r, frame_peak(spec)))
-            assert r <= TOL
+            print('separate=%d ratio %.3g (peak %.3g)' % (separate, r, np.abs(spec).max()))
+            assert r <= 1
 
 
 def torch_equal(a, b):
@@ -140,7 +146,7 @@ def test_phase_vocoder_as_audio(engine):
         T2 = int(st.shape[1])
         got = _np(D.to_waveform(st))
         assert got.shape == (2, 256 * (T2 - 1))
-        assert istft_ratio(got, _np(st)) <= TOL
+        assert istft_ratio(got, _np(st)) <= 1
 
 
 def test_bad_arguments(engine):
