@@ -217,16 +217,14 @@ int timed_fused(iris_ctx* c, FusedParams& p, int mode, cudaStream_t st, int out_
 }
 
 // min-max log-mel: k_fused (fp32 features + per-clip extrema at p.out) -> k_logmel_post (normalise + log
-// in place at d_out == p.out), or for bfloat16 / float16 features k_logmel_post_to from the fp32
-// scratch at p.out into d_out
+// in place at d_out == p.out, or for bfloat16 / float16 features from the fp32 scratch at p.out into d_out)
 int run_logmel_minmax(iris_ctx* c, FusedParams& p, void* d_out, cudaStream_t st, int out_type) {
     const size_t per_clip = size_t(c->n_mel) * c->T * p.c_out;
     uint32_t* mm = c->minmax.as<uint32_t>();
     unsigned* done = reinterpret_cast<unsigned*>(mm + 2 * size_t(c->B));
     int rc = timed_fused(c, p, FM_MEL, st, OUT_F32);
     if (rc) return rc;
-    if (out_type == OUT_F32) CU(launch_logmel_post(p.out, mm, done, c->B, per_clip, 1, 1, st));
-    else CU(launch_logmel_post_to(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
+    CU(launch_logmel_post(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
     return IRIS_OK;
 }
 
@@ -321,7 +319,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         p.out = d_out;
         p.do_log = mode != IRIS_FEAT_MEL;
         p.do_minmax = mode == IRIS_FEAT_LOGMEL_MINMAX;
-        const bool convert = p.do_minmax && out_type != OUT_F32;   // fp32 mel in scratch, k_logmel_post_to converts
+        const bool convert = p.do_minmax && out_type != OUT_F32;   // fp32 mel in scratch, k_logmel_post converts
         if (p.do_minmax) {
             CU(c->minmax.reserve(size_t(c->B) * 12));
             CU(cudaMemsetAsync(c->minmax.p, 0, size_t(c->B) * 12, st));
@@ -335,8 +333,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
                           c->mel_len.as<int32_t>(), st, convert ? OUT_F32 : out_type));
         uint32_t* mm = c->minmax.as<uint32_t>();
         unsigned* done = c->minmax.as<unsigned>() + 2 * size_t(c->B);
-        if (convert) CU(launch_logmel_post_to(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
-        else if (p.do_minmax) CU(launch_logmel_post(d_out, mm, done, c->B, per_clip, 1, 1, st));
+        if (p.do_minmax) CU(launch_logmel_post(p.out, d_out, out_type, mm, done, c->B, per_clip, 1, 1, st));
         return IRIS_OK;
     }
     // many channels: magnitudes through a scratch spectrogram (remapped by store_bin), then the stand-alone
@@ -355,10 +352,7 @@ int spec_features(iris_ctx* c, int mode, int select, float* d_out, cudaStream_t 
         int rc = iris_op_minmax(c, 0, mel_out, mel_out, c->B, int64_t(per_clip), 1, st);
         if (rc) return rc;
     }
-    if (out_type != OUT_F32)
-        CU(launch_logmel_post_to(mel_out, d_out, out_type, nullptr, nullptr, c->B, per_clip, 0, mode != IRIS_FEAT_MEL, st));
-    else if (mode != IRIS_FEAT_MEL)
-        CU(launch_logmel_post(d_out, nullptr, nullptr, c->B, per_clip, 0, 1, st));
+    CU(launch_logmel_post(mel_out, d_out, out_type, nullptr, nullptr, c->B, per_clip, 0, mode != IRIS_FEAT_MEL, st));
     return IRIS_OK;
 }
 
@@ -1186,7 +1180,7 @@ int iris_features_select(iris_ctx* c, int mode, int select, float* d_out, iris_s
             CU(c->minmax.reserve(size_t(c->B) * 12));   // [B,2] min/max words + [B] k_logmel_post counters
             if (c->minmax.p != before) CU(cudaMemsetAsync(c->minmax.p, 0, c->minmax.cap, st));
             p.minmax = c->minmax.as<uint32_t>();
-            if (out_type != OUT_F32) {   // k_fused writes fp32 mel + extrema to scratch, k_logmel_post_to converts
+            if (out_type != OUT_F32) {   // k_fused writes fp32 mel + extrema to scratch, k_logmel_post converts
                 rc = mel_scratch(c, &p.out);
                 if (rc) return rc;
             }

@@ -173,7 +173,7 @@ struct iris_ctx {
     int prof_clips = 0;               // clips of the launch the hook timed last
     // stand-alone ops (iris_ops_abi.cu): dense mel matrix + column supports, small scratch
     DevBuf mel_dense, mel_lo, mel_len, op_small, minmax_ops, eval_scratch, spec_scratch;
-    // fp32 mel features [B, n_mel, T, C] of a bfloat16 / float16 launch whose last pass (k_logmel_post_to)
+    // fp32 mel features [B, n_mel, T, C] of a bfloat16 / float16 launch whose last pass (k_logmel_post)
     // converts: the min-max log-mel modes and the many-channel spectrogram-bank fallback
     DevBuf mel_scratch;
     bool spec_mode = false;            // the uploaded plan mixes spectrogram banks

@@ -18,18 +18,14 @@ int fused_max_segments();      // mixing segments one clip may have
 bool fused_stages_output(int mode, int remap, int fr);   // FusedParams::stage_out for a launch
 int fused_max_mel_taps();      // sum over the 32-filter rounds of the longest filter
 int fused_max_mel_filter();    // taps of the longest filter
-int fused_max_frames_per_tile();
 int fused_pick_fr(int mel_taps);   // frames per tile (consumer warps per CTA)
 size_t fused_tile_bytes(const FusedParams& p, int* stride_out);   // size of p.tile_blocks
 
-// k_post.cu
-// minmax: [B,2] extrema words of the clips at x; done: [B] zeroed counters (both may be null without do_minmax)
-cudaError_t launch_logmel_post(float* x, uint32_t* minmax, unsigned* done, int B, size_t per_clip, int do_minmax,
-                               int do_log, cudaStream_t stream);
-// the same from the fp32 features at src into dst of OutType out_type (OUT_BF16 / OUT_F16); with neither
-// do_minmax nor do_log it only converts
-cudaError_t launch_logmel_post_to(const float* src, void* dst, int out_type, uint32_t* minmax, unsigned* done,
-                                  int B, size_t per_clip, int do_minmax, int do_log, cudaStream_t stream);
+// k_post.cu -- from the fp32 features at src into dst of OutType out_type.  src == dst: in place (OUT_F32
+// only), nothing to do without do_minmax or do_log; src != dst: with neither flag it only converts.
+// minmax: [B,2] extrema words of the clips at src; done: [B] zeroed counters (both may be null without do_minmax)
+cudaError_t launch_logmel_post(const float* src, void* dst, int out_type, uint32_t* minmax, unsigned* done, int B,
+                               size_t per_clip, int do_minmax, int do_log, cudaStream_t stream);
 
 // k_bank.cu
 cudaError_t launch_bank_prepare(const float* wav, const int64_t* d_offsets, const int64_t* d_pad_offsets,

@@ -33,7 +33,7 @@
 //    source row enters the SM once per tile.
 //  * LOGMEL_MINMAX: the warps of a CTA combine the extrema of a run of tiles of one clip in shared
 //    memory and the last one sends them to global atomics; k_logmel_post (k_post.cu) normalises and
-//    logs the batch in place right after.
+//    logs the batch right after (in place, or from an fp32 scratch into bfloat16 / float16 features).
 #include <cstdlib>
 #include <cstring>
 
@@ -978,7 +978,6 @@ int fused_max_segments() { return kMaxStages; }
 bool fused_stages_output(int mode, int remap, int fr) { return stages_output(mode, remap, fr); }
 int fused_max_mel_taps() { return kMaxTaps; }
 int fused_max_mel_filter() { return kMaxFilter; }
-int fused_max_frames_per_tile() { return kMaxFR; }
 
 // Frames per tile = consumer warps per CTA.  FR = 8 (two CTAs of 8 + 1 warps per SM: the
 // consumer warps spread evenly over the 4 schedulers and two independent CTAs hide each
@@ -1044,12 +1043,78 @@ bool fused_reads_plane(const FusedParams& p, int mode) {
            p.mel_f_lo + p.mel_f_n <= 128 && p.seg_select == 0 && p.pl_wave[0] != nullptr;
 }
 
+// Persistent grid: as many CTAs as are resident at once, asked of the occupancy calculator once per kernel
+// instance and device.  The register cap decides between 1 and 2 CTAs per SM: measured on B200, 96 registers
+// give 2 x 9 warps, 104 and 112 only one CTA (576 x 112 = 64512 < 65536, but registers are granted per warp in
+// larger units) -- 4-ch COMPLEX 570 -> 730 us, mel 200 -> 265 us.
+template <int MODE, int NJ, int EPI, class OutT>
+static cudaError_t launch_instance(FusedParams p, long long n_tiles, size_t smem, int num_sms, cudaStream_t stream) {
+    const auto kernel = k_fused<MODE, NJ, EPI, OutT>;
+    const int threads = (p.fr + 1) * 32;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    static int attr_dev = -1;   // function attributes are per device
+    static int per_sm = 1;
+    static size_t per_sm_smem = 0;
+    if (attr_dev != dev) {
+        cudaFuncAttributes fa;
+        cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+        if (e != cudaSuccess) return e;
+        e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024 - int(fa.sharedSizeBytes));
+        if (e != cudaSuccess) return e;
+        cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        attr_dev = dev;
+        per_sm_smem = 0;
+    }
+    if (per_sm_smem != smem) {
+        int nb = 0;
+        cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, kernel, threads, smem);
+        if (e != cudaSuccess) return e;
+        per_sm = nb < 1 ? 1 : nb;
+        per_sm_smem = smem;
+    }
+    const long long max_ctas = (long long)num_sms * per_sm;
+    const int grid = int(n_tiles < max_ctas ? n_tiles : max_ctas);
+    fused_schedule(p, n_tiles, grid);
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(unsigned(grid));
+    cfg.blockDim = dim3(unsigned(threads));
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, p);
+}
+
+// the instance of p.out's OutType
+template <int MODE, int NJ, int EPI>
+static cudaError_t launch_out(int out_type, const FusedParams& p, long long n_tiles, size_t smem, int num_sms,
+                              cudaStream_t stream) {
+    if (out_type == OUT_BF16) return launch_instance<MODE, NJ, EPI, __nv_bfloat16>(p, n_tiles, smem, num_sms, stream);
+    if (out_type == OUT_F16) return launch_instance<MODE, NJ, EPI, __half>(p, n_tiles, smem, num_sms, stream);
+    return launch_instance<MODE, NJ, EPI, float>(p, n_tiles, smem, num_sms, stream);
+}
+
+// a launch that reads the bin planes: EPI_PLANE | X, X = 0 or EPI_MONO for mono_chan; fixed: the default mel shape
+template <int X>
+static cudaError_t launch_plane(bool fixed, int out_type, const FusedParams& p, long long n_tiles, size_t smem,
+                                int num_sms, cudaStream_t stream) {
+    constexpr int kEpi = EPI_PLANE | X;
+    if (!fixed) return launch_out<FM_MEL, 4, kEpi>(out_type, p, n_tiles, smem, num_sms, stream);
+    if (p.do_minmax)
+        return launch_instance<FM_MEL, 4, kEpi | EPI_C2 | EPI_MINMAX, float>(p, n_tiles, smem, num_sms, stream);
+    if (p.do_log) return launch_out<FM_MEL, 4, kEpi | EPI_C2 | EPI_LOG>(out_type, p, n_tiles, smem, num_sms, stream);
+    return launch_out<FM_MEL, 4, kEpi | EPI_C2>(out_type, p, n_tiles, smem, num_sms, stream);
+}
+
 // p.tile_blocks (fused_tile_bytes) is provided by the caller; build_tiles: k_tiles builds them first
 // (otherwise the kernel in front -- k_labels -- has built them and triggers early).  out_type: OutType
 // of p.out; FM_ACTIVITY and the min-max epilogue write fp32 only.
-cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStream_t stream, bool build_tiles,
+cudaError_t launch_fused(const FusedParams& p, int mode, int num_sms, cudaStream_t stream, bool build_tiles,
                          int out_type) {
-    FusedParams p = p_in;
     const int FR = p.fr;
     if (FR < 1 || FR > kMaxFR) return cudaErrorInvalidValue;
     const int tpc = (p.T + FR - 1) / FR;
@@ -1067,65 +1132,11 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
     if (build_tiles) k_tiles<<<unsigned((n_tiles + 127) / 128), 128, 0, stream>>>(p);
     // k_fused is a programmatic dependent launch behind k_tiles / k_labels: its prologue overlaps
     // their tail
-    int dev = 0;
-    cudaGetDevice(&dev);
-    // persistent grid: as many CTAs as are resident at once, asked of the occupancy calculator once
-    // per kernel variant.  The register cap decides between 1 and 2 CTAs per SM: measured on B200,
-    // 96 registers give 2 x 9 warps, 104 and 112 only one CTA (576 x 112 = 64512 < 65536, but
-    // registers are granted per warp in larger units) -- 4-ch COMPLEX 570 -> 730 us, mel 200 -> 265 us.
-#define IRIS_LAUNCH(M, NJV, EPIV, T)                                                                   \
-    {                                                                                           \
-        const int threads = (FR + 1) * 32;                                                      \
-        static int attr_dev = -1;   /* function attributes are per device */                    \
-        static int per_sm = 1;                                                                  \
-        static size_t per_sm_smem = 0;                                                          \
-        if (attr_dev != dev) {                                                                  \
-            cudaFuncAttributes fa;                                                              \
-            cudaError_t e = cudaFuncGetAttributes(&fa, k_fused<M, NJV, EPIV, T>);                  \
-            if (e != cudaSuccess) return e;                                                     \
-            e = cudaFuncSetAttribute(k_fused<M, NJV, EPIV, T>,                                     \
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize,               \
-                                     227 * 1024 - int(fa.sharedSizeBytes));                     \
-            if (e != cudaSuccess) return e;                                                     \
-            cudaFuncSetAttribute(k_fused<M, NJV, EPIV, T>, cudaFuncAttributePreferredSharedMemoryCarveout, \
-                                 cudaSharedmemCarveoutMaxShared);                               \
-            attr_dev = dev;                                                                     \
-            per_sm_smem = 0;                                                                    \
-        }                                                                                       \
-        if (per_sm_smem != smem) {                                                              \
-            int nb = 0;                                                                         \
-            cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_fused<M, NJV, EPIV, T>, \
-                                                                          threads, smem);       \
-            if (e != cudaSuccess) return e;                                                     \
-            per_sm = nb < 1 ? 1 : nb;                                                           \
-            per_sm_smem = smem;                                                                 \
-        }                                                                                       \
-        const long long max_ctas = (long long)num_sms * per_sm;                                 \
-        const int grid = int(n_tiles < max_ctas ? n_tiles : max_ctas);                          \
-        fused_schedule(p, n_tiles, grid);                                                       \
-        cudaLaunchConfig_t cfg{};                                                               \
-        cfg.gridDim = dim3(unsigned(grid));                                                     \
-        cfg.blockDim = dim3(unsigned(threads));                                                 \
-        cfg.dynamicSmemBytes = smem;                                                            \
-        cfg.stream = stream;                                                                    \
-        cudaLaunchAttribute attr[1];                                                            \
-        attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                        \
-        attr[0].val.programmaticStreamSerializationAllowed = 1;                                 \
-        cfg.attrs = attr;                                                                       \
-        cfg.numAttrs = 1;                                                                       \
-        cudaError_t le = cudaLaunchKernelEx(&cfg, k_fused<M, NJV, EPIV, T>, p);                    \
-        if (le != cudaSuccess) return le;                                                       \
-    }
-#define IRIS_LAUNCH_OUT(M, NJV, EPIV)                                                         \
-    {                                                                                           \
-        if (out_type == OUT_BF16) IRIS_LAUNCH(M, NJV, EPIV, __nv_bfloat16)                      \
-        else if (out_type == OUT_F16) IRIS_LAUNCH(M, NJV, EPIV, __half)                         \
-        else IRIS_LAUNCH(M, NJV, EPIV, float)                                                   \
-    }
+    cudaError_t e;
     switch (mode) {
-        case FM_COMPLEX: IRIS_LAUNCH_OUT(FM_COMPLEX, 8, 0) break;
-        case FM_MAGPHASE: IRIS_LAUNCH_OUT(FM_MAGPHASE, 8, 0) break;
-        case FM_LOGMAGPHASE: IRIS_LAUNCH_OUT(FM_LOGMAGPHASE, 8, 0) break;
+        case FM_COMPLEX: e = launch_out<FM_COMPLEX, 8, 0>(out_type, p, n_tiles, smem, num_sms, stream); break;
+        case FM_MAGPHASE: e = launch_out<FM_MAGPHASE, 8, 0>(out_type, p, n_tiles, smem, num_sms, stream); break;
+        case FM_LOGMAGPHASE: e = launch_out<FM_LOGMAGPHASE, 8, 0>(out_type, p, n_tiles, smem, num_sms, stream); break;
         case FM_MEL: {
             // p.plane (fused_reads_plane): 2 channels, no remap or mono_chan, support below bin 128 -- the mix of
             // the banks' stored bins, fixed-shape or generic instance.  Otherwise the FFT path: NJ = 8 for a
@@ -1136,41 +1147,33 @@ cudaError_t launch_fused(const FusedParams& p_in, int mode, int num_sms, cudaStr
                 const bool fixed = p.mel_L[0] == fixed_mel_L(0) && p.mel_L[1] == fixed_mel_L(1) &&
                                    p.mel_L[2] == fixed_mel_L(2) && p.mel_L[3] == fixed_mel_L(3) && FR == kFixFR &&
                                    p.mel_taps == 12 && !getenv("IRIS_NO_FIXED_EPI");
-                // X = 0, or EPI_MONO for mono_chan
-#define IRIS_LAUNCH_PLANE(X)                                                                    \
-    {                                                                                           \
-        if (!fixed) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | X)                                   \
-        else if (p.do_minmax) IRIS_LAUNCH(FM_MEL, 4, EPI_PLANE | EPI_C2 | EPI_MINMAX | X, float) \
-        else if (p.do_log) IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | EPI_C2 | EPI_LOG | X)         \
-        else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_PLANE | EPI_C2 | X)                                 \
-    }
-                if (p.remap == REMAP_MONO_CHAN) IRIS_LAUNCH_PLANE(EPI_MONO)
-                else IRIS_LAUNCH_PLANE(0)
-#undef IRIS_LAUNCH_PLANE
+                if (p.remap == REMAP_MONO_CHAN)
+                    e = launch_plane<EPI_MONO>(fixed, out_type, p, n_tiles, smem, num_sms, stream);
+                else
+                    e = launch_plane<0>(fixed, out_type, p, n_tiles, smem, num_sms, stream);
             } else if (p.remap == REMAP_MONO_CHAN) {
                 if (!nj8) return cudaErrorInvalidValue;   // bins below 128 only: the plane path
-                IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_MONO)
+                e = launch_out<FM_MEL, 8, EPI_MONO>(out_type, p, n_tiles, smem, num_sms, stream);
             } else if (p.remap != REMAP_NONE) {
-                if (nj8) IRIS_LAUNCH_OUT(FM_MEL, 8, EPI_REMAP)
-                else IRIS_LAUNCH_OUT(FM_MEL, 4, EPI_REMAP)
+                if (nj8) e = launch_out<FM_MEL, 8, EPI_REMAP>(out_type, p, n_tiles, smem, num_sms, stream);
+                else e = launch_out<FM_MEL, 4, EPI_REMAP>(out_type, p, n_tiles, smem, num_sms, stream);
             } else if (nj8) {
-                IRIS_LAUNCH_OUT(FM_MEL, 8, 0)
+                e = launch_out<FM_MEL, 8, 0>(out_type, p, n_tiles, smem, num_sms, stream);
             } else {
                 if (p.C == 2) return cudaErrorInvalidValue;   // the plane path
-                IRIS_LAUNCH_OUT(FM_MEL, 4, 0)
+                e = launch_out<FM_MEL, 4, 0>(out_type, p, n_tiles, smem, num_sms, stream);
             }
             break;
         }
-        case FM_ACTIVITY: IRIS_LAUNCH(FM_ACTIVITY, 8, 0, float) break;
-        case FM_PLANE: IRIS_LAUNCH(FM_PLANE, 4, 0, float) break;
+        case FM_ACTIVITY: e = launch_instance<FM_ACTIVITY, 8, 0, float>(p, n_tiles, smem, num_sms, stream); break;
+        case FM_PLANE: e = launch_instance<FM_PLANE, 4, 0, float>(p, n_tiles, smem, num_sms, stream); break;
         case FM_SE:   // both virtual pairs of a (clip, time) range in one CTA: the combined store
             if (out_type != OUT_F32 || !p.pair_merge || p.seg_select != 3) return cudaErrorInvalidValue;
-            IRIS_LAUNCH(FM_SE, 8, 0, float)
+            e = launch_instance<FM_SE, 8, 0, float>(p, n_tiles, smem, num_sms, stream);
             break;
         default: return cudaErrorInvalidValue;
     }
-#undef IRIS_LAUNCH_OUT
-#undef IRIS_LAUNCH
+    if (e != cudaSuccess) return e;
     return cudaGetLastError();
 }
 

@@ -281,43 +281,47 @@ cudaError_t launch_spec_activity(const float* specs, const int64_t* frame_off, i
 
 size_t specmix_mel_smem(int C, int f_n) { return size_t(f_n) * kSpecTile * C * 4; }
 
+// one k_specmix instance; FM_MEL: its dynamic shared memory attribute is set once per instance
+template <int MODE, class OutT, bool kMono = false>
+static cudaError_t launch_specmix_instance(const FusedParams& p, const float* melW, const int32_t* mel_lo,
+                                           const int32_t* mel_len, cudaStream_t st) {
+    size_t smem = 0;
+    if constexpr (MODE == FM_MEL) {
+        smem = specmix_mel_smem(p.c_out, p.mel_f_n);
+        if (smem > 200 * 1024) return cudaErrorInvalidValue;
+        static bool attr_set = false;
+        if (!attr_set) {
+            cudaError_t e = cudaFuncSetAttribute(k_specmix<MODE, OutT, kMono>,
+                                                 cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+            if (e != cudaSuccess) return e;
+            attr_set = true;
+        }
+    }
+    const dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
+    k_specmix<MODE, OutT, kMono><<<grid, kSpecWarps * 32, smem, st>>>(p, melW, mel_lo, mel_len);
+    return cudaGetLastError();
+}
+
 template <class OutT>
 static cudaError_t launch_specmix_t(const FusedParams& p, int mode, const float* melW, const int32_t* mel_lo,
                                     const int32_t* mel_len, cudaStream_t st) {
-    dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
-    const int threads = kSpecWarps * 32;
     const bool mono = p.remap == REMAP_MONO_CHAN;   // the spectrogram modes of mono_chan: instances of their own
     if (mono && (p.C != 2 || p.c_out != 2)) return cudaErrorInvalidValue;
     switch (mode) {
         case FM_COMPLEX:
-            if (mono) k_specmix<FM_COMPLEX, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            else k_specmix<FM_COMPLEX, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            break;
+            return mono ? launch_specmix_instance<FM_COMPLEX, OutT, true>(p, nullptr, nullptr, nullptr, st)
+                        : launch_specmix_instance<FM_COMPLEX, OutT>(p, nullptr, nullptr, nullptr, st);
         case FM_MAGPHASE:
-            if (mono) k_specmix<FM_MAGPHASE, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            else k_specmix<FM_MAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            break;
+            return mono ? launch_specmix_instance<FM_MAGPHASE, OutT, true>(p, nullptr, nullptr, nullptr, st)
+                        : launch_specmix_instance<FM_MAGPHASE, OutT>(p, nullptr, nullptr, nullptr, st);
         case FM_LOGMAGPHASE:
-            if (mono) k_specmix<FM_LOGMAGPHASE, OutT, true><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            else k_specmix<FM_LOGMAGPHASE, OutT><<<grid, threads, 0, st>>>(p, nullptr, nullptr, nullptr);
-            break;
-        case FM_MEL: {
+            return mono ? launch_specmix_instance<FM_LOGMAGPHASE, OutT, true>(p, nullptr, nullptr, nullptr, st)
+                        : launch_specmix_instance<FM_LOGMAGPHASE, OutT>(p, nullptr, nullptr, nullptr, st);
+        case FM_MEL:
             if (p.remap != REMAP_NONE && !mono && (p.C != 2 || p.c_out < 3)) return cudaErrorInvalidValue;
-            const size_t smem = specmix_mel_smem(p.c_out, p.mel_f_n);
-            if (smem > 200 * 1024) return cudaErrorInvalidValue;
-            static bool attr_set = false;   // per instance
-            if (!attr_set) {
-                cudaError_t e = cudaFuncSetAttribute(k_specmix<FM_MEL, OutT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                     200 * 1024);
-                if (e != cudaSuccess) return e;
-                attr_set = true;
-            }
-            k_specmix<FM_MEL, OutT><<<grid, threads, smem, st>>>(p, melW, mel_lo, mel_len);
-            break;
-        }
+            return launch_specmix_instance<FM_MEL, OutT>(p, melW, mel_lo, mel_len, st);
         default: return cudaErrorInvalidValue;
     }
-    return cudaGetLastError();
 }
 
 // mode FM_MEL: p.out [B, n_mel, T, c_out], p.do_log / p.do_minmax / p.minmax as in the fused kernel;
@@ -330,9 +334,7 @@ cudaError_t launch_specmix(const FusedParams& p, int mode, const float* melW, co
     if (out_type != OUT_F32 && p.do_minmax) return cudaErrorInvalidValue;
     if (mode == FM_SE) {   // fp32, 2 channels, no remap; every segment kept (the subsets are split per cell)
         if (out_type != OUT_F32 || p.C != 2 || p.remap != REMAP_NONE || p.seg_select != 0) return cudaErrorInvalidValue;
-        dim3 grid(unsigned((p.T + kSpecTile - 1) / kSpecTile), unsigned(p.B));
-        k_specmix<FM_SE, float><<<grid, kSpecWarps * 32, 0, st>>>(p, nullptr, nullptr, nullptr);
-        return cudaGetLastError();
+        return launch_specmix_instance<FM_SE, float>(p, nullptr, nullptr, nullptr, st);
     }
     switch (out_type) {
         case OUT_F32: return launch_specmix_t<float>(p, mode, melW, mel_lo, mel_len, st);
